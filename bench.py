@@ -2,6 +2,7 @@
 """bench.py -- predicted frames/s of the ExtDM sampling hot path (BASELINE.json metric) on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]           # this repo's CUDA path
+  python bench.py [...] --dump-outputs DIR                      # + the last timed step's predicted frames, as .npy
   python bench.py --impl reference [...]                        # the UNMODIFIED reference on the host CPU cores
 
 Headline workload = the configuration BASELINE.json's metric names: BAIR 64x64, 2 -> 28 autoregressive rollout
@@ -105,6 +106,26 @@ def make_clip(name, B, tc, hw, seed):
     return torch.rand(B, c, tc, hw, hw, generator=g).expand(B, 3, tc, hw, hw).contiguous()
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_frames(path, frames, seed=0):
+    """--dump-outputs: the predicted frames (B, 3, T, H, W) of the last timed step as <path>/pred_frames.npy, float32.
+    Above DUMP_BYTES only a fixed, seeded subset of the videos is written, in index order; a single video over
+    DUMP_BYTES is cut to its first frames (one frame of 3 x H x W floats is assumed to fit)."""
+    import numpy as np
+    import torch
+    per_video = frames[0].numel() * 4
+    if frames.shape[0] * per_video > DUMP_BYTES:
+        keep = max(1, DUMP_BYTES // per_video)
+        idx = torch.randperm(frames.shape[0], generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+        frames = frames[idx.to(frames.device)]
+    if frames.numel() * 4 > DUMP_BYTES:
+        frames = frames[:, :, :DUMP_BYTES // (frames[0, :, 0].numel() * 4)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pred_frames.npy"), frames.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------ reference legs
 def build_reference(name, device, seed=1234):
     """The UNMODIFIED reference FlowDiffusion for a dataset (oracle/_ref staged by oracle/make_ref.py, import shims of
@@ -201,8 +222,9 @@ def cpu_reference(name=HEADLINE, videos=1, repeats=1, threads=None):
                       f"torch {torch.__version__}", "seconds_per_rollout": sec, "timed_rollouts": repeats}, sec
 
 
-def cpu_port_fallback(threads=None):
-    """Only when oracle/_ref was not staged: the oracle port (kind 'port'), one BAIR round at batch 1."""
+def cpu_port_fallback(threads=None, repeats=1):
+    """Only when oracle/_ref was not staged: the oracle port (kind 'port'), one BAIR round at batch 1, timed `repeats`
+    times."""
     import torch
     from oracle import extdm_oracle as O
     from extdm_b200.manifest import UnetConfig, unet_manifest
@@ -217,22 +239,25 @@ def cpu_port_fallback(threads=None):
     nz = [torch.randn(1, 3, tp, 32, 32, generator=g) for _ in range(10)]
     with torch.no_grad():
         O.ddim_sample(O.SD(sd), O.unet_config("u12", tc, tp), x_cond, fea, nz[0], nz[1:2] + [None], sampling=1)
-        t0 = time.perf_counter()
-        O.ddim_sample(O.SD(sd), O.unet_config("u12", tc, tp), x_cond, fea, nz[0], nz[1:] + [None], sampling=10)
-        sec = time.perf_counter() - t0
+        times = []
+        for _ in range(repeats):
+            t0 = time.perf_counter()
+            O.ddim_sample(O.SD(sd), O.unet_config("u12", tc, tp), x_cond, fea, nz[0], nz[1:] + [None], sampling=10)
+            times.append(time.perf_counter() - t0)
+        sec = sum(times) / len(times)
     return {"value": tp / sec, "unit": "frames/s", "cores": threads, "kind": "port",
             "sample": f"oracle/_ref not staged: oracle port, BAIR u12 batch 1, ONE round's 10-step DDIM loop timed "
-                      f"({sec:.1f} s; conditioning and decode excluded)"}, sec
+                      f"{repeats}x ({sec:.1f} s each; conditioning and decode excluded)"}, sec
 
 
 def run_reference_arm(args):
     """`--impl reference`: the reference's own CPU implementation of the path on the host cores, on the headline
     configuration (bounded sample: one video per step, the whole rollout) and on BASELINE config 1 (SMMNIST 10->10,
-    batch 1).  Steps are really executed; `steps` in the line is the number executed (capped so the run ends in minutes)."""
+    batch 1).  `--steps` timed repeats are really executed (one rollout on the host cores takes minutes)."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     from oracle import ref_shims
-    n = max(1, min(args.steps, 3))
+    n = args.steps
     if ref_shims.available():
         cb, sec = cpu_reference(HEADLINE, videos=1, repeats=n)
         try:
@@ -242,9 +267,8 @@ def run_reference_arm(args):
         except Exception as e:
             per_config = {"smmnist_b1": {"error": str(e)}}
     else:
-        cb, sec = cpu_port_fallback()
+        cb, sec = cpu_port_fallback(repeats=n)
         per_config = {}
-        n = 1
     line = {"metric": METRIC, "value": cb["value"], "unit": "frames/s", "n_gpus": args.gpus, "steps": n,
             "steps_requested": args.steps, "warmup": 1, "ms_per_step": 1e3 * sec, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
@@ -331,7 +355,14 @@ def main():
     ap.add_argument("--ncu-range", action="store_true",
                     help="for `ncu --profile-from-start off`: after the warm-up, bracket ONE step with "
                          "cudaProfilerStart/Stop and exit without printing a bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the predicted frames of the last timed step to DIR/pred_frames.npy (float32; above "
+                         "64 MB a fixed, seeded subset of the videos), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -382,11 +413,13 @@ def main():
     copy_stream = torch.cuda.Stream(device=dev)
     h2d_done = [torch.cuda.Event() for _ in range(2)]
     keep = [None, None]
+    last = {}                                                  # what the latest step_dev returned (--dump-outputs)
 
     def step_dev(i):
         pred = configs.rollout(model, clip_dev, total_pred)
         if world > 1:
-            sharding.gather_predictions(pred.contiguous(), world * B)
+            pred = sharding.gather_predictions(pred.contiguous(), world * B)
+        last["pred"] = pred
         return pred
 
     def issue_h2d(i):
@@ -434,9 +467,14 @@ def main():
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
+    # the timed steps draw their DDIM noise from the default generator: seeded here, the same arguments give the same
+    # outputs run after run, whatever ran before
+    torch.manual_seed(1234)
     ms_dev = time_rollouts(step_dev, args.steps)
     ms_e2e = timed_e2e(args.steps)
     clock_info = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_frames(args.dump_outputs, last["pred"])
 
     # ---- kernel accounting: the per-kernel roofline, measured live with CUDA events (eager replay of the launch lists)
     runner = next(iter(model.unet._runners.values()))

@@ -3,7 +3,9 @@
 Run in the build container only:   python tests/golden/make_golden.py
 Writes tests/golden/<case>.pt = {cfg, manifest (key -> shape of the reference state_dict), seeds,
 outputs}.  Inputs and weights are NOT stored: they are regenerated from seeds by `inputs_for()` below
-and `weights.synth_state_dict` (both deterministic on the CPU generator), so fixtures stay small.
+and `weights.synth_state_dict` (both deterministic on the CPU generator), so fixtures stay small.  The pipeline and
+rollout fixtures go through tests/rollout_common.py::save: xz-compressed as <case>.pt.xz above 1 MB, and a rollout in
+a compact form that rollout_common.load() expands exactly; save() refuses a file over 1 MB.
 """
 import importlib
 import os
@@ -15,8 +17,10 @@ import yaml
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 
 from oracle import ref_shims  # noqa: E402
+from rollout_common import save  # noqa: E402
 
 ref_shims.install()
 import extdm_b200  # noqa: E402
@@ -175,9 +179,8 @@ def gen_pipeline():
             ret = fd.sample_one_video(cond_scale=1.0, real_vid=real_vid.contiguous())
     finally:
         torch.randn, torch.randn_like = real_randn, real_randn_like
-    torch.save(dict(kind="pipeline", cfg=cfg, B=B, weight_seeds=seeds, manifests=mans, input_seed=500,
-                    noise_seed=600, out={k: v.clone() for k, v in ret.items()}),
-               os.path.join(HERE, "pipeline_kth_c2p5.pt"))
+    save(dict(kind="pipeline", cfg=cfg, B=B, weight_seeds=seeds, manifests=mans, input_seed=500,
+              noise_seed=600, out={k: v.clone() for k, v in ret.items()}), "pipeline_kth_c2p5")
     print("pipeline", {k: tuple(v.shape) for k, v in ret.items()})
 
 
@@ -211,8 +214,8 @@ def gen_pipeline_full():
         torch.randn, torch.randn_like = real_randn, real_randn_like
     out = {"sample_vid_grid": ret["sample_vid_grid"].clone(), "sample_vid_conf": ret["sample_vid_conf"].clone(),
            "sample_out_vid": ret["sample_out_vid"].half()}
-    torch.save(dict(kind="pipeline_full", B=B, tc=tc, tp=tp, steps=steps, weight_seeds=seeds, input_seed=700,
-                    noise_seed=800, noises_left=len(queue), out=out), os.path.join(HERE, "pipeline_kth_full.pt"))
+    save(dict(kind="pipeline_full", B=B, tc=tc, tp=tp, steps=steps, weight_seeds=seeds, input_seed=700,
+              noise_seed=800, noises_left=len(queue), out=out), "pipeline_kth_full")
     print("pipeline_full", {k: tuple(v.shape) for k, v in out.items()}, "unused noises", len(queue))
 
 
@@ -225,7 +228,8 @@ PIPELINE_CASES = {
     "rollout_smmnist": ("smmnist", "VideoFlowDiffusion_multi1248", "base", 2, 10),          # the full 10 -> 10 rollout
     "rollout_bair": ("bair", "VideoFlowDiffusion_multi_w_ref", "u12", 3, 10),               # the full 2 -> 28 rollout
     "rollout_ucf": ("ucf", "VideoFlowDiffusion_multi_w_ref", "ada", 2, 10),                 # the full 4 -> 12 rollout
-    "rollout_cityscapes": ("cityscapes", "VideoFlowDiffusion_multi_w_ref", "ada", 2, 10),   # 128x128, sf 0.25, perspective
+    # 128x128, sf 0.25, perspective; one round: two rounds of 128x128 frames do not fit in 1 MB
+    "rollout_cityscapes": ("cityscapes", "VideoFlowDiffusion_multi_w_ref", "ada", 1, 10),
     "rollout_cityscapes_u22": ("cityscapes", "VideoFlowDiffusion_multi_w_ref_u22", "u22", 1, 10),
 }
 PIPELINE_SEEDS = dict(generator=21, region_predictor=22, bg_predictor=23, diffusion=11)
@@ -295,10 +299,9 @@ def gen_rollout(name):
                            "sample_out_vid": ret["sample_out_vid"].half()})
         cond = ret["sample_out_vid"][:, :, -tc:].clone()             # scripts/DM/valid.py:171
         print(name, "round", r, "flow abs-mean", float(ret["sample_vid_grid"].abs().mean()), flush=True)
-    torch.save(dict(kind="rollout", dataset=dataset, dm_arch=dm_arch, variant=variant, rounds=rounds, steps=steps,
-                    cfg=cfg, B=B, tc=tc, tp=tp, hw=hw, weight_seeds=PIPELINE_SEEDS, input_seed=in_seed, noise_seed=nz_seed,
-                    manifests={k: v for k, v in mans.items() if k != "diffusion"}, out=out_rounds),
-               os.path.join(HERE, name + ".pt"))
+    save(dict(kind="rollout", dataset=dataset, dm_arch=dm_arch, variant=variant, rounds=rounds, steps=steps,
+              cfg=cfg, B=B, tc=tc, tp=tp, hw=hw, weight_seeds=PIPELINE_SEEDS, input_seed=in_seed, noise_seed=nz_seed,
+              manifests={k: v for k, v in mans.items() if k != "diffusion"}, out=out_rounds), name)
 
 
 if __name__ == "__main__":

@@ -11,6 +11,7 @@ import torch
 import extdm_b200  # noqa: F401
 from extdm_b200 import lib
 from extdm_b200.manifest import UnetConfig, adaptor_layers, unet_manifest
+from rollout_common import load as load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
@@ -40,7 +41,7 @@ def test_adaptor_layers():
 
 def test_wrapper_state_dicts_match_reference():
     from extdm_b200.flow_diffusion import FlowDiffusion
-    fx = torch.load(os.path.join(GOLD, "pipeline_kth_c2p5.pt"))
+    fx = load_golden("pipeline_kth_c2p5")
     fd = FlowDiffusion(config=fx["cfg"], pretrained_pth="", is_train=False,
                        Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada")
     for part in ("generator", "region_predictor", "bg_predictor", "diffusion"):
@@ -52,9 +53,10 @@ def test_wrapper_state_dicts_match_reference():
 def test_conditioning_stage_matches_reference_on_cpu():
     from extdm_b200.flow_diffusion import FlowDiffusion
     from extdm_b200.weights import synth_state_dict
-    fx = torch.load(os.path.join(GOLD, "pipeline_kth_c2p5.pt"))
+    fx = load_golden("pipeline_kth_c2p5")
+    # the constructor puts the LFAE modules on cuda:0 when there is one (as the reference does): keep them on the CPU
     fd = FlowDiffusion(config=fx["cfg"], pretrained_pth="", is_train=False,
-                       Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada").eval()
+                       Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada").eval().cpu()
     for part, seed in fx["weight_seeds"].items():
         m = getattr(fd, part)
         m.load_state_dict(synth_state_dict(fx["manifests"][part], seed, base=m.state_dict()), strict=True)
@@ -160,7 +162,7 @@ def test_result_wire_format(tmp_path):
     assert torch.equal(torch.load(tmp_path / "origin.pt"), origin[:, 0])
     assert torch.equal(torch.load(tmp_path / "result_2.pt"), result[:, 2])
     from extdm_b200.flow_diffusion import FlowDiffusion
-    fx = torch.load(os.path.join(GOLD, "pipeline_kth_c2p5.pt"))
+    fx = load_golden("pipeline_kth_c2p5")
     fd = FlowDiffusion(config=fx["cfg"], pretrained_pth="", is_train=False,
                        Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada").eval()
     sd = {k: v.clone() + 1 for k, v in fd.diffusion.state_dict().items() if v.dtype.is_floating_point}

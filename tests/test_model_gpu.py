@@ -17,6 +17,7 @@ pytestmark = pytest.mark.gpu
 
 import extdm_b200  # noqa: E402
 from extdm_b200.weights import synth_state_dict  # noqa: E402
+from rollout_common import load as load_golden  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
@@ -173,7 +174,7 @@ def test_generator_decode_matches_reference():
     import yaml  # noqa: F401
     from extdm_b200.lfae import Generator
     fx = torch.load(os.path.join(GOLD, "generator_fwf.pt"))
-    pipe = torch.load(os.path.join(GOLD, "pipeline_kth_c2p5.pt"))
+    pipe = load_golden("pipeline_kth_c2p5")
     fp = pipe["cfg"]["flow_params"]["model_params"]
     gen = Generator(num_regions=fp["num_regions"], num_channels=fp["num_channels"],
                     revert_axis_swap=fp["revert_axis_swap"], **fp["generator_params"]).cuda().eval()
@@ -194,7 +195,7 @@ def test_generator_decode_matches_reference():
 
 def test_pipeline_matches_reference(request):
     from extdm_b200.flow_diffusion import FlowDiffusion
-    fx = torch.load(os.path.join(GOLD, "pipeline_kth_c2p5.pt"))
+    fx = load_golden("pipeline_kth_c2p5")
     fd = FlowDiffusion(config=fx["cfg"], pretrained_pth="", is_train=False,
                        Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada").eval()
     for part, seed in fx["weight_seeds"].items():
@@ -331,7 +332,7 @@ def test_full_size_round_matches_reference(request):
     end-to-end latent flow rel-L2 <= 2e-2, decoded frames PSNR >= 35 dB (smooth, natural-video-like clip)."""
     from extdm_b200 import configs
     from extdm_b200.flow_diffusion import FlowDiffusion
-    fx = torch.load(os.path.join(GOLD, "pipeline_kth_full.pt"))
+    fx = load_golden("pipeline_kth_full")
     cfg = configs.dataset("kth")[0]
     fd = FlowDiffusion(config=cfg, pretrained_pth="", is_train=False,
                        Unet3D_architecture="DenoiseNet_STWAtt_w_w_ref_adaptor_cross_multi_traj_ada").eval()

@@ -1,4 +1,4 @@
-"""CPU: the end-to-end fixtures of every BASELINE.json configuration (tests/golden/rollout_*.pt, produced by the
+"""CPU: the end-to-end fixtures of every BASELINE.json configuration (tests/golden/rollout_*, produced by the
 unmodified reference wrappers through the autoregressive loop of scripts/DM/valid.py:167-172) against
 
   * this repo's configuration table (configs.py) -- the fields FlowDiffusion reads equal the reference yaml's,

@@ -1,5 +1,5 @@
 """End-to-end parity (-m gpu) of every BASELINE.json configuration against the UNMODIFIED reference wrappers run through
-the autoregressive loop of scripts/DM/valid.py:167-172 (tests/golden/rollout_*.pt; generator:
+the autoregressive loop of scripts/DM/valid.py:167-172 (tests/golden/rollout_*; generator:
 tests/golden/make_golden.py::gen_rollout): SMMNIST via VideoFlowDiffusion_multi1248 (10 -> 10, the full rollout), BAIR
 via multi_w_ref + traj_u12 (2 -> 28, the full rollout), UCF (64 regions), Cityscapes 128x128 (perspective background,
 scale factor 0.25) and the shipped multi_w_ref_u22 + traj_ada_u22 pairing.  Shipped (tc, tp), 10 DDIM steps, eta = 1,
