@@ -2,6 +2,8 @@
 // (model/BaseDM_adaptor/Diffusion.py:231-255); the per-sample 0.9-quantile of |x_start| reproduces
 // torch.quantile (linear interpolation, rank computed in fp32) through an exact radix select of the two
 // neighbouring order statistics instead of a full sort.
+// The DDPM ancestral step (GaussianDiffusion.p_sample_loop) shares that select; its per-step coefficients, step index and
+// Philox noise live on the device, so one captured iteration can be replayed for every timestep.
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -12,11 +14,12 @@ __device__ __forceinline__ float x_start_of(float img, float pred, float c_recip
   return __fsub_rn(__fmul_rn(c_recip, img), __fmul_rn(c_recipm1, pred));
 }
 
-// One CTA per sample.  |x| >= 0 so the IEEE bit pattern orders like an unsigned integer.
-__global__ void __launch_bounds__(1024) ddim_threshold_kernel(const float* __restrict__ img,
-                                                              const float* __restrict__ pred, float c_recip,
-                                                              float c_recipm1, float q, float* __restrict__ s_out,
-                                                              int n) {
+// One CTA per sample: s_out[b] = max(1, quantile_q(|x_start[b]|)).  |x| >= 0 so the IEEE bit pattern orders like an
+// unsigned integer.  Shared by the DDIM kernel (coefficients as arguments) and the DDPM kernel (coefficients read from
+// the schedule table on the device), so both take the same select path.
+__device__ __forceinline__ void threshold_sample(const float* __restrict__ img, const float* __restrict__ pred,
+                                                 float c_recip, float c_recipm1, float q, float* __restrict__ s_out,
+                                                 int n) {
   __shared__ unsigned int hist[256];
   __shared__ unsigned int s_prefix, s_k;
   __shared__ unsigned int s_cnt_le, s_min_gt;
@@ -79,6 +82,13 @@ __global__ void __launch_bounds__(1024) ddim_threshold_kernel(const float* __res
   }
 }
 
+__global__ void __launch_bounds__(1024) ddim_threshold_kernel(const float* __restrict__ img,
+                                                              const float* __restrict__ pred, float c_recip,
+                                                              float c_recipm1, float q, float* __restrict__ s_out,
+                                                              int n) {
+  threshold_sample(img, pred, c_recip, c_recipm1, q, s_out, n);
+}
+
 __global__ void __launch_bounds__(256) ddim_update_kernel(const float* __restrict__ img,
                                                           const float* __restrict__ pred,
                                                           const float* __restrict__ noise,
@@ -108,6 +118,125 @@ __global__ void __launch_bounds__(256) ddim_update_kernel(const float* __restric
   }
 }
 
+// ------------------------------------------------------------------------------------------------ DDPM (ancestral)
+// One schedule row per step: {sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod, posterior_mean_coef1,
+// posterior_mean_coef2, nonzero_mask * exp(0.5 * posterior_log_variance_clipped)} at t = times[step].
+constexpr int kDdpmRow = 5;
+// Philox counter word 2: which draw of a step (the loop noise of step `step`, or the initial x_T)
+constexpr unsigned int kStreamStep = 0u, kStreamInit = 1u;
+
+// Philox4x32-10 (Salmon et al., SC'11), counter-based: the output depends on (counter, key) only.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+  constexpr unsigned int M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) { k.x += W0; k.y += W1; }
+    const unsigned int hi0 = __umulhi(M0, c.x), lo0 = M0 * c.x;
+    const unsigned int hi1 = __umulhi(M1, c.z), lo1 = M1 * c.z;
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+
+// Box-Muller: u1 in (0, 1) with 23 bits (never 0, so the log is finite), u2 in [0, 1) with 24 bits.
+__device__ __forceinline__ float2 box_muller(unsigned int a, unsigned int b) {
+  const float u1 = (static_cast<float>(a >> 9) + 0.5f) * 0x1p-23f;
+  const float u2 = static_cast<float>(b >> 8) * 0x1p-24f;
+  const float r = sqrtf(-2.0f * logf(u1));
+  float sn, cs;
+  sincospif(2.0f * u2, &sn, &cs);
+  return make_float2(r * cs, r * sn);
+}
+
+// Four N(0, 1) draws for elements 4*quad .. 4*quad+3 of the video with this seed.  Keying by the video's own seed and
+// the element index within the video makes a video's noise independent of the batch it is sampled in.
+__device__ __forceinline__ float4 normal4(long long seed, unsigned int quad, unsigned int step, unsigned int stream) {
+  const unsigned long long sd = static_cast<unsigned long long>(seed);
+  const uint4 r = philox4x32_10(make_uint4(quad, step, stream, 0u),
+                                make_uint2(static_cast<unsigned int>(sd), static_cast<unsigned int>(sd >> 32)));
+  const float2 p = box_muller(r.x, r.y), q = box_muller(r.z, r.w);
+  return make_float4(p.x, p.y, q.x, q.y);
+}
+
+__global__ void __launch_bounds__(1024) ddpm_threshold_kernel(const float* __restrict__ img,
+                                                              const float* __restrict__ pred,
+                                                              const float* __restrict__ rows,
+                                                              const int* __restrict__ step, float q,
+                                                              float* __restrict__ s_out, int n) {
+  const float* row = rows + static_cast<long long>(*step) * kDdpmRow;
+  threshold_sample(img, pred, row[0], row[1], q, s_out, n);
+}
+
+// x0 = clamp(c_recip*img - c_recipm1*pred, -s, s) / s;  out = (c1*x0 + c2*img) + sig*z, op by op as
+// GaussianDiffusion.p_sample evaluates it in fp32 (no FMA).  z is slice *step of `noise` when given, else Philox.
+__global__ void __launch_bounds__(256) ddpm_update_kernel(const float* __restrict__ img,
+                                                          const float* __restrict__ pred,
+                                                          const float* __restrict__ rows,
+                                                          const int* __restrict__ step,
+                                                          const long long* __restrict__ seeds,
+                                                          const float* __restrict__ noise,
+                                                          const float* __restrict__ s,
+                                                          float* __restrict__ img_out, float* __restrict__ xs_out,
+                                                          int n4_per_sample, long long total4) {
+  const int st = __ldg(step);
+  const float* row = rows + static_cast<long long>(st) * kDdpmRow;
+  const float c_recip = __ldg(row + 0), c_recipm1 = __ldg(row + 1), c1 = __ldg(row + 2), c2 = __ldg(row + 3),
+              sig = __ldg(row + 4);
+  const float4* nz = noise ? reinterpret_cast<const float4*>(noise) + st * total4 : nullptr;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    const float sb = __ldg(s + b);
+    const float4 x = reinterpret_cast<const float4*>(img)[i];
+    const float4 e = reinterpret_cast<const float4*>(pred)[i];
+    const float4 z = nz ? nz[i]
+                        : normal4(__ldg(seeds + b), static_cast<unsigned int>(i - b * n4_per_sample),
+                                  static_cast<unsigned int>(st), kStreamStep);
+    float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, zv[4] = {z.x, z.y, z.z, z.w}, o[4], xs[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
+      v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+      xs[j] = v;
+      const float mean = __fadd_rn(__fmul_rn(c1, v), __fmul_rn(c2, xv[j]));
+      o[j] = __fadd_rn(mean, __fmul_rn(sig, zv[j]));       // added at t = 0 too (sig = 0): torch's signed zeros
+    }
+    reinterpret_cast<float4*>(img_out)[i] = make_float4(o[0], o[1], o[2], o[3]);
+    if (xs_out) reinterpret_cast<float4*>(xs_out)[i] = make_float4(xs[0], xs[1], xs[2], xs[3]);
+  }
+}
+
+__global__ void __launch_bounds__(256) ddpm_fill_normal_kernel(const long long* __restrict__ seeds,
+                                                               float* __restrict__ out, int n4_per_sample,
+                                                               long long total4) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    reinterpret_cast<float4*>(out)[i] =
+        normal4(__ldg(seeds + b), static_cast<unsigned int>(i - b * n4_per_sample), 0u, kStreamInit);
+  }
+}
+
+// out[b, :] = table[*step, :] for every sample: the time-conditioned rows of the step, shared by the whole batch.
+__global__ void __launch_bounds__(256) ddpm_broadcast_row_kernel(const float* __restrict__ table,
+                                                                 const int* __restrict__ step,
+                                                                 float* __restrict__ out, int n_row, long long total) {
+  const float* row = table + static_cast<long long>(__ldg(step)) * n_row;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x)
+    out[i] = __ldg(row + i % n_row);
+}
+
+// One block: step += 1, then time[:] = times[step] for the next iteration's time MLP.
+__global__ void __launch_bounds__(256) ddpm_advance_kernel(int* __restrict__ step, const long long* __restrict__ times,
+                                                           int n_steps, long long* __restrict__ time, int B) {
+  const int next = *step + 1;
+  __syncthreads();                                        // every thread has read the old value
+  if (threadIdx.x == 0) *step = next;
+  if (next < n_steps)
+    for (int b = threadIdx.x; b < B; b += blockDim.x) time[b] = times[next];
+}
+
 }  // namespace extdm
 
 using namespace extdm;
@@ -135,6 +264,70 @@ extern "C" int extdm_ddim_update(const float* img, const float* pred, const floa
   if (g > 148 * 8) g = 148 * 8;
   ddim_update_kernel<<<static_cast<int>(g), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       img, pred, noise, s, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out, x_start_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+static int ddpm_grid(long long total4) {
+  long long g = (total4 + 255) / 256;
+  return static_cast<int>(g > 148 * 8 ? 148 * 8 : g);
+}
+
+extern "C" int extdm_ddpm_threshold(const float* img, const float* pred, const float* rows, const int* step, float q,
+                                    float* s, int B, int n, void* stream) {
+  if (n < 2 || B < 1) {
+    extdm_set_error("ddpm_threshold: need n >= 2", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  ddpm_threshold_kernel<<<B, 1024, 0, static_cast<cudaStream_t>(stream)>>>(img, pred, rows, step, q, s, n);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_ddpm_update(const float* img, const float* pred, const float* rows, const int* step,
+                                 const long long* seeds, const float* noise, const float* s, float* img_out,
+                                 float* x_start_out, int B, int n, void* stream) {
+  if (n % 4 || B < 1 || (!noise && !seeds)) {
+    extdm_set_error("ddpm_update: need n % 4 == 0, B >= 1 and seeds or noise", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  ddpm_update_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      img, pred, rows, step, seeds, noise, s, img_out, x_start_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_ddpm_fill_normal(const long long* seeds, float* out, int B, int n, void* stream) {
+  if (n % 4 || B < 1) {
+    extdm_set_error("ddpm_fill_normal: elements per sample must be a multiple of 4", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  ddpm_fill_normal_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(seeds, out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_ddpm_advance(int* step, const long long* times, int n_steps, long long* time, int B,
+                                  void* stream) {
+  if (B < 1 || n_steps < 1) {
+    extdm_set_error("ddpm_advance: need B >= 1 and n_steps >= 1", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  ddpm_advance_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(step, times, n_steps, time, B);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_ddpm_broadcast_row(const float* table, const int* step, float* out, int B, int n, void* stream) {
+  if (B < 1 || n < 1) {
+    extdm_set_error("ddpm_broadcast_row: need B >= 1 and n >= 1", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total = static_cast<long long>(B) * n;
+  ddpm_broadcast_row_kernel<<<ddpm_grid((total + 3) / 4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      table, step, out, n, total);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

@@ -1,10 +1,12 @@
-"""GaussianDiffusion: DDIM(eta) sampler with dynamic thresholding on the CUDA kernels.
+"""GaussianDiffusion: DDIM(eta) and DDPM (ancestral) samplers with dynamic thresholding on the CUDA kernels.
 
 Mirrors model/BaseDM_adaptor/Diffusion.py: same constructor, the same 12 schedule buffers (so
-`load_state_dict(ckpt['diffusion'])` works, scripts/DM/valid.py:111-112), `sample()` / `ddim_sample()`.
-The whole sampling loop (UNet prologue + sampling_timesteps x (UNet step + threshold + update)) is
-captured once per shape into a CUDA graph and replayed.  Training paths (p_losses, q_sample) and the
-reference's broken ancestral sampler (SURVEY.md App. E10) are out of scope.
+`load_state_dict(ckpt['diffusion'])` works, scripts/DM/valid.py:111-112), `sample()` / `ddim_sample()` /
+`p_sample_loop()`.  sampling_timesteps < timesteps selects DDIM: the whole sampling loop (UNet prologue +
+sampling_timesteps x (UNet step + threshold + update)) is captured once per shape into a CUDA graph and replayed.
+sampling_timesteps == timesteps (or None) selects the ancestral sampler, whose loop is too long for one graph: ONE
+iteration is captured and replayed timesteps times, with its per-step values on the device.  Training paths
+(p_losses, q_sample) are out of scope.
 """
 import torch
 import torch.nn.functional as F
@@ -74,11 +76,10 @@ class GaussianDiffusion(nn.Module):
     # ------------------------------------------------------------------ sampling
     @torch.no_grad()
     def sample(self, x_cond, cond_fea, cond=None, cond_scale=1.0, batch_size=16, noise=None):
-        if not self.is_ddim_sampling:
-            raise NotImplementedError("the reference's ancestral sampler (p_sample_loop) raises TypeError "
-                                      "(Diffusion.py:169,186); only DDIM sampling is defined")
         B = x_cond.shape[0]
         shape = (B, 3, self.num_frames - x_cond.size(2), x_cond.shape[3], x_cond.shape[4])
+        if not self.is_ddim_sampling:
+            return self.p_sample_loop(x_cond, shape, cond_fea, noise=noise)
         return self.ddim_sample(x_cond, shape, cond_fea=cond_fea, cond=cond, cond_scale=cond_scale, noise=noise)
 
     @torch.no_grad()
@@ -144,3 +145,102 @@ class GaussianDiffusion(nn.Module):
             if trace is not None:
                 trace[-1].update(x_start=xs, s=s.clone(), img=r.x.clone())
         return r.x
+
+    # ------------------------------------------------------------------ DDPM (ancestral) sampler
+    def ddpm_schedule(self, device=None):
+        """(times, rows) of p_sample_loop: times (num_timesteps,) int64 running T-1 .. 0, rows (num_timesteps, 5) fp32
+        {sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod, posterior_mean_coef1, posterior_mean_coef2, sig}[t]
+        with sig = nonzero_mask * exp(0.5 * posterior_log_variance_clipped[t]), evaluated with the fp32 torch ops of
+        Diffusion.py:144-166,174-177 on `device` (default: the buffers' device)."""
+        dev = self.betas.device if device is None else torch.device(device)
+        times = torch.arange(self.num_timesteps - 1, -1, -1, dtype=torch.long, device=dev)
+
+        def take(name):
+            return getattr(self, name).to(dev)[times]
+
+        nonzero_mask = 1 - (times == 0).float()
+        sig = nonzero_mask * (0.5 * take("posterior_log_variance_clipped")).exp()
+        rows = torch.stack([take("sqrt_recip_alphas_cumprod"), take("sqrt_recipm1_alphas_cumprod"),
+                            take("posterior_mean_coef1"), take("posterior_mean_coef2"), sig], dim=1).contiguous()
+        return times, rows
+
+    @torch.no_grad()
+    def p_sample_loop(self, x_cond, shape, cond_fea, noise=None, trace=None):
+        """Ancestral sampling over all num_timesteps (Diffusion.py:136-189, with cond_fea and t passed by keyword:
+        SURVEY.md App. E10), clip_denoised=True with dynamic thresholding.  Returns the final img (no
+        un-normalisation, as ddim_sample).
+
+        noise: optional (num_timesteps + 1, *shape) tensor; noise[0] replaces x_T and noise[1 + i] the randn_like of
+        iteration i.  Default: Philox4x32-10 noise drawn inside the kernels, keyed by one seed per video that is taken
+        from torch's default generator on every call (so torch.manual_seed reproduces a run, and a video's noise
+        does not depend on its batch neighbours).  trace: list that receives per-step tensors (tests)."""
+        if not self.use_dynamic_thres:
+            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
+        if x_cond.device.type != "cuda":
+            raise RuntimeError("p_sample_loop runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        T, B, dev = self.num_timesteps, shape[0], x_cond.device
+        if noise is not None and tuple(noise.shape) != (T + 1, *shape):
+            raise ValueError(f"p_sample_loop: noise must have shape {(T + 1, *shape)}, got {tuple(noise.shape)}")
+        r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
+        seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long) if noise is None else None
+        if trace is not None or not self.use_cuda_graph:
+            st = self._ddpm_state(r, noise is not None)
+            self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
+            for _ in range(T):
+                self._ddpm_iteration(r, st, trace)
+            return r.x.clone()
+        # One iteration (time-MLP rows, UNet step, threshold, update, advance) is captured; its per-step values come from
+        # the device tables and step counter, so the same graph serves every timestep.  Like ddim_graphs it lives on the
+        # runner, whose buffers it points into.
+        graphs = r.ddpm_graphs
+        key = (tuple(shape), float(self.dynamic_thres_percentile), T, noise is not None)
+        if key not in graphs:
+            st = self._ddpm_state(r, noise is not None)
+            self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)           # warm-up (lazy inits)
+            self._ddpm_iteration(r, st)
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._ddpm_iteration(r, st)
+            graphs[key] = (g, st)
+        g, st = graphs[key]
+        self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
+        for _ in range(T):
+            g.replay()
+        return r.x.clone()
+
+    def _ddpm_state(self, r, injected):
+        """Device state of the loop: schedule table, time-MLP rows per step, step counter, per-video seeds,
+        thresholds, injected noise."""
+        times, rows = self.ddpm_schedule(r.dev)
+        return dict(times=times, rows=rows, ss_rows=r.ss_rows_for_times(range(self.num_timesteps - 1, -1, -1)),
+                    step=torch.zeros(1, dtype=torch.int32, device=r.dev),
+                    seeds=torch.zeros(r.B, dtype=torch.long, device=r.dev), s=torch.zeros(r.B, device=r.dev),
+                    noise=torch.zeros(self.num_timesteps, *r.x.shape, device=r.dev) if injected else None)
+
+    def _ddpm_round(self, r, st, x_cond, cond_fea, seeds, noise):
+        """Once per round, before the iterations: conditioning, UNet prologue, x_T, step counter and time reset."""
+        r.set_conditioning(x_cond.float(), cond_fea.float())
+        r.run_prologue()
+        if noise is None:
+            st["seeds"].copy_(seeds.pin_memory(), non_blocking=True)      # no host sync before the replays
+            ops.ddpm_fill_normal(ops.IMMEDIATE, st["seeds"], r.x)
+        else:
+            r.x.copy_(noise[0])
+            st["noise"].copy_(noise[1:])
+        st["step"].zero_()
+        r.time.fill_(self.num_timesteps - 1)
+
+    def _ddpm_iteration(self, r, st, trace=None):
+        rec = ops.IMMEDIATE
+        ops.ddpm_broadcast_row(rec, st["ss_rows"], st["step"], r.ss)      # this step's time-MLP rows
+        r.step.run()
+        ops.ddpm_threshold(rec, r.x, r.out, st["rows"], st["step"], float(self.dynamic_thres_percentile), st["s"])
+        xs = None
+        if trace is not None:
+            xs = torch.empty_like(r.x)
+            trace.append(dict(img_in=r.x.clone(), pred_noise=r.out.clone()))
+        ops.ddpm_update(rec, r.x, r.out, st["rows"], st["step"], st["seeds"], st["noise"], st["s"], r.x, xs)
+        if trace is not None:
+            trace[-1].update(x_start=xs, s=st["s"].clone(), img=r.x.clone())
+        ops.ddpm_advance(rec, st["step"], st["times"], r.time)

@@ -77,6 +77,11 @@ PROTOTYPES = {
     "extdm_temporal_attention": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P],
     "extdm_ddim_threshold": [_P, _P, _F, _F, _F, _P, _I, _I, _P],
     "extdm_ddim_update": [_P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _I, _I, _P],
+    "extdm_ddpm_threshold": [_P, _P, _P, _P, _F, _P, _I, _I, _P],
+    "extdm_ddpm_update": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P],
+    "extdm_ddpm_fill_normal": [_P, _P, _I, _I, _P],
+    "extdm_ddpm_broadcast_row": [_P, _P, _P, _I, _I, _P],
+    "extdm_ddpm_advance": [_P, _P, _I, _P, _I, _P],
     "extdm_warp_blend_cl": [_P, _P, _P, _P, _P, _L, _L, _I, _I, _I, _I, _I, _I, _P],
     "extdm_warp_image": [_P, _P, _I, _P, _P, _P, _P, _L, _L, _I, _I, _I, _I, _P],
     "extdm_warp_taps": [_P, _P, _P, _P, _P, _L, _I, _I, _I, _I, _P],

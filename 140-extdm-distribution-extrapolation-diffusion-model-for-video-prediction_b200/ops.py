@@ -532,6 +532,55 @@ def ddim_update(rec, img, pred, noise, s, c_recip, c_recipm1, sqrt_alpha_next, c
              keep=(img, pred, noise, s, img_out, x_start_out))
 
 
+def ddpm_threshold(rec, img, pred, rows, step, q, s):
+    """As ddim_threshold, with (c_recip, c_recipm1) read from rows[step] on the device."""
+    _chk(rows, torch.float32, "rows")
+    _chk(step, torch.int32, "step")
+    B = img.shape[0]
+    rec.emit("extdm_ddpm_threshold", (_p(img), _p(pred), _p(rows), _p(step), C.c_float(q), _p(s), B, img.numel() // B),
+             keep=(img, pred, rows, step, s))
+
+
+def ddpm_update(rec, img, pred, rows, step, seeds, noise, s, img_out, x_start_out=None):
+    """One ancestral step with the coefficients of rows[step]; noise (n_steps, *img.shape) or None (Philox of seeds)."""
+    _chk(rows, torch.float32, "rows")
+    _chk(step, torch.int32, "step")
+    _chk(seeds, torch.int64, "seeds")
+    _chk(noise, torch.float32, "noise")
+    B = img.shape[0]
+    rec.emit("extdm_ddpm_update", (_p(img), _p(pred), _p(rows), _p(step), _p(seeds), _p(noise), _p(s), _p(img_out),
+                                   _p(x_start_out), B, img.numel() // B),
+             keep=(img, pred, rows, step, seeds, noise, s, img_out, x_start_out))
+
+
+def ddpm_fill_normal(rec, seeds, out):
+    """out[b] = the x_T draw of video seed seeds[b]."""
+    _chk(seeds, torch.int64, "seeds")
+    _chk(out, torch.float32, "out")
+    B = out.shape[0]
+    rec.emit("extdm_ddpm_fill_normal", (_p(seeds), _p(out), B, out.numel() // B), keep=(seeds, out))
+
+
+def ddpm_broadcast_row(rec, table, step, out):
+    """out[b] = table[step] for every row b of out."""
+    _chk(table, torch.float32, "table")
+    _chk(step, torch.int32, "step")
+    _chk(out, torch.float32, "out")
+    if table.shape[-1] != out.shape[-1]:
+        raise ValueError(f"ddpm_broadcast_row: rows of {table.shape[-1]} and {out.shape[-1]} floats")
+    rec.emit("extdm_ddpm_broadcast_row", (_p(table), _p(step), _p(out), out.shape[0], out.shape[-1]),
+             keep=(table, step, out))
+
+
+def ddpm_advance(rec, step, times, time):
+    """step += 1; time[:] = times[step] (while step < len(times))."""
+    _chk(step, torch.int32, "step")
+    _chk(times, torch.int64, "times")
+    _chk(time, torch.int64, "time")
+    rec.emit("extdm_ddpm_advance", (_p(step), _p(times), times.numel(), _p(time), time.numel()),
+             keep=(step, times, time))
+
+
 # ----------------------------------------------------------------------------- LFAE decode
 def warp_blend_cl(rec, skip, prev, flow, occ, out, up2=False):
     """skip (Fs,H,W,C) bf16, prev (F,H,W,C) or None, flow (F,h,w,2) fp32, occ (F,1,h,w) fp32 or None."""

@@ -171,8 +171,10 @@ class UnetRunner:
         # sampler evaluates it once per schedule (ss_for_times) instead of once per DDIM step and round
         self.time_rec = ops.Recorder(record=True)
         self._ss_tables = {}
+        self._ss_rows = {}
         self.taps = {}                      # name -> buffer, for layer-by-layer parity tests
         self.ddim_graphs = {}               # CUDA graphs of the sampling loop over these buffers (GaussianDiffusion)
+        self.ddpm_graphs = {}               # CUDA graphs of one ancestral-sampler iteration (GaussianDiffusion)
         self._build()
 
     # ------------------------------------------------------------------ helpers
@@ -665,6 +667,20 @@ class UnetRunner:
                 rows.append(self.ss.clone())
             self._ss_tables[key] = torch.stack(rows)
         return self._ss_tables[key]
+
+    def ss_rows_for_times(self, times):
+        """(len(times), n_ss): as ss_for_times, one row per timestep instead of B identical ones (each sample's rows
+        are computed independently, so row 0 is every sample's row), cached per schedule.  The ancestral sampler
+        broadcasts row `step` into self.ss on the device (ops.ddpm_broadcast_row)."""
+        key = tuple(int(t) for t in times)
+        if key not in self._ss_rows:
+            rows = torch.empty(len(key), self.pk.n_ss, device=self.dev)
+            for i, t in enumerate(key):
+                self.time.fill_(t)
+                self.time_rec.run()
+                rows[i].copy_(self.ss[0])
+            self._ss_rows[key] = rows
+        return self._ss_rows[key]
 
 
 class Unet3D(ParamTree):

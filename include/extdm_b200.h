@@ -279,6 +279,36 @@ int extdm_ddim_update(const float* img, const float* pred, const float* noise, c
                       float* x_start_out, int B, int n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * DDPM ancestral sampler (GaussianDiffusion.p_sample_loop, model/BaseDM_adaptor/Diffusion.py:136-189 with the
+ * keyword fix of SURVEY App. E10), fp32.  Added under ABI version 5 (backward compatible).
+ *
+ * Per-step values live on the device so that one captured iteration replays for every timestep:
+ *   rows  (n_steps, 5) fp32: {sqrt_recip_alphas_cumprod, sqrt_recipm1_alphas_cumprod, posterior_mean_coef1,
+ *                             posterior_mean_coef2, nonzero_mask * exp(0.5 * posterior_log_variance_clipped)}[times[i]]
+ *   step  one int32, the current row; seeds (B,) int64, one per video.
+ * Noise is Philox4x32-10 + Box-Muller with key = the video's seed and counter = (element index / 4 within the video,
+ * step, stream, 0); stream 0 is the noise of loop step `step`, stream 1 the initial x_T.
+ */
+
+/* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
+ * extdm_ddim_threshold). */
+int extdm_ddpm_threshold(const float* img, const float* pred, const float* rows, const int* step, float q, float* s,
+                         int B, int n, void* stream);
+/* x0 = clamp(c_recip*img - c_recipm1*pred, -s, s)/s; img_out = (c1*x0 + c2*img) + sig*z with row *step.  z is slice
+ * *step of `noise` ((n_steps, B, n)) when noise != NULL, else the Philox draw of (seeds[b], *step).  x_start_out
+ * (optional) receives x0. */
+int extdm_ddpm_update(const float* img, const float* pred, const float* rows, const int* step, const long long* seeds,
+                      const float* noise, const float* s, float* img_out, float* x_start_out, int B, int n,
+                      void* stream);
+/* out (B, n) = the x_T draw (stream 1) of each video's seed. */
+int extdm_ddpm_fill_normal(const long long* seeds, float* out, int B, int n, void* stream);
+/* out (B, n) = row *step of table (n_steps, n) for every b: the per-step time-MLP (scale, shift) rows, which do not
+ * depend on the sample. */
+int extdm_ddpm_broadcast_row(const float* table, const int* step, float* out, int B, int n, void* stream);
+/* *step += 1; time[0..B) = times[*step] while *step < n_steps (one block). */
+int extdm_ddpm_advance(int* step, const long long* times, int n_steps, long long* time, int B, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * LFAE decode (Generator.forward_with_flow / deform_input / apply_optical, model/LFAE/generator.py:63-93,
  * 152-206).  flow: (F, h, w, 2) fp32 normalised (x, y); occ: (F, 1, h, w) fp32 or NULL.
  */
