@@ -73,17 +73,25 @@ def build_model(name, seed=1234, device="cuda"):
     return model.to(device), cfg
 
 
-def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None):
+def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None, seeds=None):
     """Autoregressive rollout of scripts/DM/valid.py:167-172 -> (B, 3, total_pred, H, W).
     host_buffers=None keeps every round on the device (SURVEY.md section 8f-2).  With
     host_buffers=(pinned_in, pinned_out) each round copies its conditioning clip host->device and its
-    sample_out_vid device->host exactly like the reference driver (`.cuda()` / `.cpu()` per round)."""
+    sample_out_vid device->host exactly like the reference driver (`.cuda()` / `.cpu()` per round).
+    seeds: optional per-video base seeds ((B,) int64 tensor or list); round r samples video b with the seed
+    sharding.video_seeds(seeds[b], 0, r), so every round draws fresh noise and a video's rollout depends on its own
+    base seed only."""
     import math
     import torch
+    from .sharding import video_seeds
+    if seeds is not None and noise_fn is not None:
+        raise ValueError("rollout: pass noise_fn or seeds, not both")
+    if seeds is not None and len(seeds) != clip.shape[0]:
+        raise ValueError(f"rollout: {len(seeds)} seeds for {clip.shape[0]} videos")
     tc, tp = model.cond_frame_num, model.pred_frame_num
     preds = []
     cond = clip
-    for _ in range(math.ceil(total_pred / tp)):
+    for r in range(math.ceil(total_pred / tp)):
         if host_buffers is not None:
             pin_in, pin_out = host_buffers
             pin_in.copy_(cond)                                   # host -> pinned staging (host memcpy)
@@ -91,7 +99,8 @@ def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None):
         else:
             dev_in = cond
         out = model.sample_one_video(cond_scale=1.0, real_vid=dev_in,
-                                     noise=None if noise_fn is None else noise_fn())["sample_out_vid"]
+                                     noise=None if noise_fn is None else noise_fn(),
+                                     seeds=None if seeds is None else video_seeds(seeds, 0, r))["sample_out_vid"]
         if host_buffers is not None:
             pin_out.copy_(out, non_blocking=True)
             torch.cuda.current_stream().synchronize()

@@ -4,6 +4,7 @@
 // neighbouring order statistics instead of a full sort.
 // The DDPM ancestral step (GaussianDiffusion.p_sample_loop) shares that select; its per-step coefficients, step index and
 // Philox noise live on the device, so one captured iteration can be replayed for every timestep.
+// DDIM with per-video seeds draws its noise from the same Philox generator inside the update.
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -89,6 +90,26 @@ __global__ void __launch_bounds__(1024) ddim_threshold_kernel(const float* __res
   threshold_sample(img, pred, c_recip, c_recipm1, q, s_out, n);
 }
 
+// Four elements of one DDIM step: x0 = clamp(c_recip*img - c_recipm1*pred, -s, s)/s;
+// out = (x0*sqrt_alpha_next + c*pred) + sigma*z, op by op (no FMA), the sigma*z term only when with_noise.
+// Shared by the kernel that reads z from a noise tensor and the one that draws it with Philox.
+__device__ __forceinline__ void ddim_quad(float4 x, float4 e, float4 z, bool with_noise, float sb, float c_recip,
+                                          float c_recipm1, float sqrt_alpha_next, float c, float sigma,
+                                          float* __restrict__ img_out, float* __restrict__ xs_out, long long i) {
+  float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, zv[4] = {z.x, z.y, z.z, z.w}, o[4], xs[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
+    v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+    xs[j] = v;
+    float r = __fadd_rn(__fmul_rn(v, sqrt_alpha_next), __fmul_rn(c, ev[j]));
+    if (with_noise) r = __fadd_rn(r, __fmul_rn(sigma, zv[j]));
+    o[j] = r;
+  }
+  reinterpret_cast<float4*>(img_out)[i] = make_float4(o[0], o[1], o[2], o[3]);
+  if (xs_out) reinterpret_cast<float4*>(xs_out)[i] = make_float4(xs[0], xs[1], xs[2], xs[3]);
+}
+
 __global__ void __launch_bounds__(256) ddim_update_kernel(const float* __restrict__ img,
                                                           const float* __restrict__ pred,
                                                           const float* __restrict__ noise,
@@ -103,18 +124,7 @@ __global__ void __launch_bounds__(256) ddim_update_kernel(const float* __restric
     const float4 e = reinterpret_cast<const float4*>(pred)[i];
     float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
     if (noise) z = reinterpret_cast<const float4*>(noise)[i];
-    float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, zv[4] = {z.x, z.y, z.z, z.w}, o[4], xs[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
-      v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
-      xs[j] = v;
-      float r = __fadd_rn(__fmul_rn(v, sqrt_alpha_next), __fmul_rn(c, ev[j]));
-      if (noise) r = __fadd_rn(r, __fmul_rn(sigma, zv[j]));
-      o[j] = r;
-    }
-    reinterpret_cast<float4*>(img_out)[i] = make_float4(o[0], o[1], o[2], o[3]);
-    if (xs_out) reinterpret_cast<float4*>(xs_out)[i] = make_float4(xs[0], xs[1], xs[2], xs[3]);
+    ddim_quad(x, e, z, noise != nullptr, sb, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out, xs_out, i);
   }
 }
 
@@ -217,6 +227,29 @@ __global__ void __launch_bounds__(256) ddpm_fill_normal_kernel(const long long* 
   }
 }
 
+// DDIM step whose z is the Philox draw of (seeds[b], step, stream 0), the generator of ddpm_update_kernel: a video's
+// noise depends on its own seed only.  Step i of the DDIM loop uses step = i; x_T is ddpm_fill_normal (stream 1).
+__global__ void __launch_bounds__(256) ddim_update_seeded_kernel(const float* __restrict__ img,
+                                                                 const float* __restrict__ pred,
+                                                                 const long long* __restrict__ seeds,
+                                                                 unsigned int step, const float* __restrict__ s,
+                                                                 float c_recip, float c_recipm1,
+                                                                 float sqrt_alpha_next, float c, float sigma,
+                                                                 float* __restrict__ img_out,
+                                                                 float* __restrict__ xs_out, int n4_per_sample,
+                                                                 long long total4) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    const float sb = __ldg(s + b);
+    const float4 x = reinterpret_cast<const float4*>(img)[i];
+    const float4 e = reinterpret_cast<const float4*>(pred)[i];
+    const float4 z =
+        normal4(__ldg(seeds + b), static_cast<unsigned int>(i - b * n4_per_sample), step, kStreamStep);
+    ddim_quad(x, e, z, true, sb, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out, xs_out, i);
+  }
+}
+
 // out[b, :] = table[*step, :] for every sample: the time-conditioned rows of the step, shared by the whole batch.
 __global__ void __launch_bounds__(256) ddpm_broadcast_row_kernel(const float* __restrict__ table,
                                                                  const int* __restrict__ step,
@@ -271,6 +304,22 @@ extern "C" int extdm_ddim_update(const float* img, const float* pred, const floa
 static int ddpm_grid(long long total4) {
   long long g = (total4 + 255) / 256;
   return static_cast<int>(g > 148 * 8 ? 148 * 8 : g);
+}
+
+extern "C" int extdm_ddim_update_seeded(const float* img, const float* pred, const long long* seeds, int step,
+                                        const float* s, float c_recip, float c_recipm1, float sqrt_alpha_next,
+                                        float c, float sigma, float* img_out, float* x_start_out, int B, int n,
+                                        void* stream) {
+  if (n % 4 || B < 1 || !seeds || step < 0) {
+    extdm_set_error("ddim_update_seeded: need n % 4 == 0, B >= 1, seeds and step >= 0", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  ddim_update_seeded_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      img, pred, seeds, static_cast<unsigned int>(step), s, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out,
+      x_start_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
 }
 
 extern "C" int extdm_ddpm_threshold(const float* img, const float* pred, const float* rows, const int* step, float q,

@@ -4,6 +4,8 @@ Mirrors model/BaseDM_adaptor/Diffusion.py: same constructor, the same 12 schedul
 `load_state_dict(ckpt['diffusion'])` works, scripts/DM/valid.py:111-112), `sample()` / `ddim_sample()` /
 `p_sample_loop()`.  sampling_timesteps < timesteps selects DDIM: the whole sampling loop (UNet prologue +
 sampling_timesteps x (UNet step + threshold + update)) is captured once per shape into a CUDA graph and replayed.
+With `seeds` (one int64 per video) DDIM draws its noise inside the update kernel from a Philox stream keyed by the
+video's seed, so a video's sample does not depend on the rest of its batch and no noise tensor is stored.
 sampling_timesteps == timesteps (or None) selects the ancestral sampler, whose loop is too long for one graph: ONE
 iteration is captured and replayed timesteps times, with its per-step values on the device.  Training paths
 (p_losses, q_sample) are out of scope.
@@ -13,6 +15,29 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
+
+
+def _seed_vector(seeds, noise, B, who):
+    """Validate the per-video seeds of a sampler call: None, or a (B,) int64 tensor (any device) or a list of ints."""
+    if seeds is None:
+        return None
+    if noise is not None:
+        raise ValueError(f"{who}: pass noise or seeds, not both")
+    if not torch.is_tensor(seeds):
+        try:
+            seeds = torch.tensor(list(seeds))
+        except (TypeError, RuntimeError, OverflowError) as e:
+            raise ValueError(f"{who}: seeds must be int64 values ({e})") from None
+    if seeds.dtype != torch.int64:
+        raise ValueError(f"{who}: seeds must be int64, got {seeds.dtype}")
+    if tuple(seeds.shape) != (B,):
+        raise ValueError(f"{who}: need one seed per video, shape ({B},), got {tuple(seeds.shape)}")
+    return seeds
+
+
+def _load_seeds(dst, seeds):
+    """dst (device) <- seeds without a host synchronisation: host seeds go through pinned memory."""
+    dst.copy_(seeds.pin_memory() if seeds.device.type == "cpu" else seeds, non_blocking=True)
 
 
 def _schedule_tables(timesteps, s=0.008):
@@ -75,26 +100,34 @@ class GaussianDiffusion(nn.Module):
 
     # ------------------------------------------------------------------ sampling
     @torch.no_grad()
-    def sample(self, x_cond, cond_fea, cond=None, cond_scale=1.0, batch_size=16, noise=None):
+    def sample(self, x_cond, cond_fea, cond=None, cond_scale=1.0, batch_size=16, noise=None, seeds=None):
+        """seeds: optional (B,) int64 tensor or list, one seed per video (see ddim_sample / p_sample_loop)."""
         B = x_cond.shape[0]
         shape = (B, 3, self.num_frames - x_cond.size(2), x_cond.shape[3], x_cond.shape[4])
         if not self.is_ddim_sampling:
-            return self.p_sample_loop(x_cond, shape, cond_fea, noise=noise)
-        return self.ddim_sample(x_cond, shape, cond_fea=cond_fea, cond=cond, cond_scale=cond_scale, noise=noise)
+            return self.p_sample_loop(x_cond, shape, cond_fea, noise=noise, seeds=seeds)
+        return self.ddim_sample(x_cond, shape, cond_fea=cond_fea, cond=cond, cond_scale=cond_scale, noise=noise,
+                                seeds=seeds)
 
     @torch.no_grad()
     def ddim_sample(self, x_cond, shape, cond_fea, cond=None, cond_scale=1.0, clip_denoised=True, noise=None,
-                    trace=None):
+                    trace=None, seeds=None):
         """noise: optional (n_steps, B, 3, tp, h, w) tensor; noise[0] replaces the initial torch.randn and
         noise[i] (i >= 1) the randn_like of iteration i-1 (Diffusion.py:218, 251).  Default: torch.randn on the
-        device, in the reference's draw order.  trace: list that receives per-step tensors (tests)."""
+        device, in the reference's draw order.  seeds: optional (B,) int64 tensor or list, one per video, instead of
+        noise: x_T and the noise of iteration i are the Philox draws of the video's seed (stream 1, and step i of
+        stream 0: include/extdm_b200.h), made inside the kernels, so video b's sample depends on seeds[b] only and
+        no noise tensor is stored.  trace: list that receives per-step tensors (tests)."""
+        B = shape[0]
+        seeds = _seed_vector(seeds, noise, B, "ddim_sample")
         if not clip_denoised or not self.use_dynamic_thres:
             raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
         unet = self.denoise_fn
-        B = shape[0]
         dev = x_cond.device
         sched = self.ddim_schedule()
         r = unet.runner(B, shape[3], shape[4], cond_fea.shape[-1])
+        if seeds is not None:
+            return self._ddim_seeded(r, sched, shape, x_cond, cond_fea, seeds, trace)
         if noise is None:
             noise = torch.empty(len(sched), *shape, device=dev)
             noise[0] = torch.randn(shape, device=dev)
@@ -106,8 +139,7 @@ class GaussianDiffusion(nn.Module):
         # Unet3D.invalidate() (load_state_dict, device move) drops runner and graphs together.  The schedule scalars are
         # baked into the capture, hence part of the key.
         graphs = r.ddim_graphs
-        key = (tuple(shape), float(self.ddim_sampling_eta), float(self.dynamic_thres_percentile),
-               int(self.sampling_timesteps), int(self.num_timesteps))
+        key = self._ddim_key(shape)
         if key not in graphs:
             st = dict(noise=torch.zeros_like(noise), s=torch.zeros(B, device=dev))
             st["x_cond"], st["cond_fea"] = r.cond_frames, r.cond_fea
@@ -123,25 +155,67 @@ class GaussianDiffusion(nn.Module):
         g.replay()
         return r.x.clone()
 
+    def _ddim_key(self, shape):
+        return (tuple(shape), float(self.ddim_sampling_eta), float(self.dynamic_thres_percentile),
+                int(self.sampling_timesteps), int(self.num_timesteps))
+
+    def _ddim_seeded(self, r, sched, shape, x_cond, cond_fea, seeds, trace):
+        """ddim_sample with per-video seeds.  The graph reads the seeds from a device buffer of its state (there is
+        no noise buffer), so one capture serves every seed vector; each call only copies the seeds in."""
+        def state():
+            return dict(seeds=torch.zeros(r.B, dtype=torch.long, device=r.dev), s=torch.zeros(r.B, device=r.dev))
+        if trace is not None or not self.use_cuda_graph:
+            st = state()
+            _load_seeds(st["seeds"], seeds)
+            return self._run_loop(r, sched, x_cond, cond_fea, None, trace, st).clone()
+        graphs = r.ddim_graphs
+        key = self._ddim_key(shape) + (("seeded", True),)
+        if key not in graphs:
+            st = state()
+            _load_seeds(st["seeds"], seeds)
+            st["x_cond"], st["cond_fea"] = r.cond_frames, r.cond_fea
+            self._run_loop(r, sched, x_cond, cond_fea, None, None, st)            # warm-up (lazy inits)
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._run_loop(r, sched, None, None, None, None, st)
+            graphs[key] = (g, st)
+        g, st = graphs[key]
+        r.set_conditioning(x_cond.float(), cond_fea.float())
+        _load_seeds(st["seeds"], seeds)                                           # no host sync before the replay
+        g.replay()
+        return r.x.clone()
+
     def _run_loop(self, r, sched, x_cond, cond_fea, noise, trace, st=None):
+        """The DDIM loop.  Its noise is noise[0] (x_T) and noise[i + 1] (iteration i), or, when st holds "seeds", the
+        Philox draws of those seeds."""
         if x_cond is not None:
             r.set_conditioning(x_cond.float(), cond_fea.float())
         s = st["s"] if st is not None else torch.zeros(r.B, device=r.dev)
+        seeds = st.get("seeds") if st is not None else None
         rec = ops.IMMEDIATE
         r.run_prologue()
-        r.x.copy_(noise[0])
+        if seeds is not None:
+            ops.ddpm_fill_normal(rec, seeds, r.x)
+        else:
+            r.x.copy_(noise[0])
         q = float(self.dynamic_thres_percentile)
         ss = r.ss_for_times([s_[0] for s_ in sched])       # evaluated once per schedule, outside the captured loop
         for i, (time, time_next, c_recip, c_recipm1, san, c, sigma) in enumerate(sched):
             r.run_step(ss[i])
             ops.ddim_threshold(rec, r.x, r.out, c_recip, c_recipm1, q, s)
-            nz = noise[i + 1] if (time_next > 0 and i + 1 < noise.shape[0]) else None
-            if time_next > 0 and nz is None:
-                raise ValueError("ddim_sample: not enough noise tensors supplied")
+            nz = None
+            if seeds is None:
+                nz = noise[i + 1] if (time_next > 0 and i + 1 < noise.shape[0]) else None
+                if time_next > 0 and nz is None:
+                    raise ValueError("ddim_sample: not enough noise tensors supplied")
             xs = torch.empty_like(r.x) if trace is not None else None
             if trace is not None:
                 trace.append(dict(img_in=r.x.clone(), pred_noise=r.out.clone()))
-            ops.ddim_update(rec, r.x, r.out, nz, s, c_recip, c_recipm1, san, c, sigma, r.x, xs)
+            if seeds is not None and time_next > 0:
+                ops.ddim_update_seeded(rec, r.x, r.out, seeds, i, s, c_recip, c_recipm1, san, c, sigma, r.x, xs)
+            else:
+                ops.ddim_update(rec, r.x, r.out, nz, s, c_recip, c_recipm1, san, c, sigma, r.x, xs)
             if trace is not None:
                 trace[-1].update(x_start=xs, s=s.clone(), img=r.x.clone())
         return r.x
@@ -165,7 +239,7 @@ class GaussianDiffusion(nn.Module):
         return times, rows
 
     @torch.no_grad()
-    def p_sample_loop(self, x_cond, shape, cond_fea, noise=None, trace=None):
+    def p_sample_loop(self, x_cond, shape, cond_fea, noise=None, trace=None, seeds=None):
         """Ancestral sampling over all num_timesteps (Diffusion.py:136-189, with cond_fea and t passed by keyword:
         SURVEY.md App. E10), clip_denoised=True with dynamic thresholding.  Returns the final img (no
         un-normalisation, as ddim_sample).
@@ -173,7 +247,9 @@ class GaussianDiffusion(nn.Module):
         noise: optional (num_timesteps + 1, *shape) tensor; noise[0] replaces x_T and noise[1 + i] the randn_like of
         iteration i.  Default: Philox4x32-10 noise drawn inside the kernels, keyed by one seed per video that is taken
         from torch's default generator on every call (so torch.manual_seed reproduces a run, and a video's noise
-        does not depend on its batch neighbours).  trace: list that receives per-step tensors (tests)."""
+        does not depend on its batch neighbours).  seeds: optional (B,) int64 tensor or list that replaces those
+        drawn seeds.  trace: list that receives per-step tensors (tests)."""
+        seeds = _seed_vector(seeds, noise, shape[0], "p_sample_loop")
         if not self.use_dynamic_thres:
             raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
         if x_cond.device.type != "cuda":
@@ -182,7 +258,8 @@ class GaussianDiffusion(nn.Module):
         if noise is not None and tuple(noise.shape) != (T + 1, *shape):
             raise ValueError(f"p_sample_loop: noise must have shape {(T + 1, *shape)}, got {tuple(noise.shape)}")
         r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
-        seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long) if noise is None else None
+        if noise is None and seeds is None:
+            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
         if trace is not None or not self.use_cuda_graph:
             st = self._ddpm_state(r, noise is not None)
             self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
@@ -223,7 +300,7 @@ class GaussianDiffusion(nn.Module):
         r.set_conditioning(x_cond.float(), cond_fea.float())
         r.run_prologue()
         if noise is None:
-            st["seeds"].copy_(seeds.pin_memory(), non_blocking=True)      # no host sync before the replays
+            _load_seeds(st["seeds"], seeds)                                # no host sync before the replays
             ops.ddpm_fill_normal(ops.IMMEDIATE, st["seeds"], r.x)
         else:
             r.x.copy_(noise[0])

@@ -33,22 +33,31 @@ def load_dm_checkpoint(model, ckpt):
 
 
 @torch.no_grad()
-def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=True):
+def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=True, seed=None, video_offset=0):
     """valid.py:156-197 for one batch: real_vids (B, C, T, H, W) in [0,1] with T >= cond frames (+ total_pred ground
     truth frames if available) -> (origin, result), both (B, n, T', C, H, W) on the CPU, result = cond frames followed
-    by total_pred predicted frames.  on_device=False reproduces the reference's per-round .cpu()/.cuda() hops."""
+    by total_pred predicted frames.  on_device=False reproduces the reference's per-round .cpu()/.cuda() hops.
+
+    seed: optional int.  Then repeat k of video b is sampled with the per-video base seed
+    sharding.video_seeds(seed, (video_offset + b) * num_sample_video + k), a function of its *global* index only:
+    a sharded evaluation passes video_offset = lo of sharding.shard_range and samples every video with the same noise
+    as a single-GPU run.  Default: the sampler's own noise (torch's default generator)."""
     from .configs import rollout
+    from .sharding import video_seeds
     tc = model.cond_frame_num
     dev = next(model.parameters()).device
     B = real_vids.shape[0]
     rep = real_vids.repeat_interleave(num_sample_video, dim=0)                     # 'b c t h w -> (b n) c t h w'
     cond = rep[:, :, :tc].to(dev).float().contiguous()
+    seeds = None
+    if seed is not None:                                                            # row b*n + k of rep = (b, k)
+        seeds = video_seeds(seed, torch.arange(B * num_sample_video) + video_offset * num_sample_video)
     if on_device:
-        pred = rollout(model, cond, total_pred)
+        pred = rollout(model, cond, total_pred, seeds=seeds)
     else:
         pin_in = torch.empty(cond.shape).pin_memory()
         pin_out = torch.empty(cond.shape[0], cond.shape[1], tc + model.pred_frame_num, *cond.shape[3:]).pin_memory()
-        pred = rollout(model, cond.cpu(), total_pred, host_buffers=(pin_in, pin_out))
+        pred = rollout(model, cond.cpu(), total_pred, host_buffers=(pin_in, pin_out), seeds=seeds)
     res = torch.cat([rep[:, :, :tc].cpu().float(), pred.cpu()], dim=2)
 
     def shape(t):                                                                   # '(b n) c t h w -> b n t c h w'

@@ -170,9 +170,11 @@ class FlowDiffusion(nn.Module):
 
     # ------------------------------------------------------------------ full round
     @torch.no_grad()
-    def sample_one_video(self, cond_scale, real_vid, noise=None):
+    def sample_one_video(self, cond_scale, real_vid, noise=None, seeds=None):
+        """seeds: optional (B,) int64 tensor or list, one sampler seed per video (GaussianDiffusion.sample)."""
         ret, x_cond, cond_fea, ref = self.condition(real_vid)
-        pred = self.diffusion.sample(x_cond, cond_fea=cond_fea, batch_size=1, cond_scale=cond_scale, noise=noise)
+        pred = self.diffusion.sample(x_cond, cond_fea=cond_fea, batch_size=1, cond_scale=cond_scale, noise=noise,
+                                     seeds=seeds)
         tc = self.cond_frame_num
         grid = pred[:, :2]
         if self.use_residual_flow:

@@ -77,6 +77,7 @@ PROTOTYPES = {
     "extdm_temporal_attention": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P],
     "extdm_ddim_threshold": [_P, _P, _F, _F, _F, _P, _I, _I, _P],
     "extdm_ddim_update": [_P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _I, _I, _P],
+    "extdm_ddim_update_seeded": [_P, _P, _P, _I, _P, _F, _F, _F, _F, _F, _P, _P, _I, _I, _P],
     "extdm_ddpm_threshold": [_P, _P, _P, _P, _F, _P, _I, _I, _P],
     "extdm_ddpm_update": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P],
     "extdm_ddpm_fill_normal": [_P, _P, _I, _I, _P],

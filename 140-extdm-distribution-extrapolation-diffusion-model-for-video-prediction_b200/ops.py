@@ -532,6 +532,24 @@ def ddim_update(rec, img, pred, noise, s, c_recip, c_recipm1, sqrt_alpha_next, c
              keep=(img, pred, noise, s, img_out, x_start_out))
 
 
+def ddim_update_seeded(rec, img, pred, seeds, step, s, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out,
+                       x_start_out=None):
+    """ddim_update with sigma * z, z the Philox draw of (seeds[b], step) (the generator of ddpm_update)."""
+    if seeds is None:
+        raise ValueError("ddim_update_seeded: seeds are required")
+    _chk(seeds, torch.int64, "seeds")
+    B = img.shape[0]
+    if seeds.numel() != B or seeds.device != img.device:
+        raise ValueError(f"ddim_update_seeded: seeds must be {B} int64 on {img.device}, got {seeds.numel()} on "
+                         f"{seeds.device}")
+    if (img.numel() // B) % 4:
+        raise ValueError("ddim_update_seeded: elements per sample must be a multiple of 4")
+    rec.emit("extdm_ddim_update_seeded", (_p(img), _p(pred), _p(seeds), int(step), _p(s), C.c_float(c_recip),
+                                          C.c_float(c_recipm1), C.c_float(sqrt_alpha_next), C.c_float(c),
+                                          C.c_float(sigma), _p(img_out), _p(x_start_out), B, img.numel() // B),
+             keep=(img, pred, seeds, s, img_out, x_start_out))
+
+
 def ddpm_threshold(rec, img, pred, rows, step, q, s):
     """As ddim_threshold, with (c_recip, c_recipm1) read from rows[step] on the device."""
     _chk(rows, torch.float32, "rows")

@@ -277,6 +277,16 @@ int extdm_ddim_threshold(const float* img, const float* pred, float c_recip, flo
 int extdm_ddim_update(const float* img, const float* pred, const float* noise, const float* s, float c_recip,
                       float c_recipm1, float sqrt_alpha_next, float c, float sigma, float* img_out,
                       float* x_start_out, int B, int n, void* stream);
+/* As extdm_ddim_update, with z drawn inside the kernel instead of read from a noise tensor: the Philox draw of
+ * (seeds[b], step, stream 0) documented with the DDPM sampler below, so a video's noise depends on its seed only.
+ * Iteration i of the DDIM loop passes step = i (counter (element index / 4 within the video, i, 0, 0)); x_T is
+ * extdm_ddpm_fill_normal (stream 1, counter (element index / 4, 0, 1, 0)); the last iteration (time_next == 0) adds
+ * no noise and calls extdm_ddim_update with noise = NULL.  sigma*z is always added (a signed zero at eta = 0), so
+ * the result equals extdm_ddim_update fed the same draws, bit for bit.  seeds: (B,) int64.  Added under ABI
+ * version 5 (backward compatible). */
+int extdm_ddim_update_seeded(const float* img, const float* pred, const long long* seeds, int step, const float* s,
+                             float c_recip, float c_recipm1, float sqrt_alpha_next, float c, float sigma,
+                             float* img_out, float* x_start_out, int B, int n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * DDPM ancestral sampler (GaussianDiffusion.p_sample_loop, model/BaseDM_adaptor/Diffusion.py:136-189 with the
@@ -287,7 +297,9 @@ int extdm_ddim_update(const float* img, const float* pred, const float* noise, c
  *                             posterior_mean_coef2, nonzero_mask * exp(0.5 * posterior_log_variance_clipped)}[times[i]]
  *   step  one int32, the current row; seeds (B,) int64, one per video.
  * Noise is Philox4x32-10 + Box-Muller with key = the video's seed and counter = (element index / 4 within the video,
- * step, stream, 0); stream 0 is the noise of loop step `step`, stream 1 the initial x_T.
+ * step, stream, 0); stream 0 is the noise of loop step `step`, stream 1 the initial x_T.  The DDIM sampler with
+ * per-video seeds (extdm_ddim_update_seeded) uses the same counter layout: x_T from stream 1, the noise of DDIM
+ * iteration i from (step = i, stream 0).
  */
 
 /* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
