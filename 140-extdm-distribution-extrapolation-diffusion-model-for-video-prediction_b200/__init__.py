@@ -14,6 +14,9 @@ def __getattr__(name):
     if name == "Unet3D":
         from .unet import Unet3D
         return Unet3D
+    if name == "FlowAE":
+        from .flow_autoenc import FlowAE
+        return FlowAE
     if name in ("Generator", "RegionPredictor", "BGMotionPredictor"):
         from . import lfae
         return getattr(lfae, name)

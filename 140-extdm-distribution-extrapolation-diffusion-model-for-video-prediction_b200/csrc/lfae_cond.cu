@@ -173,19 +173,18 @@ __global__ void pca_affine_kernel(const float* __restrict__ covar, float* __rest
 
 // ------------------------------------------------------------------------------------------------ sparse motions
 // PixelwiseFlowPredictor.create_heatmap_representations / create_sparse_motions / create_deformed_source_image
-// (pixelwise_flow_predictor.py:48-112) for one frame per block.  Driving parameters are per frame, source parameters
-// are those of frame src_of(f) = (f / tc) * tc + tc - 1 (the reference frame of the video, whose region parameters are
-// the same values the reference computes in a separate RegionPredictor call on the same image).
+// (pixelwise_flow_predictor.py:48-112) for one frame f per block.  Driving parameters are those of frame f, source
+// parameters and the deformed source image those of frame fs, another frame of the same batch: the source frame is
+// part of the driving batch, and its region parameters are the values a separate RegionPredictor call on the same
+// image computes.
 //   inp   (F, h, w, cpad): channel 4k = heat_k (0 for the background k = 0), 4k+1..4k+3 = source warped by motion k
 //   motion(F, K+1, h, w, 2)
 // src: (F, h, w, src_ld) fp32 channels-last, channels 0..2 = the down-sampled frames.
-__global__ void sparse_motion_kernel(const float* __restrict__ src, int src_ld, const float* __restrict__ shift,
-                                     const float* __restrict__ covar, const float* __restrict__ affine,
-                                     const float* __restrict__ bg, int K, int tc, int h, int w, int revert_axis_swap,
-                                     int use_covar, float region_var, float* __restrict__ inp, int cpad,
-                                     float* __restrict__ motion) {
-  extern __shared__ float sm[];          // per region: [0..3] inv cov drv, [4..7] inv cov src, [8..11] aff, [12..15] shifts
-  const int f = blockIdx.x, fs = (f / tc) * tc + tc - 1;
+__device__ __forceinline__ void sparse_motion_frame(int f, int fs, float* sm, const float* __restrict__ src, int src_ld,
+                                                    const float* __restrict__ shift, const float* __restrict__ covar,
+                                                    const float* __restrict__ affine, const float* __restrict__ bg, int K,
+                                                    int h, int w, int revert_axis_swap, int use_covar, float region_var,
+                                                    float* __restrict__ inp, int cpad, float* __restrict__ motion) {
   for (int k = threadIdx.x; k < K; k += blockDim.x) {
     float* s = sm + k * 16;
     const float* cd = covar + (static_cast<long long>(f) * K + k) * 4;
@@ -270,6 +269,31 @@ __global__ void sparse_motion_kernel(const float* __restrict__ src, int src_ld, 
     }
     for (int c = 4 * (K + 1); c < cpad; ++c) o[c] = 0.f;
   }
+}
+
+// The conditioning stage: the source of frame f is its video's last conditioning frame, fs = (f / tc) * tc + tc - 1.
+__global__ void sparse_motion_kernel(const float* __restrict__ src, int src_ld, const float* __restrict__ shift,
+                                     const float* __restrict__ covar, const float* __restrict__ affine,
+                                     const float* __restrict__ bg, int K, int tc, int h, int w, int revert_axis_swap,
+                                     int use_covar, float region_var, float* __restrict__ inp, int cpad,
+                                     float* __restrict__ motion) {
+  extern __shared__ float sm[];          // per region: [0..3] inv cov drv, [4..7] inv cov src, [8..11] aff, [12..15] shifts
+  const int f = blockIdx.x, fs = (f / tc) * tc + tc - 1;
+  sparse_motion_frame(f, fs, sm, src, src_ld, shift, covar, affine, bg, K, h, w, revert_axis_swap, use_covar, region_var,
+                      inp, cpad, motion);
+}
+
+// Any source slot: frames come in groups of `group` (one video each), the source of frame f is slot src_slot of its
+// group, fs = (f / group) * group + src_slot.  Reconstruction (FlowAE) uses group = T frames per video.
+__global__ void sparse_motion_src_kernel(const float* __restrict__ src, int src_ld, const float* __restrict__ shift,
+                                         const float* __restrict__ covar, const float* __restrict__ affine,
+                                         const float* __restrict__ bg, int K, int group, int src_slot, int h, int w,
+                                         int revert_axis_swap, int use_covar, float region_var, float* __restrict__ inp,
+                                         int cpad, float* __restrict__ motion) {
+  extern __shared__ float sm[];
+  const int f = blockIdx.x, fs = (f / group) * group + src_slot;
+  sparse_motion_frame(f, fs, sm, src, src_ld, shift, covar, affine, bg, K, h, w, revert_axis_swap, use_covar, region_var,
+                      inp, cpad, motion);
 }
 
 // ------------------------------------------------------------------------------------------------ flow composition
@@ -410,6 +434,21 @@ extern "C" int extdm_sparse_motion(const float* src, int src_ld, const float* sh
   }
   sparse_motion_kernel<<<F_, 256, K * 16 * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
       src, src_ld, shift, covar, affine, bg, K, tc, h, w, revert_axis_swap, use_covar, region_var, inp, cpad, motion);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_sparse_motion_src(const float* src, int src_ld, const float* shift, const float* covar,
+                                       const float* affine, const float* bg, int F_, int K, int group, int src_slot, int h,
+                                       int w, int revert_axis_swap, int use_covar, float region_var, float* inp, int cpad,
+                                       float* motion, void* stream) {
+  if (K < 1 || group < 1 || F_ % group || src_slot < 0 || src_slot >= group || 4 * (K + 1) > cpad || src_ld < 3) {
+    extdm_set_error("sparse_motion_src: bad arguments", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  sparse_motion_src_kernel<<<F_, 256, K * 16 * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
+      src, src_ld, shift, covar, affine, bg, K, group, src_slot, h, w, revert_axis_swap, use_covar, region_var, inp, cpad,
+      motion);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

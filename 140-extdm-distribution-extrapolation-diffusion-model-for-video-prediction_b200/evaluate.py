@@ -7,6 +7,11 @@ SSIM of metrics/calculate_psnr.py:6-15 and metrics/calculate_ssim.py:6-42 as bat
     origin, result = evaluate.sample_videos(model, real_vids, total_pred, num_sample_video=n)
     evaluate.save_results(log_dir, origin, result)
     evaluate.psnr_videos(origin[:, 0], result[:, 0]);  evaluate.ssim_videos(...)
+
+Stage 1 (LFAE reconstruction, the upper bound of every DM prediction) uses the same layout and metrics:
+
+    ae = extdm_b200.FlowAE(cfg, pretrained_pth=ae_ckpt)        # or FlowAE.from_flow_diffusion(model)
+    origin, result = evaluate.reconstruct_videos(ae, real_vids)
 """
 import os
 
@@ -63,6 +68,19 @@ def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=Tr
     def shape(t):                                                                   # '(b n) c t h w -> b n t c h w'
         return t.reshape(B, num_sample_video, *t.shape[1:]).permute(0, 1, 3, 2, 4, 5).contiguous()
     return shape(rep.cpu().float()), shape(res)
+
+
+@torch.no_grad()
+def reconstruct_videos(ae, real_vids, source_frame=0):
+    """Stage-1 counterpart of sample_videos: real_vids (B, C, T, H, W) in [0,1] -> (origin, result), both (B, 1, T, C,
+    H, W) on the CPU, result = FlowAE.reconstruct(real_vids, source_frame)['prediction'], every frame reconstructed
+    from frame `source_frame` of its video.  psnr_videos / ssim_videos / summarize / save_results apply unchanged."""
+    dev = ae.generator.final.weight.device
+    pred = ae.reconstruct(real_vids.to(dev).float(), source_frame)["prediction"]
+
+    def shape(t):                                                                   # 'b c t h w -> b 1 t c h w'
+        return t.cpu().float().permute(0, 2, 1, 3, 4).unsqueeze(1).contiguous()
+    return shape(real_vids), shape(pred)
 
 
 def save_results(log_dir, origin_videos, result_videos, best_videos=None):

@@ -570,7 +570,8 @@ def _pad32(c):
 
 class CondRunner:
     """The conditioning stage of FlowDiffusion.sample_one_video (VideoFlowDiffusion_multi_w_ref.py:231-262) for F = B*tc
-    frames on the CUDA kernels: RegionPredictor -> BGMotionPredictor -> PixelwiseFlowPredictor.
+    frames on the CUDA kernels: RegionPredictor -> BGMotionPredictor -> PixelwiseFlowPredictor.  The same stage serves
+    stage-1 reconstruction (ReconRunner) with tc = T frames per video and the source at slot `src_slot` of each video.
 
     Convolutions run on the tcgen05 implicit GEMM in its tf32 mode (fp32 tensors, fp32 accumulate: the precision of the
     reference's cuDNN path), everything else on the fp32 kernels of csrc/lfae_cond.cu, including the PCA of the region
@@ -580,7 +581,8 @@ class CondRunner:
     halves instead (the fixture tests route it through LAPACK, whose signs differ: DESIGN.md section 1).
 
     The reference evaluates the region predictor twice on each video's last conditioning frame (once as `ref_img`,
-    once as driving frame tc-1, same weights, same input); here the source parameters are read from frame tc-1."""
+    once as driving frame tc-1, same weights, same input); here the source parameters are read from frame tc-1, or in
+    general from the driving batch's copy of the source frame, slot `src_slot` (default tc - 1) of each video."""
 
     pca = "gesvdj"           # class-level switch, see above
     use_cuda_graph = True
@@ -591,7 +593,10 @@ class CondRunner:
                 and rp.scale_factor in (1, 0.5, 0.25) and pfp.use_deformed_source
                 and rp.regions.kernel_size == (7, 7) and rp.regions.padding[0] <= 3)
 
-    def __init__(self, rp, bgp, pfp, dev, B, tc, H, W):
+    def __init__(self, rp, bgp, pfp, dev, B, tc, H, W, src_slot=None):
+        self.src_slot = tc - 1 if src_slot is None else src_slot
+        if not 0 <= self.src_slot < tc:
+            raise ValueError(f"CondRunner: src_slot {self.src_slot} outside [0, {tc})")
         self.recA, self.recB = ops.Recorder(record=True), ops.Recorder(record=True)
         self.recP = ops.Recorder(record=True)                  # the closed-form PCA between the two halves
         self._graph = None
@@ -634,8 +639,12 @@ class CondRunner:
         cin = 4 * (K + 1)
         cpad = _pad32(cin)
         inp, self.motion = buf(Fn, h, w, cpad), buf(Fn, K + 1, h, w, 2)
-        ops.sparse_motion(rec, xd, self.shift, self.covar, self.affine, self.bg, tc, pfp.revert_axis_swap,
-                          pfp.use_covar_heatmap, float(pfp.region_var), inp, self.motion)
+        if self.src_slot == tc - 1:                             # the conditioning stage's own entry
+            ops.sparse_motion(rec, xd, self.shift, self.covar, self.affine, self.bg, tc, pfp.revert_axis_swap,
+                              pfp.use_covar_heatmap, float(pfp.region_var), inp, self.motion)
+        else:
+            ops.sparse_motion_src(rec, xd, self.shift, self.covar, self.affine, self.bg, tc, self.src_slot,
+                                  pfp.revert_axis_swap, pfp.use_covar_heatmap, float(pfp.region_var), inp, self.motion)
         feat, xin = self._hourglass(rec, pfp.hourglass, inp, cin, buf)
         be = feat.shape[-1]
         heads = [pfp.mask] + ([pfp.occlusion] if pfp.occlusion is not None else [])
@@ -691,29 +700,87 @@ class CondRunner:
         """The stage's launch lists, in execution order (bench.py / tools/kernel_table.py account for them)."""
         return [self.recA, self.recP, self.recB] if self.pca == "gesvdj" else [self.recA, self.recB]
 
-    def run(self, real_vid):
-        """real_vid (B, 3, tc, H, W) fp32 on the device -> (grid (B,2,tc,h,w), conf (B,1,tc,h,w) | None)."""
+    def stage(self, real_vid):
+        """Copy real_vid (B, 3, tc, H, W) fp32 on the device into the static input buffers."""
         B, _, tc, H, W = real_vid.shape
         self.frames.view(B, tc, 3, H, W).copy_(real_vid.permute(0, 2, 1, 3, 4))
-        self.ref.copy_(real_vid[:, :, tc - 1])
+        self.ref.copy_(real_vid[:, :, self.src_slot])
+
+    def launch(self):
+        """Issue the stage on the current stream, without the graph."""
         if self.pca != "gesvdj":
             self.recA.run()
             u, s, _ = torch.svd(self.covar.view(-1, 2, 2))                 # region_predictor.py:130-136
             self.affine.view(-1, 2, 2).copy_(u @ torch.diag_embed(s ** 0.5))
             self.recB.run()
-            return self.grid, self.conf
-        if not self.use_cuda_graph or torch.cuda.is_current_stream_capturing():
-            for rec in (self.recA, self.recP, self.recB):
-                rec.run()
+            return
+        for rec in (self.recA, self.recP, self.recB):
+            rec.run()
+
+    def run(self, real_vid):
+        """real_vid (B, 3, tc, H, W) fp32 on the device -> (grid (B,2,tc,h,w), conf (B,1,tc,h,w) | None)."""
+        self.stage(real_vid)
+        if self.pca != "gesvdj" or not self.use_cuda_graph or torch.cuda.is_current_stream_capturing():
+            self.launch()
             return self.grid, self.conf
         if self._graph is None:                                # static buffers: the launch lists replay as one graph
-            for rec in (self.recA, self.recP, self.recB):      # warm-up (lazy per-kernel attribute set-up)
-                rec.run()
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                for rec in (self.recA, self.recP, self.recB):
-                    rec.run()
-            self._graph = g
+            self._graph = _capture(self.launch)
         self._graph.replay()
         return self.grid, self.conf
+
+
+def _capture(launch):
+    """One CUDA graph of `launch` (a function that issues kernels on the current stream), after one eager warm-up run
+    (lazy per-kernel attribute set-up)."""
+    launch()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        launch()
+    return g
+
+
+class ReconRunner:
+    """Stage-1 reconstruction (the LFAE forward of model/LFAE/generator.py:105-144, FlowAE.reconstruct) of B videos of T
+    frames on the CUDA kernels: CondRunner with tc = T and the source at slot src_slot of each video, then the
+    DecodeRunner of Generator.decode_video (encoder once per video, fused warp + blend, bf16 decoder).  Static buffers;
+    with the closed-form PCA the whole thing replays as one CUDA graph with no host sync and no library call inside.
+    `use_cuda_graph = False` (or CondRunner.pca = "torch") issues the same launch lists eagerly."""
+
+    use_cuda_graph = True
+
+    def __init__(self, gen, rp, bgp, dev, B, T, H, W, src_slot):
+        pfp = gen.pixelwise_flow_predictor
+        self.cond = CondRunner(rp, bgp, pfp, dev, B, T, H, W, src_slot=src_slot)
+        h, w = self.cond.grid.shape[-2:]
+        self.dec = gen.decoder(B, T, H, W, h, w, pfp.occlusion is not None)
+        self.src_slot = src_slot
+        self._graph = None
+
+    def launch(self):
+        c, d = self.cond, self.dec
+        c.launch()
+        # (B, 2, T, h, w) -> the decoder's (B*T, h, w, 2); the occlusion map has the same memory order in both
+        d.flow.view(c.grid.shape[0], c.grid.shape[2], *d.flow.shape[1:]).copy_(c.grid.permute(0, 2, 3, 4, 1))
+        if d.occ is not None:
+            d.occ.view(c.conf.shape).copy_(c.conf)
+        d.run()
+
+    def run(self, real_vid):
+        """real_vid (B, 3, T, H, W) fp32 on the device -> dict of (B, C, T, ...) tensors (views of the static buffers
+        but optical_flow / occlusion_map, which are the CondRunner's)."""
+        B, _, T, H, W = real_vid.shape
+        self.cond.stage(real_vid)
+        self.dec.src.copy_(real_vid[:, :, self.src_slot])
+        if self.cond.pca != "gesvdj" or not self.use_cuda_graph or torch.cuda.is_current_stream_capturing():
+            self.launch()
+        else:
+            if self._graph is None:
+                self._graph = _capture(self.launch)
+            self._graph.replay()
+        per_video = lambda t: t.view(B, T, *t.shape[1:]).transpose(1, 2)
+        out = {"prediction": per_video(self.dec.prediction), "deformed": per_video(self.dec.deformed),
+               "optical_flow": self.cond.grid}
+        if self.cond.conf is not None:
+            out["occlusion_map"] = self.cond.conf
+        return out

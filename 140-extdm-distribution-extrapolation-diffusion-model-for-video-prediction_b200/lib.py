@@ -46,6 +46,7 @@ PROTOTYPES = {
     "extdm_region_moments": [_P, _I, _I, _I, _I, _I, _I, _F, _P, _P, _P],
     "extdm_pca_affine": [_P, _P, _I, _P],
     "extdm_sparse_motion": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _P, _I, _P, _P],
+    "extdm_sparse_motion_src": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _F, _P, _I, _P, _P],
     "extdm_flow_compose": [_P, _I, _P, _I, _I, _I, _I, _I, _P, _P, _P],
     "extdm_bg_head": [_P, _I, _I, _I, _P, _P, _I, _I, _P, _P],
     "extdm_groupnorm_stats": [_P, _P, _I, _L, _I, _I, _P],

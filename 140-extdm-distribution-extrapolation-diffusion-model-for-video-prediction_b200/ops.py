@@ -697,6 +697,18 @@ def sparse_motion(rec, src, shift, covar, affine, bg, tc, revert_axis_swap, use_
              keep=(src, shift, covar, affine, bg, inp, motion))
 
 
+def sparse_motion_src(rec, src, shift, covar, affine, bg, group, src_slot, revert_axis_swap, use_covar, region_var, inp,
+                      motion):
+    """sparse_motion with the source of frame f at slot src_slot of its group of `group` frames (one video each)."""
+    F_, h, w, cpad = inp.shape
+    K = shift.shape[1]
+    rec.emit("extdm_sparse_motion_src", (_p(src), src.shape[-1], _p(shift), _p(covar), _p(affine),
+                                         _p(bg) if bg is not None else None, F_, K, group, src_slot, h, w,
+                                         int(revert_axis_swap), int(use_covar), C.c_float(region_var), _p(inp), cpad,
+                                         _p(motion)),
+             keep=(src, shift, covar, affine, bg, inp, motion))
+
+
 def flow_compose(rec, head, motion, K, tc, grid, conf):
     F_, h, w, ldc = head.shape
     rec.emit("extdm_flow_compose", (_p(head), ldc, _p(motion), F_, K, tc, h, w, _p(grid),

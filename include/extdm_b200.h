@@ -391,6 +391,14 @@ int extdm_pca_affine(const float* covar, float* affine, int n, void* stream);
 int extdm_sparse_motion(const float* src, int src_ld, const float* shift, const float* covar, const float* affine,
                         const float* bg, int F, int K, int tc, int h, int w, int revert_axis_swap, int use_covar,
                         float region_var, float* inp, int cpad, float* motion, void* stream);
+/* extdm_sparse_motion with any source slot: frames come in groups of `group` consecutive frames (one video each), and
+ * the source parameters / image of frame f are those of frame (f / group) * group + src_slot, 0 <= src_slot < group,
+ * F % group == 0.  extdm_sparse_motion is this entry with group = tc, src_slot = tc - 1; flow-autoencoder
+ * reconstruction (FlowAE.reconstruct) calls it with group = T frames per video.  Added under ABI version 5 (backward
+ * compatible). */
+int extdm_sparse_motion_src(const float* src, int src_ld, const float* shift, const float* covar, const float* affine,
+                            const float* bg, int F, int K, int group, int src_slot, int h, int w, int revert_axis_swap,
+                            int use_covar, float region_var, float* inp, int cpad, float* motion, void* stream);
 /* mask softmax, flow = sum_k mask_k * motion_k, occlusion = sigmoid (pixelwise_flow_predictor.py:140-152).  head (F, h, w,
  * ldc): channels [0, K] mask logits, K+1 occlusion logit.  grid (B, 2, tc, h, w), conf (B, 1, tc, h, w) or NULL. */
 int extdm_flow_compose(const float* head, int ldc, const float* motion, int F, int K, int tc, int h, int w, float* grid,
