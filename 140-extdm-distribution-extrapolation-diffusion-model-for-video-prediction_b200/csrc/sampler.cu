@@ -5,6 +5,8 @@
 // The DDPM ancestral step (GaussianDiffusion.p_sample_loop) shares that select; its per-step coefficients, step index and
 // Philox noise live on the device, so one captured iteration can be replayed for every timestep.
 // DDIM with per-video seeds draws its noise from the same Philox generator inside the update.
+// The denoising-loss evaluation (GaussianDiffusion.denoising_loss) draws its epsilon from that generator too (stream 2)
+// in the forward-diffusion kernel, and reduces the per-(video, frame) loss in a fixed order.
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -250,6 +252,68 @@ __global__ void __launch_bounds__(256) ddim_update_seeded_kernel(const float* __
   }
 }
 
+// ------------------------------------------------------------------------------------------------ denoising loss
+// Philox counter word 2 of the loss evaluation's epsilon; word 1 is the video's timestep t[b]
+constexpr unsigned int kStreamLoss = 2u;
+
+// x_t = a * x_start + b * eps with a = sqrt_alphas_cumprod[t], b = sqrt_one_minus_alphas_cumprod[t]: two roundings then a
+// sum, never an FMA, as torch evaluates `extract(a, t) * x_start + extract(b, t) * noise`.
+__device__ __forceinline__ float q_sample_of(float x0, float eps, float a, float b) {
+  return __fadd_rn(__fmul_rn(a, x0), __fmul_rn(b, eps));
+}
+
+__global__ void __launch_bounds__(256) q_sample_kernel(const float* __restrict__ x_start,
+                                                       const long long* __restrict__ t,
+                                                       const long long* __restrict__ seeds,
+                                                       const float* __restrict__ noise,
+                                                       const float* __restrict__ sqrt_acp,
+                                                       const float* __restrict__ sqrt_1m_acp,
+                                                       float* __restrict__ x_t, float* __restrict__ eps_out,
+                                                       int n4_per_sample, long long total4) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    const long long tb = __ldg(t + b);
+    const float a = __ldg(sqrt_acp + tb), c = __ldg(sqrt_1m_acp + tb);
+    const float4 e = noise ? reinterpret_cast<const float4*>(noise)[i]
+                           : normal4(__ldg(seeds + b), static_cast<unsigned int>(i - b * n4_per_sample),
+                                     static_cast<unsigned int>(tb), kStreamLoss);
+    const float4 x = reinterpret_cast<const float4*>(x_start)[i];
+    reinterpret_cast<float4*>(x_t)[i] =
+        make_float4(q_sample_of(x.x, e.x, a, c), q_sample_of(x.y, e.y, a, c), q_sample_of(x.z, e.z, a, c),
+                    q_sample_of(x.w, e.w, a, c));
+    reinterpret_cast<float4*>(eps_out)[i] = e;
+  }
+}
+
+// One block per (video b, frame f) of (B, 3, tp, hw) tensors: out[b, f] = mean over (3, hw) of (eps - pred)^2 (or
+// |eps - pred|).  The difference of two floats is exact in double, so the terms are exact and the sum is in fp64; each
+// thread sums a fixed strided subset in order, then a fixed shared-memory tree: the result depends on the (b, f) slice
+// only, bit for bit, whatever the batch, the call or the launch.
+constexpr int kLossThreads = 256;
+__global__ void __launch_bounds__(kLossThreads) denoise_loss_kernel(const float* __restrict__ eps,
+                                                                    const float* __restrict__ pred,
+                                                                    float* __restrict__ out, int tp, int hw, int l1) {
+  __shared__ double part[kLossThreads];
+  const int b = blockIdx.x / tp, f = blockIdx.x % tp;
+  const long long plane = static_cast<long long>(tp) * hw;
+  const long long base = static_cast<long long>(b) * 3 * plane + static_cast<long long>(f) * hw;
+  double acc = 0.0;
+  for (int j = threadIdx.x; j < 3 * hw; j += kLossThreads) {
+    const long long k = base + (j / hw) * plane + j % hw;
+    const double d = static_cast<double>(__ldg(eps + k)) - static_cast<double>(__ldg(pred + k));
+    acc += l1 ? fabs(d) : d * d;
+  }
+  part[threadIdx.x] = acc;
+  __syncthreads();
+#pragma unroll
+  for (int s = kLossThreads / 2; s > 0; s >>= 1) {
+    if (threadIdx.x < s) part[threadIdx.x] += part[threadIdx.x + s];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[blockIdx.x] = static_cast<float>(part[0] / static_cast<double>(3 * hw));
+}
+
 // out[b, :] = table[*step, :] for every sample: the time-conditioned rows of the step, shared by the whole batch.
 __global__ void __launch_bounds__(256) ddpm_broadcast_row_kernel(const float* __restrict__ table,
                                                                  const int* __restrict__ step,
@@ -365,6 +429,33 @@ extern "C" int extdm_ddpm_advance(int* step, const long long* times, int n_steps
     return EXTDM_ERR_ARG;
   }
   ddpm_advance_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(step, times, n_steps, time, B);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_q_sample(const float* x_start, const long long* t, const long long* seeds, const float* noise,
+                              const float* sqrt_acp, const float* sqrt_1m_acp, float* x_t_out, float* eps_out, int B,
+                              int n, void* stream) {
+  if (n % 4 || n < 4 || B < 1 || !t || (!noise && !seeds) || !sqrt_acp || !sqrt_1m_acp || !x_t_out || !eps_out) {
+    extdm_set_error("q_sample: need n % 4 == 0, B >= 1, t, seeds or noise, both tables and both outputs", __FILE__,
+                    __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  q_sample_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t_out, eps_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_denoise_loss(const float* eps, const float* pred, float* out, int B, int tp, int per_frame, int l1,
+                                  void* stream) {
+  if (B < 1 || tp < 1 || per_frame < 3 || per_frame % 3 || static_cast<long long>(B) * tp > 0x7FFFFFFFLL) {
+    extdm_set_error("denoise_loss: need B, tp >= 1 and per_frame a positive multiple of 3", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  denoise_loss_kernel<<<B * tp, kLossThreads, 0, static_cast<cudaStream_t>(stream)>>>(eps, pred, out, tp,
+                                                                                     per_frame / 3, l1 != 0);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

@@ -7,8 +7,10 @@ sampling_timesteps x (UNet step + threshold + update)) is captured once per shap
 With `seeds` (one int64 per video) DDIM draws its noise inside the update kernel from a Philox stream keyed by the
 video's seed, so a video's sample does not depend on the rest of its batch and no noise tensor is stored.
 sampling_timesteps == timesteps (or None) selects the ancestral sampler, whose loop is too long for one graph: ONE
-iteration is captured and replayed timesteps times, with its per-step values on the device.  Training paths
-(p_losses, q_sample) are out of scope.
+iteration is captured and replayed timesteps times, with its per-step values on the device.
+`denoising_loss()` evaluates the training objective of p_losses (Diffusion.py:286-319) forward-only, under no_grad:
+forward diffusion to one timestep per video, one UNet forward, the per-(video, frame) loss, as one CUDA graph.
+Training itself (gradients, optimisers) is out of scope.
 """
 import torch
 import torch.nn.functional as F
@@ -33,6 +35,27 @@ def _seed_vector(seeds, noise, B, who):
     if tuple(seeds.shape) != (B,):
         raise ValueError(f"{who}: need one seed per video, shape ({B},), got {tuple(seeds.shape)}")
     return seeds
+
+
+def _timestep_vector(timesteps, B, num_timesteps, who):
+    """Validate per-video timesteps: None, or a (B,) int64 tensor (any device) or a list of ints, each in
+    [0, num_timesteps).  The range is checked on the host (a device tensor is copied there, one synchronisation):
+    the forward-diffusion kernel indexes the schedule tables with these values."""
+    if timesteps is None:
+        return None
+    if not torch.is_tensor(timesteps):
+        try:
+            timesteps = torch.tensor(list(timesteps))
+        except (TypeError, RuntimeError, OverflowError) as e:
+            raise ValueError(f"{who}: timesteps must be int64 values ({e})") from None
+    if timesteps.dtype != torch.int64:
+        raise ValueError(f"{who}: timesteps must be int64, got {timesteps.dtype}")
+    if tuple(timesteps.shape) != (B,):
+        raise ValueError(f"{who}: need one timestep per video, shape ({B},), got {tuple(timesteps.shape)}")
+    host = timesteps.cpu()
+    if B and (int(host.min()) < 0 or int(host.max()) >= num_timesteps):
+        raise ValueError(f"{who}: timesteps must lie in [0, {num_timesteps}), got {host.tolist()}")
+    return timesteps
 
 
 def _load_seeds(dst, seeds):
@@ -321,3 +344,103 @@ class GaussianDiffusion(nn.Module):
         if trace is not None:
             trace[-1].update(x_start=xs, s=st["s"].clone(), img=r.x.clone())
         ops.ddpm_advance(rec, st["step"], st["times"], r.time)
+
+    # ------------------------------------------------------------------ denoising loss (forward-only p_losses)
+    def loss_args(self, B, shape, timesteps=None, seeds=None, noise=None, who="denoising_loss"):
+        """Check the arguments of denoising_loss for B videos whose x_start has `shape` (B, 3, tp, h, w): loss_type,
+        timesteps (_timestep_vector), seeds (_seed_vector, not together with noise), the shape of noise.  Returns
+        (timesteps, seeds), either None when not given.  Runs on the host only, before anything is launched."""
+        if self.loss_type not in ("l1", "l2"):
+            raise ValueError(f"{who}: loss_type {self.loss_type!r} is not 'l1' or 'l2'")
+        seeds = _seed_vector(seeds, noise, B, who)
+        if noise is not None and (not torch.is_tensor(noise) or tuple(noise.shape) != tuple(shape)):
+            raise ValueError(f"{who}: noise must have shape {tuple(shape)}, got "
+                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
+        return _timestep_vector(timesteps, B, self.num_timesteps, who), seeds
+
+    @torch.no_grad()
+    def denoising_loss(self, x_start, x_cond, cond_fea, timesteps=None, seeds=None, noise=None):
+        """The epsilon-prediction loss of p_losses (Diffusion.py:286-319) per video, forward only.  DESIGN.md section 1
+        specifies it:
+
+            x_t  = sqrt_alphas_cumprod[t] * x_start + sqrt_one_minus_alphas_cumprod[t] * eps    (fp32, no FMA)
+            pred = Unet3D(x_t, t, cond_frames=x_cond, cond_fea=cond_fea)
+            loss_per_frame[b, f] = mean over (3, h, w) of (eps - pred)^2 ('l2') or |eps - pred| ('l1')
+
+        x_start (B, 3, tp, h, w), x_cond (B, 3, tc, h, w), cond_fea as for sample().  timesteps: optional (B,) int64
+        tensor or list in [0, num_timesteps); default torch.randint(0, num_timesteps, (B,)) from the default generator,
+        as the reference draws it.  seeds: optional (B,) int64 tensor or list; eps of video b is then the Philox draw
+        of (seeds[b], t[b], stream 2) (include/extdm_b200.h), so it depends on the video's seed and timestep only;
+        default: seeds drawn from the default generator (after t), as p_sample_loop does.  noise: optional
+        (B, 3, tp, h, w) eps instead of seeds.  Returns {'loss': (B,), 'loss_per_frame': (B, tp), 'timesteps': (B,)
+        int64}, on x_start's device; loss.mean() is the reference's F.mse_loss(noise, x_recon) for 'l2'.
+
+        The launches (UNet prologue, forward diffusion, time MLP, UNet step, loss) run as one CUDA graph per shape and
+        loss_type, kept on the UNet runner; t and the seeds are copied in before each replay without a host
+        synchronisation (a (B,) timestep tensor on the device is range-checked on the host first)."""
+        for name, v in (("x_start", x_start), ("x_cond", x_cond), ("cond_fea", cond_fea)):
+            if not torch.is_tensor(v) or v.dim() != 5:
+                raise ValueError(f"denoising_loss: {name} must be a 5-D tensor")
+        B, C, tp, h, w = x_start.shape
+        tc = x_cond.shape[2]
+        if C != 3 or tc + tp != self.num_frames or tuple(x_cond.shape) != (B, 3, tc, h, w) or cond_fea.shape[0] != B:
+            raise ValueError(f"denoising_loss: x_start {tuple(x_start.shape)}, x_cond {tuple(x_cond.shape)}, cond_fea "
+                             f"{tuple(cond_fea.shape)}: expected (B, 3, tp, h, w), (B, 3, tc, h, w) and (B, ...) with "
+                             f"tc + tp = {self.num_frames}")
+        t, seeds = self.loss_args(B, x_start.shape, timesteps, seeds, noise)
+        if x_start.device.type != "cuda":
+            raise RuntimeError("denoising_loss runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        if t is None:
+            t = torch.randint(0, self.num_timesteps, (B,))
+        if noise is None and seeds is None:
+            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        r = self.denoise_fn.runner(B, h, w, cond_fea.shape[-1])
+        l1 = self.loss_type == "l1"
+
+        def state():
+            f32 = dict(device=r.dev, dtype=torch.float32)
+            return dict(x_start=torch.zeros(x_start.shape, **f32), eps=torch.zeros(x_start.shape, **f32),
+                        lpf=torch.zeros(B, tp, **f32),
+                        seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if noise is None else None,
+                        noise=torch.zeros(x_start.shape, **f32) if noise is not None else None,
+                        acp=self.sqrt_alphas_cumprod.to(**f32).clone(),
+                        a1m=self.sqrt_one_minus_alphas_cumprod.to(**f32).clone())
+
+        def stage(st):
+            r.set_conditioning(x_cond.float(), cond_fea.float())
+            st["x_start"].copy_(x_start)
+            if noise is not None:
+                st["noise"].copy_(noise)
+            else:
+                _load_seeds(st["seeds"], seeds)
+            _load_seeds(r.time, t)                                     # no host sync before the launches / replay
+
+        if not self.use_cuda_graph:
+            st = state()
+            stage(st)
+            self._loss_launch(r, st, l1)
+        else:
+            # like ddim_graphs the graph points into the runner's buffers, so it lives on the runner
+            key = (tuple(x_start.shape), self.loss_type, noise is not None, self.num_timesteps)
+            if key not in r.loss_graphs:
+                st = state()
+                stage(st)
+                self._loss_launch(r, st, l1)                           # warm-up (lazy inits)
+                torch.cuda.synchronize()
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._loss_launch(r, st, l1)
+                r.loss_graphs[key] = (g, st)
+            g, st = r.loss_graphs[key]
+            stage(st)
+            g.replay()
+        lpf = st["lpf"].clone()           # a copy: the next call of the same shape rewrites the state
+        return {"loss": lpf.mean(dim=1), "loss_per_frame": lpf, "timesteps": r.time.clone()}
+
+    def _loss_launch(self, r, st, l1):
+        """UNet prologue, x_t and eps, time MLP on r.time, UNet step (pred in r.out), per-(video, frame) loss."""
+        rec = ops.IMMEDIATE
+        r.run_prologue()
+        ops.q_sample(rec, st["x_start"], r.time, st["seeds"], st["noise"], st["acp"], st["a1m"], r.x, st["eps"])
+        r.run_step()
+        ops.denoise_loss(rec, st["eps"], r.out, st["lpf"], l1)

@@ -12,6 +12,11 @@ Stage 1 (LFAE reconstruction, the upper bound of every DM prediction) uses the s
 
     ae = extdm_b200.FlowAE(cfg, pretrained_pth=ae_ckpt)        # or FlowAE.from_flow_diffusion(model)
     origin, result = evaluate.reconstruct_videos(ae, real_vids)
+
+The diffusion model's own training objective on held-out clips of tc + tp frames (checkpoint selection, loss against
+timestep):
+
+    out = evaluate.denoising_loss_videos(model, real_vids, timesteps=[100, 500, 900], seed=0)
 """
 import os
 
@@ -81,6 +86,44 @@ def reconstruct_videos(ae, real_vids, source_frame=0):
     def shape(t):                                                                   # 'b c t h w -> b 1 t c h w'
         return t.cpu().float().permute(0, 2, 1, 3, 4).unsqueeze(1).contiguous()
     return shape(real_vids), shape(pred)
+
+
+@torch.no_grad()
+def denoising_loss_videos(model, real_vids, timesteps=None, seed=None, video_offset=0):
+    """FlowDiffusion.denoising_loss over real_vids (B, C, tc + tp, H, W) in [0, 1] (any device) -> dict of CPU tensors
+    {'loss', 'loss_per_frame', 'timesteps'}.
+
+    timesteps: None (drawn), an int (every video at that timestep), a (B,) int64 tensor, or a list of K ints: a loss
+    curve, one graph replay per timestep on the same conditioning, and then 'loss' is (B, K), 'loss_per_frame'
+    (B, K, tp) and 'timesteps' (B, K); otherwise (B,), (B, tp) and (B,).
+
+    seed: optional int.  Then video b, whose *global* index is g = video_offset + b, draws its epsilon with the seed
+    sharding.video_seeds(seed, g, 0), and, when timesteps is None, is evaluated at the timestep
+    sharding.video_seeds(seed, g, 1) % num_timesteps.  Both depend on (seed, g) only, so a sharded evaluation that
+    passes video_offset = lo of sharding.shard_range evaluates every video exactly as a single-GPU run does.  Within a
+    loss curve the epsilon still differs per timestep (the Philox counter holds t).  Without seed, the timesteps and
+    the seeds come from torch's default generator (GaussianDiffusion.denoising_loss)."""
+    from .sharding import video_seeds
+    B = real_vids.shape[0]
+    n_t = model.diffusion.num_timesteps
+    ids = torch.arange(B) + video_offset
+    seeds = video_seeds(seed, ids, 0) if seed is not None else None
+    curve = isinstance(timesteps, (list, tuple))
+    if timesteps is None:
+        ts = [video_seeds(seed, ids, 1) % n_t if seed is not None else None]
+    elif curve or not torch.is_tensor(timesteps):
+        ks = list(timesteps) if curve else [timesteps]
+        if not ks or any(isinstance(k, bool) or not isinstance(k, int) or not 0 <= k < n_t for k in ks):
+            raise ValueError(f"denoising_loss_videos: timesteps must be ints in [0, {n_t}), got {timesteps!r}")
+        ts = [torch.full((B,), k, dtype=torch.long) for k in ks]
+    else:
+        ts = [timesteps]
+    dev = next(model.parameters()).device
+    inputs = model.loss_inputs(real_vids.to(dev).float())
+    outs = [model.diffusion.denoising_loss(*inputs, timesteps=t, seeds=seeds) for t in ts]
+    if not curve:
+        return {k: v.cpu() for k, v in outs[0].items()}
+    return {k: torch.stack([o[k] for o in outs], dim=1).cpu() for k in outs[0]}
 
 
 def save_results(log_dir, origin_videos, result_videos, best_videos=None):

@@ -119,7 +119,15 @@ class FlowDiffusion(nn.Module):
                 raise KeyError("occlusion_map")
         else:
             ret = self._condition_torch(real_vid, ref, frames, with_decode)
-        # bottleneck features: encoder of frames 0..tc-2, then the reference frame's repeated
+        fea = self._cond_fea(frames, B, ret["real_vid_grid"].shape[-2:])
+        x_cond = flow_to_x_start(ret["real_vid_grid"], ret.get("real_vid_conf"), False)
+        return ret, x_cond, fea, ref
+
+    def _cond_fea(self, frames, B, flow_hw):
+        """cond_fea of condition() from its (B*tc, 3, H, W) frames: the bottleneck features of frames 0..tc-2, then the
+        reference frame's repeated."""
+        tc, tp = self.cond_frame_num, self.pred_frame_num
+        H, W = frames.shape[-2:]
         enc_frames = self.generator.forward_bottle(frames).reshape(B, tc, 256, H // 4, W // 4)
         ref_fea = enc_frames[:, tc - 1]
         n_rep = (1 + tp) if self.WRAPPER == "w_ref" else tp
@@ -130,15 +138,9 @@ class FlowDiffusion(nn.Module):
             # CUDA path the UNet prologue does that resize itself (extdm_bilinear_resize_cl, align_corners=False like
             # F.interpolate), so the features stay at H/4 here; this branch serves the CPU parity fixtures only.
             n, c, t, h, w = fea.shape
-            hw = ret["real_vid_grid"].shape[-2:]
-            fea = F.interpolate(fea.transpose(1, 2).reshape(n * t, c, h, w), size=hw, mode="bilinear")
-            fea = fea.reshape(n, t, c, *hw).transpose(1, 2).contiguous()
-        grid = ret["real_vid_grid"]
-        if self.estimate_occlusion_map:
-            x_cond = torch.cat((grid, ret["real_vid_conf"] * 2 - 1), dim=1)
-        else:
-            x_cond = torch.cat((grid, torch.zeros_like(grid)[:, 0:1]), dim=1)
-        return ret, x_cond, fea, ref
+            fea = F.interpolate(fea.transpose(1, 2).reshape(n * t, c, h, w), size=flow_hw, mode="bilinear")
+            fea = fea.reshape(n, t, c, *flow_hw).transpose(1, 2).contiguous()
+        return fea
 
     def _condition_torch(self, real_vid, ref, frames, with_decode):
         """The same stage as ordinary torch modules (cuDNN on a GPU): CPU parity fixtures, unsupported predictor
@@ -176,13 +178,11 @@ class FlowDiffusion(nn.Module):
         pred = self.diffusion.sample(x_cond, cond_fea=cond_fea, batch_size=1, cond_scale=cond_scale, noise=noise,
                                      seeds=seeds)
         tc = self.cond_frame_num
-        grid = pred[:, :2]
-        if self.use_residual_flow:
-            grid = grid + self.get_grid(grid.shape[0], 1, grid.shape[3], grid.shape[4]).to(grid.device)
+        grid, conf = x_start_to_flow(pred, self.use_residual_flow, self.estimate_occlusion_map)
         sample_vid_grid = torch.cat([ret["real_vid_grid"][:, :, :tc], grid], dim=2)
         sample_vid_conf = None
         if self.estimate_occlusion_map:
-            sample_vid_conf = torch.cat([ret["real_vid_conf"][:, :, :tc], (pred[:, 2:3] + 1) * 0.5], dim=2)
+            sample_vid_conf = torch.cat([ret["real_vid_conf"][:, :, :tc], conf], dim=2)
         out, warped = self.generator.decode_video(ref, sample_vid_grid, sample_vid_conf)
         ret["sample_vid_grid"] = sample_vid_grid
         if sample_vid_conf is not None:
@@ -192,6 +192,59 @@ class FlowDiffusion(nn.Module):
         ret["real_out_vid"] = out[:, :, :tc]
         ret["real_warped_vid"] = warped[:, :, :tc]
         return ret
+
+    # ------------------------------------------------------------------ denoising loss (forward-only training objective)
+    def _loss_video_shape(self, real_vid):
+        """(B, h, w) of a denoising-loss input: real_vid (B, 3, tc + tp, H, W); (h, w) is the flow resolution."""
+        if not torch.is_tensor(real_vid) or real_vid.dim() != 5:
+            raise ValueError("denoising_loss: real_vid must be a (B, 3, tc + tp, H, W) tensor")
+        B, C, T, H, W = real_vid.shape
+        if C != 3 or T != self.frame_num or B < 1:
+            raise ValueError(f"denoising_loss: real_vid {tuple(real_vid.shape)}: expected (B >= 1, 3, "
+                             f"{self.frame_num} = tc + tp, H, W)")
+        st = int(round(1 / self.region_predictor.scale_factor))
+        return B, H // st, W // st
+
+    @torch.no_grad()
+    def loss_inputs(self, real_vid):
+        """(x_start, x_cond, cond_fea) of denoising_loss for real_vid (B, 3, tc + tp, H, W) in [0, 1] (DESIGN.md
+        section 1): one CondRunner over all tc + tp frames of each video with the source at slot tc - 1.  Its first tc
+        flows give x_cond, cond_fea is condition()'s, and x_start is flow_to_x_start of frames tc .. tc + tp - 1, the
+        inverse of sample_one_video's post-processing: decoding x_start gives the LFAE reconstruction of those frames."""
+        B, _, _ = self._loss_video_shape(real_vid)
+        if not real_vid.is_cuda:
+            raise RuntimeError("denoising_loss runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        rp, bgp, pfp = self.region_predictor, self.bg_predictor, self.generator.pixelwise_flow_predictor
+        if not CondRunner.supported(rp, bgp, pfp):
+            raise NotImplementedError("denoising_loss: the conditioning kernels do not cover these predictor "
+                                      "hyper-parameters (lfae.CondRunner.supported)")
+        if not self.estimate_occlusion_map and self.WRAPPER != "w_ref":
+            raise KeyError("occlusion_map")                            # as condition()
+        tc, T = self.cond_frame_num, self.frame_num
+        _, _, _, H, W = real_vid.shape
+        key = (real_vid.device, B, T, H, W, tc - 1)
+        if key not in self._cond_runners:
+            self._cond_runners[key] = CondRunner(rp, bgp, pfp, real_vid.device, B, T, H, W, src_slot=tc - 1)
+        grid, conf = self._cond_runners[key].run(real_vid.float())
+        frames = real_vid[:, :, :tc].permute(0, 2, 1, 3, 4).reshape(B * tc, 3, H, W) \
+            .contiguous(memory_format=torch.channels_last)
+        fea = self._cond_fea(frames, B, grid.shape[-2:])
+        if not self.estimate_occlusion_map:
+            conf = None
+        x_cond = flow_to_x_start(grid[:, :, :tc], None if conf is None else conf[:, :, :tc], False)
+        x_start = flow_to_x_start(grid[:, :, tc:], None if conf is None else conf[:, :, tc:], self.use_residual_flow)
+        return x_start, x_cond, fea
+
+    @torch.no_grad()
+    def denoising_loss(self, real_vid, timesteps=None, seeds=None, noise=None):
+        """The diffusion model's training objective evaluated forward-only on real_vid (B, 3, tc + tp, H, W) in [0, 1]:
+        GaussianDiffusion.denoising_loss on loss_inputs(real_vid).  timesteps, seeds, noise: as there (noise has the
+        shape of x_start, (B, 3, tp, h, w)).  Returns {'loss': (B,), 'loss_per_frame': (B, tp), 'timesteps': (B,)}.
+        Argument errors raise ValueError before anything runs; CPU tensors then raise RuntimeError."""
+        B, h, w = self._loss_video_shape(real_vid)
+        self.diffusion.loss_args(B, (B, 3, self.pred_frame_num, h, w), timesteps, seeds, noise)
+        x_start, x_cond, cond_fea = self.loss_inputs(real_vid)
+        return self.diffusion.denoising_loss(x_start, x_cond, cond_fea, timesteps=timesteps, seeds=seeds, noise=noise)
 
     def forward(self, real_vid):
         raise NotImplementedError("training forward is outside the sampling hot path (SURVEY.md section 2, row 3a)")
@@ -204,6 +257,24 @@ class FlowDiffusion(nn.Module):
             hr, wr = torch.arange(0, H), torch.arange(0, W)
         grid = torch.stack(torch.meshgrid(hr, wr, indexing="xy"), -1).repeat(b, 1, 1, 1).flip(3).float()
         return grid.permute(0, 3, 1, 2).unsqueeze(dim=2).repeat(1, 1, nf, 1, 1)
+
+
+def x_start_to_flow(x, use_residual_flow, with_conf):
+    """sample_one_video's post-processing of a sampled x (B, 3, tp, h, w): (grid (B, 2, tp, h, w), conf (B, 1, tp, h, w)
+    or None).  grid = x[:, :2] (+ the identity grid with use_residual_flow); conf = (x[:, 2:3] + 1) * 0.5."""
+    grid = x[:, :2]
+    if use_residual_flow:
+        grid = grid + FlowDiffusion.get_grid(grid.shape[0], 1, grid.shape[3], grid.shape[4]).to(grid.device)
+    return grid, ((x[:, 2:3] + 1) * 0.5 if with_conf else None)
+
+
+def flow_to_x_start(grid, conf, use_residual_flow):
+    """The inverse of x_start_to_flow: (grid - the identity grid with use_residual_flow | conf * 2 - 1, or zeros
+    without an occlusion map) -> (B, 3, T, h, w).  With use_residual_flow=False this is condition()'s x_cond."""
+    if use_residual_flow:
+        grid = grid - FlowDiffusion.get_grid(grid.shape[0], 1, grid.shape[3], grid.shape[4]).to(grid.device)
+    third = conf * 2 - 1 if conf is not None else torch.zeros_like(grid)[:, 0:1]
+    return torch.cat((grid, third), dim=1)
 
 
 class FlowDiffusionMulti1248(FlowDiffusion):

@@ -599,6 +599,54 @@ def ddpm_advance(rec, step, times, time):
              keep=(step, times, time))
 
 
+def q_sample(rec, x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t, eps):
+    """x_t = sqrt_acp[t[b]] * x_start + sqrt_1m_acp[t[b]] * eps, eps = noise when given, else the Philox draw of
+    (seeds[b], t[b], stream 2); eps is written too.  t must lie in [0, len(sqrt_acp)): the kernel indexes the tables
+    with it, so the caller validates it on the host."""
+    for v, name in ((x_start, "x_start"), (x_t, "x_t"), (eps, "eps"), (sqrt_acp, "sqrt_acp"),
+                    (sqrt_1m_acp, "sqrt_1m_acp")):
+        if v is None:
+            raise ValueError(f"q_sample: {name} is required")
+        _chk(v, torch.float32, name)
+    _chk(t, torch.int64, "t")
+    _chk(seeds, torch.int64, "seeds")
+    _chk(noise, torch.float32, "noise")
+    B = x_start.shape[0]
+    if t is None or t.numel() != B or t.device != x_start.device:
+        raise ValueError(f"q_sample: t must be {B} int64 on {x_start.device}")
+    if (seeds is None) == (noise is None):
+        raise ValueError("q_sample: pass exactly one of seeds and noise")
+    if seeds is not None and (seeds.numel() != B or seeds.device != x_start.device):
+        raise ValueError(f"q_sample: seeds must be {B} int64 on {x_start.device}, got {seeds.numel()} on "
+                         f"{seeds.device}")
+    for v, name in ((noise, "noise"), (x_t, "x_t"), (eps, "eps")):
+        if v is not None and v.shape != x_start.shape:
+            raise ValueError(f"q_sample: {name} {tuple(v.shape)} != x_start {tuple(x_start.shape)}")
+    if sqrt_acp.numel() != sqrt_1m_acp.numel():
+        raise ValueError("q_sample: the two schedule tables differ in length")
+    if (x_start.numel() // B) % 4:
+        raise ValueError("q_sample: elements per sample must be a multiple of 4")
+    rec.emit("extdm_q_sample", (_p(x_start), _p(t), _p(seeds), _p(noise), _p(sqrt_acp), _p(sqrt_1m_acp), _p(x_t),
+                                _p(eps), B, x_start.numel() // B),
+             keep=(x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t, eps))
+
+
+def denoise_loss(rec, eps, pred, out, l1=False):
+    """out (B, tp) = mean over (3, h, w) of (eps - pred)^2, or |eps - pred| with l1, per (video, frame) of eps, pred
+    (B, 3, tp, h, w)."""
+    _chk(eps, torch.float32, "eps")
+    _chk(pred, torch.float32, "pred")
+    _chk(out, torch.float32, "out")
+    if eps.dim() != 5 or eps.shape[1] != 3 or pred.shape != eps.shape:
+        raise ValueError(f"denoise_loss: eps and pred must be one (B, 3, tp, h, w) shape, got {tuple(eps.shape)} and "
+                         f"{tuple(pred.shape)}")
+    B, _, tp, h, w = eps.shape
+    if tuple(out.shape) != (B, tp):
+        raise ValueError(f"denoise_loss: out must be ({B}, {tp}), got {tuple(out.shape)}")
+    rec.emit("extdm_denoise_loss", (_p(eps), _p(pred), _p(out), B, tp, 3 * h * w, int(bool(l1))),
+             keep=(eps, pred, out))
+
+
 # ----------------------------------------------------------------------------- LFAE decode
 def warp_blend_cl(rec, skip, prev, flow, occ, out, up2=False):
     """skip (Fs,H,W,C) bf16, prev (F,H,W,C) or None, flow (F,h,w,2) fp32, occ (F,1,h,w) fp32 or None."""

@@ -175,6 +175,7 @@ class UnetRunner:
         self.taps = {}                      # name -> buffer, for layer-by-layer parity tests
         self.ddim_graphs = {}               # CUDA graphs of the sampling loop over these buffers (GaussianDiffusion)
         self.ddpm_graphs = {}               # CUDA graphs of one ancestral-sampler iteration (GaussianDiffusion)
+        self.loss_graphs = {}               # CUDA graphs of the denoising-loss evaluation (GaussianDiffusion)
         self._build()
 
     # ------------------------------------------------------------------ helpers

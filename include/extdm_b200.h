@@ -299,7 +299,9 @@ int extdm_ddim_update_seeded(const float* img, const float* pred, const long lon
  * Noise is Philox4x32-10 + Box-Muller with key = the video's seed and counter = (element index / 4 within the video,
  * step, stream, 0); stream 0 is the noise of loop step `step`, stream 1 the initial x_T.  The DDIM sampler with
  * per-video seeds (extdm_ddim_update_seeded) uses the same counter layout: x_T from stream 1, the noise of DDIM
- * iteration i from (step = i, stream 0).
+ * iteration i from (step = i, stream 0).  Stream 2 is the epsilon of the denoising-loss evaluation (extdm_q_sample):
+ * counter (element index / 4 within the video, t[b], 2, 0), so a video's epsilon depends on its seed and its timestep
+ * only, and every timestep of a loss curve draws its own.
  */
 
 /* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
@@ -319,6 +321,26 @@ int extdm_ddpm_fill_normal(const long long* seeds, float* out, int B, int n, voi
 int extdm_ddpm_broadcast_row(const float* table, const int* step, float* out, int B, int n, void* stream);
 /* *step += 1; time[0..B) = times[*step] while *step < n_steps (one block). */
 int extdm_ddpm_advance(int* step, const long long* times, int n_steps, long long* time, int B, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Denoising-loss evaluation (GaussianDiffusion.denoising_loss: the forward of Diffusion.py p_losses, :286-319, under
+ * no_grad), fp32.  Added under ABI version 5 (backward compatible).
+ */
+
+/* Forward diffusion q(x_t | x_0): x_t_out = sqrt_acp[t[b]] * x_start + sqrt_1m_acp[t[b]] * eps, two roundings and one
+ * sum (no FMA), bit-exact against the torch fp32 expression.  eps is read from `noise` when noise != NULL, else it is
+ * the Philox draw of (seeds[b], t[b], stream 2) documented above; eps_out receives it.  x_start, noise, x_t_out,
+ * eps_out: (B, n) fp32; t, seeds: (B,) int64 with every t[b] in [0, length of the tables) -- the caller checks it;
+ * sqrt_acp, sqrt_1m_acp: the fp32 sqrt_alphas_cumprod / sqrt_one_minus_alphas_cumprod buffers. */
+int extdm_q_sample(const float* x_start, const long long* t, const long long* seeds, const float* noise,
+                   const float* sqrt_acp, const float* sqrt_1m_acp, float* x_t_out, float* eps_out, int B, int n,
+                   void* stream);
+/* out (B, tp) fp32 = mean over (3, h*w) of (eps - pred)^2 (l1 == 0) or |eps - pred| (l1 != 0) per (video, frame) of
+ * eps, pred (B, 3, tp, h*w) fp32; per_frame = 3*h*w elements of one (video, frame).  Terms and sum in fp64, one block
+ * per (video, frame) with a fixed reduction tree: repeated calls are bit-identical and out[b] depends on video b's
+ * data only. */
+int extdm_denoise_loss(const float* eps, const float* pred, float* out, int B, int tp, int per_frame, int l1,
+                       void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * LFAE decode (Generator.forward_with_flow / deform_input / apply_optical, model/LFAE/generator.py:63-93,
