@@ -7,6 +7,8 @@
 // DDIM with per-video seeds draws its noise from the same Philox generator inside the update.
 // The denoising-loss evaluation (GaussianDiffusion.denoising_loss) draws its epsilon from that generator too (stream 2)
 // in the forward-diffusion kernel, and reduces the per-(video, frame) loss in a fixed order.
+// DPM-Solver++(2M) (GaussianDiffusion.dpm_solver_sample) reuses the DDIM threshold and x_start math, and draws the noise
+// of its stochastic variant from that generator too (stream 3).
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -252,6 +254,53 @@ __global__ void __launch_bounds__(256) ddim_update_seeded_kernel(const float* __
   }
 }
 
+// ------------------------------------------------------------------------------------------------ DPM-Solver++(2M)
+// Philox counter word 2 of the solver's per-iteration noise (dpmpp_2m_sde); word 1 is the iteration i
+constexpr unsigned int kStreamSolver = 3u;
+
+// One multistep iteration: D = clamp(c_recip*img - c_recipm1*pred, -s, s) / s as ddim_quad computes it, then
+// out = ((A*img + B*D) + C*d_prev) + N*z, each product rounded on its own and summed left to right (no FMA).  The C term
+// is left out when d_prev is NULL (the first, first-order step), the N term when there is no noise source (the ODE
+// solver).  final: out = D.  d_out receives D; it may alias d_prev, as img_out may alias img: each thread reads its
+// four elements before it writes them.
+__global__ void __launch_bounds__(256) dpmpp_update_kernel(const float* __restrict__ img,
+                                                           const float* __restrict__ pred,
+                                                           const float* d_prev,
+                                                           const long long* __restrict__ seeds,
+                                                           const float* __restrict__ noise, unsigned int step,
+                                                           const float* __restrict__ s, float c_recip,
+                                                           float c_recipm1, float A, float B, float C, float N,
+                                                           int final, float* img_out, float* d_out,
+                                                           int n4_per_sample, long long total4) {
+  const bool with_noise = !final && (noise != nullptr || seeds != nullptr);
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    const float sb = __ldg(s + b);
+    const float4 x = reinterpret_cast<const float4*>(img)[i];
+    const float4 e = reinterpret_cast<const float4*>(pred)[i];
+    float4 dp = make_float4(0.f, 0.f, 0.f, 0.f), z = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (d_prev && !final) dp = reinterpret_cast<const float4*>(d_prev)[i];
+    if (with_noise)
+      z = noise ? reinterpret_cast<const float4*>(noise)[i]
+                : normal4(__ldg(seeds + b), static_cast<unsigned int>(i - b * n4_per_sample), step, kStreamSolver);
+    float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, pv[4] = {dp.x, dp.y, dp.z, dp.w},
+          zv[4] = {z.x, z.y, z.z, z.w}, o[4], dv[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
+      v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+      dv[j] = v;
+      float r = __fadd_rn(__fmul_rn(A, xv[j]), __fmul_rn(B, v));
+      if (d_prev) r = __fadd_rn(r, __fmul_rn(C, pv[j]));
+      if (with_noise) r = __fadd_rn(r, __fmul_rn(N, zv[j]));
+      o[j] = final ? v : r;
+    }
+    reinterpret_cast<float4*>(img_out)[i] = make_float4(o[0], o[1], o[2], o[3]);
+    reinterpret_cast<float4*>(d_out)[i] = make_float4(dv[0], dv[1], dv[2], dv[3]);
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ denoising loss
 // Philox counter word 2 of the loss evaluation's epsilon; word 1 is the video's timestep t[b]
 constexpr unsigned int kStreamLoss = 2u;
@@ -382,6 +431,23 @@ extern "C" int extdm_ddim_update_seeded(const float* img, const float* pred, con
   ddim_update_seeded_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       img, pred, seeds, static_cast<unsigned int>(step), s, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out,
       x_start_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_dpmpp_update(const float* img, const float* pred, const float* d_prev, const long long* seeds,
+                                  const float* noise, int step, const float* s, float c_recip, float c_recipm1,
+                                  float A, float B_coef, float C_coef, float N, int final, float* img_out,
+                                  float* d_out, int B, int n, void* stream) {
+  if (n % 4 || n < 4 || B < 1 || step < 0 || !s || !img_out || !d_out || (seeds && noise)) {
+    extdm_set_error("dpmpp_update: need n % 4 == 0, B >= 1, step >= 0, s, both outputs and not both seeds and noise",
+                    __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  dpmpp_update_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      img, pred, d_prev, seeds, noise, static_cast<unsigned int>(step), s, c_recip, c_recipm1, A, B_coef, C_coef, N,
+      final != 0, img_out, d_out, n / 4, total4);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

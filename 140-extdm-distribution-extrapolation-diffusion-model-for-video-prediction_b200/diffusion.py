@@ -8,15 +8,27 @@ With `seeds` (one int64 per video) DDIM draws its noise inside the update kernel
 video's seed, so a video's sample does not depend on the rest of its batch and no noise tensor is stored.
 sampling_timesteps == timesteps (or None) selects the ancestral sampler, whose loop is too long for one graph: ONE
 iteration is captured and replayed timesteps times, with its per-step values on the device.
+`solver="dpmpp_2m"` / `"dpmpp_2m_sde"` selects DPM-Solver++(2M) instead (dpm_solver_sample): sampling_timesteps UNet
+evaluations on DDIM's timestep grid, the whole loop captured as one CUDA graph as for DDIM.
 `denoising_loss()` evaluates the training objective of p_losses (Diffusion.py:286-319) forward-only, under no_grad:
 forward diffusion to one timestep per video, one UNet forward, the per-(video, frame) loss, as one CUDA graph.
 Training itself (gradients, optimisers) is out of scope.
 """
+import math
+import struct
+
 import torch
 import torch.nn.functional as F
 from torch import nn
 
 from . import ops
+
+SOLVERS = ("dpmpp_2m", "dpmpp_2m_sde")
+
+
+def _f32(v):
+    """v rounded to the nearest fp32, as a Python float."""
+    return struct.unpack("f", struct.pack("f", v))[0]
 
 
 def _seed_vector(seeds, noise, B, who):
@@ -87,8 +99,9 @@ def _schedule_tables(timesteps, s=0.008):
 class GaussianDiffusion(nn.Module):
     def __init__(self, denoise_fn, *, image_size, num_frames, text_use_bert_cls=False, channels=3, timesteps=1000,
                  sampling_timesteps=250, ddim_sampling_eta=1.0, loss_type="l1", use_dynamic_thres=True,
-                 dynamic_thres_percentile=0.9, null_cond_prob=0.1):
+                 dynamic_thres_percentile=0.9, null_cond_prob=0.1, solver=None):
         super().__init__()
+        self.solver = solver
         self.denoise_fn = denoise_fn
         self.image_size, self.num_frames, self.channels = image_size, num_frames, channels
         self.null_cond_prob, self.loss_type = null_cond_prob, loss_type
@@ -101,6 +114,18 @@ class GaussianDiffusion(nn.Module):
         self.use_dynamic_thres = use_dynamic_thres
         self.dynamic_thres_percentile = dynamic_thres_percentile
         self.use_cuda_graph = True
+
+    @property
+    def solver(self):
+        """None (DDIM or the ancestral sampler, by sampling_timesteps), "dpmpp_2m" (DPM-Solver++(2M), probability-flow
+        ODE) or "dpmpp_2m_sde" (its stochastic variant); see dpm_solver_sample."""
+        return self._solver
+
+    @solver.setter
+    def solver(self, value):
+        if value is not None and value not in SOLVERS:
+            raise ValueError(f"solver must be None or one of {SOLVERS}, got {value!r}")
+        self._solver = value
 
     # ------------------------------------------------------------------ schedule scalars (host, fp32)
     def ddim_schedule(self):
@@ -124,9 +149,12 @@ class GaussianDiffusion(nn.Module):
     # ------------------------------------------------------------------ sampling
     @torch.no_grad()
     def sample(self, x_cond, cond_fea, cond=None, cond_scale=1.0, batch_size=16, noise=None, seeds=None):
-        """seeds: optional (B,) int64 tensor or list, one seed per video (see ddim_sample / p_sample_loop)."""
+        """seeds: optional (B,) int64 tensor or list, one seed per video (see ddim_sample / p_sample_loop /
+        dpm_solver_sample)."""
         B = x_cond.shape[0]
         shape = (B, 3, self.num_frames - x_cond.size(2), x_cond.shape[3], x_cond.shape[4])
+        if self.solver is not None:
+            return self.dpm_solver_sample(x_cond, shape, cond_fea, noise=noise, seeds=seeds)
         if not self.is_ddim_sampling:
             return self.p_sample_loop(x_cond, shape, cond_fea, noise=noise, seeds=seeds)
         return self.ddim_sample(x_cond, shape, cond_fea=cond_fea, cond=cond, cond_scale=cond_scale, noise=noise,
@@ -344,6 +372,149 @@ class GaussianDiffusion(nn.Module):
         if trace is not None:
             trace[-1].update(x_start=xs, s=st["s"].clone(), img=r.x.clone())
         ops.ddpm_advance(rec, st["step"], st["times"], r.time)
+
+    # ------------------------------------------------------------------ DPM-Solver++(2M)
+    def _solver_times(self):
+        """t_0 > ... > t_S = 0, the grid of ddim_schedule (host only, no device access); ValueError when no solver is
+        selected or the grid is not strictly decreasing."""
+        if self.solver is None:
+            raise ValueError("solver_schedule: no solver is selected")
+        T, S = self.num_timesteps, int(self.sampling_timesteps)
+        times = list(reversed(torch.linspace(0.0, T, steps=S + 2)[:-1].int().tolist())) if S >= 1 else []
+        if S < 1 or any(a <= b for a, b in zip(times, times[1:])):
+            raise ValueError(f"{self.solver}: the grid of {S} steps over {T} timesteps is not strictly decreasing "
+                             f"(need 1 <= sampling_timesteps < timesteps, and well below it): {times}")
+        return times
+
+    def solver_schedule(self):
+        """[(t_i, c_recip, c_recipm1, A, B, C, N, final)] for i < S = sampling_timesteps, DESIGN.md section 1.
+
+        The UNet is evaluated at t_0 > ... > t_{S-1}, the timesteps of ddim_schedule.  With alpha_i, sigma_i =
+        sqrt_alphas_cumprod[t_i], sqrt_one_minus_alphas_cumprod[t_i] (the convention of q_sample, not DDIM's
+        alphas_cumprod_prev indexing), lambda_i = log alpha_i - log sigma_i, h = lambda_{i+1} - lambda_i and
+        r = h_{i-1} / h, iteration i < S - 1 maps x to A*x + B*D_i + C*D_{i-1} + N*z (D = thresholded x0 prediction):
+            dpmpp_2m:     A = sigma_{i+1}/sigma_i,          G = -alpha_{i+1} expm1(-h),  N = 0
+            dpmpp_2m_sde: A = sigma_{i+1}/sigma_i e^{-h},   G = -alpha_{i+1} expm1(-2h), N = sigma_{i+1} sqrt(-expm1(-2h))
+            B = G (1 + 1/(2r)), C = -G/(2r); at i = 0 B = G, C = 0.
+        The last row is final: its output is D_{S-1}.  Computed in float64 from the fp32 buffers (a checkpoint may
+        overwrite them), each coefficient rounded to fp32 once; c_recip / c_recipm1 are the fp32 buffer values."""
+        times, S = self._solver_times(), int(self.sampling_timesteps)
+        alpha = self.sqrt_alphas_cumprod.detach().cpu().double()
+        sigma = self.sqrt_one_minus_alphas_cumprod.detach().cpu().double()
+        recip = self.sqrt_recip_alphas_cumprod.detach().cpu()
+        recipm1 = self.sqrt_recipm1_alphas_cumprod.detach().cpu()
+        lam = [math.log(alpha[t].item()) - math.log(sigma[t].item()) for t in times[:S]]
+        sde = self.solver == "dpmpp_2m_sde"
+        rows, h_prev = [], None
+        for i, t in enumerate(times[:S]):
+            if i == S - 1:
+                rows.append((t, recip[t].item(), recipm1[t].item(), 0.0, 1.0, 0.0, 0.0, True))
+                break
+            t1 = times[i + 1]
+            a1, s0, s1 = alpha[t1].item(), sigma[t].item(), sigma[t1].item()
+            h = lam[i + 1] - lam[i]
+            if sde:
+                A, G, N = s1 / s0 * math.exp(-h), -a1 * math.expm1(-2.0 * h), s1 * math.sqrt(-math.expm1(-2.0 * h))
+            else:
+                A, G, N = s1 / s0, -a1 * math.expm1(-h), 0.0
+            if h_prev is None:
+                B, C = G, 0.0
+            else:
+                r = h_prev / h
+                B, C = G * (1.0 + 1.0 / (2.0 * r)), -G / (2.0 * r)
+            rows.append((t, recip[t].item(), recipm1[t].item(), _f32(A), _f32(B), _f32(C), _f32(N), False))
+            h_prev = h
+        return rows
+
+    @torch.no_grad()
+    def dpm_solver_sample(self, x_cond, shape, cond_fea, noise=None, seeds=None, trace=None):
+        """DPM-Solver++(2M) with dynamic thresholding (self.solver: "dpmpp_2m" or "dpmpp_2m_sde"), S =
+        sampling_timesteps UNet evaluations; solver_schedule holds the per-step coefficients.  Returns the final img
+        (the thresholded x0 of the last step, |img| <= 1), as ddim_sample.
+
+        x_T is the Philox draw of each video's seed (stream 1, as DDIM with seeds and the ancestral sampler), the noise
+        z of iteration i (dpmpp_2m_sde only) the draw of (seed, i, stream 3) (include/extdm_b200.h).  seeds: optional
+        (B,) int64 tensor or list; default: seeds drawn from torch's default generator, as p_sample_loop does.
+        noise: optional (S, *shape) tensor instead of seeds; noise[0] is x_T and noise[1 + i] the z of iteration i.
+        trace: list that receives per-step tensors (tests).
+
+        The whole loop (UNet prologue, x_T, S x (UNet step, threshold, update)) is one CUDA graph per shape, solver, S,
+        T, percentile and injected-or-not, kept on the UNet runner (solver_graphs); the seeds (or the noise) are
+        copied in before each replay without a host synchronisation, so one capture serves every seed vector."""
+        B = shape[0]
+        seeds = _seed_vector(seeds, noise, B, "dpm_solver_sample")
+        S = len(self._solver_times()) - 1
+        if noise is not None and (not torch.is_tensor(noise) or not noise.is_floating_point()
+                                  or tuple(noise.shape) != (S, *shape)):
+            raise ValueError(f"dpm_solver_sample: noise must be a float tensor of shape {(S, *shape)}, got "
+                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
+        if not self.use_dynamic_thres:
+            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
+        if x_cond.device.type != "cuda":
+            raise RuntimeError("dpm_solver_sample runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        if noise is None and seeds is None:
+            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
+
+        def state():
+            return dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if noise is None else None,
+                        noise=torch.zeros(S, *shape, device=r.dev) if noise is not None else None,
+                        s=torch.zeros(B, device=r.dev), d=torch.zeros(shape, device=r.dev))
+
+        def stage(st):
+            r.set_conditioning(x_cond.float(), cond_fea.float())
+            if noise is None:
+                _load_seeds(st["seeds"], seeds)                            # no host sync before the launches / replay
+            else:
+                st["noise"].copy_(noise)
+
+        if trace is not None or not self.use_cuda_graph:
+            st = state()
+            stage(st)
+            return self._solver_loop(r, self.solver_schedule(), st, trace).clone()
+        # like ddim_graphs the graph points into the runner's buffers (and bakes in the coefficients), so it lives on
+        # the runner and its key holds what selects the coefficients
+        key = (tuple(shape), self.solver, S, self.num_timesteps, float(self.dynamic_thres_percentile),
+               noise is not None)
+        if key not in r.solver_graphs:
+            sched = self.solver_schedule()               # reads the buffers on the host: only when capturing
+            st = state()
+            stage(st)
+            self._solver_loop(r, sched, st)                                 # warm-up (lazy inits)
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._solver_loop(r, sched, st)
+            r.solver_graphs[key] = (g, st)
+        g, st = r.solver_graphs[key]
+        stage(st)
+        g.replay()
+        return r.x.clone()
+
+    def _solver_loop(self, r, sched, st, trace=None):
+        """UNet prologue, x_T, then per step: UNet step, threshold, dpmpp_update (D kept in st["d"] for the next)."""
+        rec = ops.IMMEDIATE
+        r.run_prologue()
+        if st["noise"] is None:
+            ops.ddpm_fill_normal(rec, st["seeds"], r.x)
+        else:
+            r.x.copy_(st["noise"][0])
+        q = float(self.dynamic_thres_percentile)
+        sde = self.solver == "dpmpp_2m_sde"
+        ss = r.ss_for_times([row[0] for row in sched])       # evaluated once per schedule, outside the captured loop
+        for i, (t, c_recip, c_recipm1, A, Bc, Cc, N, final) in enumerate(sched):
+            r.run_step(ss[i])
+            ops.ddim_threshold(rec, r.x, r.out, c_recip, c_recipm1, q, st["s"])
+            if trace is not None:
+                trace.append(dict(img_in=r.x.clone(), pred_noise=r.out.clone()))
+            noisy = sde and not final
+            nz = st["noise"][1 + i] if noisy and st["noise"] is not None else None
+            seeds = st["seeds"] if noisy and nz is None else None
+            ops.dpmpp_update(rec, r.x, r.out, st["d"] if i else None, seeds, nz, i, st["s"], c_recip, c_recipm1,
+                             A, Bc, Cc, N, final, r.x, st["d"])
+            if trace is not None:
+                trace[-1].update(x_start=st["d"].clone(), s=st["s"].clone(), img=r.x.clone())
+        return r.x
 
     # ------------------------------------------------------------------ denoising loss (forward-only p_losses)
     def loss_args(self, B, shape, timesteps=None, seeds=None, noise=None, who="denoising_loss"):

@@ -83,7 +83,8 @@ class FlowDiffusion(nn.Module):
             self.unet, image_size=dataset_params["frame_shape"] // 2, num_frames=tc + tp,
             sampling_timesteps=diffusion_params["sampling_timesteps"], timesteps=timesteps,
             loss_type=diffusion_params["loss_type"], use_dynamic_thres=True,
-            null_cond_prob=diffusion_params["null_cond_prob"], ddim_sampling_eta=ddim_sampling_eta).to(dev)
+            null_cond_prob=diffusion_params["null_cond_prob"], ddim_sampling_eta=ddim_sampling_eta,
+            solver=diffusion_params.get("solver")).to(dev)
         self.cond_frame_num, self.pred_frame_num, self.frame_num = tc, tp, tc + tp
         self._cond_runners = {}
         for m in (self.generator, self.region_predictor, self.bg_predictor):

@@ -84,6 +84,7 @@ PROTOTYPES = {
     "extdm_ddpm_fill_normal": [_P, _P, _I, _I, _P],
     "extdm_ddpm_broadcast_row": [_P, _P, _P, _I, _I, _P],
     "extdm_ddpm_advance": [_P, _P, _I, _P, _I, _P],
+    "extdm_dpmpp_update": [_P, _P, _P, _P, _P, _I, _P, _F, _F, _F, _F, _F, _F, _I, _P, _P, _I, _I, _P],
     "extdm_q_sample": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P],
     "extdm_denoise_loss": [_P, _P, _P, _I, _I, _I, _I, _P],
     "extdm_warp_blend_cl": [_P, _P, _P, _P, _P, _L, _L, _I, _I, _I, _I, _I, _I, _P],

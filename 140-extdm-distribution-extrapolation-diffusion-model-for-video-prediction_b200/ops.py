@@ -599,6 +599,35 @@ def ddpm_advance(rec, step, times, time):
              keep=(step, times, time))
 
 
+def dpmpp_update(rec, img, pred, d_prev, seeds, noise, step, s, c_recip, c_recipm1, coef_a, coef_b, coef_c, coef_n,
+                 final, img_out, d_out):
+    """One DPM-Solver++(2M) iteration: D = clamp(c_recip*img - c_recipm1*pred, -s, s)/s into d_out, img_out =
+    coef_a*img + coef_b*D + coef_c*d_prev + coef_n*z (d_prev None: no coef_c term; seeds and noise None: no coef_n term; z = noise, or the Philox
+    draw of (seeds[b], step, stream 3)); final: img_out = D."""
+    for v, name in ((img, "img"), (pred, "pred"), (s, "s"), (img_out, "img_out"), (d_out, "d_out")):
+        if v is None:
+            raise ValueError(f"dpmpp_update: {name} is required")
+        _chk(v, torch.float32, name)
+    _chk(d_prev, torch.float32, "d_prev")
+    _chk(seeds, torch.int64, "seeds")
+    _chk(noise, torch.float32, "noise")
+    B_ = img.shape[0]
+    if seeds is not None and noise is not None:
+        raise ValueError("dpmpp_update: pass seeds or noise, not both")
+    for v, name in ((pred, "pred"), (d_prev, "d_prev"), (noise, "noise"), (img_out, "img_out"), (d_out, "d_out")):
+        if v is not None and v.shape != img.shape:
+            raise ValueError(f"dpmpp_update: {name} {tuple(v.shape)} != img {tuple(img.shape)}")
+    if s.numel() != B_ or (seeds is not None and (seeds.numel() != B_ or seeds.device != img.device)):
+        raise ValueError(f"dpmpp_update: s and seeds must hold {B_} values on {img.device}")
+    if (img.numel() // B_) % 4 or int(step) < 0:
+        raise ValueError("dpmpp_update: elements per sample must be a multiple of 4 and step >= 0")
+    rec.emit("extdm_dpmpp_update", (_p(img), _p(pred), _p(d_prev), _p(seeds), _p(noise), int(step), _p(s),
+                                    C.c_float(c_recip), C.c_float(c_recipm1), C.c_float(coef_a), C.c_float(coef_b),
+                                    C.c_float(coef_c), C.c_float(coef_n), int(bool(final)), _p(img_out), _p(d_out), B_,
+                                    img.numel() // B_),
+             keep=(img, pred, d_prev, seeds, noise, s, img_out, d_out))
+
+
 def q_sample(rec, x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t, eps):
     """x_t = sqrt_acp[t[b]] * x_start + sqrt_1m_acp[t[b]] * eps, eps = noise when given, else the Philox draw of
     (seeds[b], t[b], stream 2); eps is written too.  t must lie in [0, len(sqrt_acp)): the kernel indexes the tables

@@ -176,6 +176,7 @@ class UnetRunner:
         self.ddim_graphs = {}               # CUDA graphs of the sampling loop over these buffers (GaussianDiffusion)
         self.ddpm_graphs = {}               # CUDA graphs of one ancestral-sampler iteration (GaussianDiffusion)
         self.loss_graphs = {}               # CUDA graphs of the denoising-loss evaluation (GaussianDiffusion)
+        self.solver_graphs = {}             # CUDA graphs of the DPM-Solver++(2M) sampling loop (GaussianDiffusion)
         self._build()
 
     # ------------------------------------------------------------------ helpers

@@ -301,7 +301,8 @@ int extdm_ddim_update_seeded(const float* img, const float* pred, const long lon
  * per-video seeds (extdm_ddim_update_seeded) uses the same counter layout: x_T from stream 1, the noise of DDIM
  * iteration i from (step = i, stream 0).  Stream 2 is the epsilon of the denoising-loss evaluation (extdm_q_sample):
  * counter (element index / 4 within the video, t[b], 2, 0), so a video's epsilon depends on its seed and its timestep
- * only, and every timestep of a loss curve draws its own.
+ * only, and every timestep of a loss curve draws its own.  Stream 3 is the noise of the stochastic DPM-Solver++(2M)
+ * (extdm_dpmpp_update): iteration i draws counter (element index / 4 within the video, i, 3, 0); its x_T is stream 1.
  */
 
 /* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
@@ -321,6 +322,23 @@ int extdm_ddpm_fill_normal(const long long* seeds, float* out, int B, int n, voi
 int extdm_ddpm_broadcast_row(const float* table, const int* step, float* out, int B, int n, void* stream);
 /* *step += 1; time[0..B) = times[*step] while *step < n_steps (one block). */
 int extdm_ddpm_advance(int* step, const long long* times, int n_steps, long long* time, int B, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * DPM-Solver++(2M) sampler (GaussianDiffusion.dpm_solver_sample; Lu et al. 2022, data prediction with dynamic
+ * thresholding), fp32.  Added under ABI version 5 (backward compatible).
+ */
+
+/* One iteration after the threshold (extdm_ddim_threshold with the same c_recip, c_recipm1 and s):
+ *   D       = clamp(c_recip*img - c_recipm1*pred, -s[b], s[b]) / s[b]          (as extdm_ddim_update's x_start)
+ *   img_out = ((A*img + B_coef*D) + C_coef*d_prev) + N*z                       (each product rounded, no FMA)
+ * The C_coef term is left out when d_prev == NULL (first step), the N term when seeds and noise are both NULL (the
+ * deterministic solver).  z is read from noise ((B, n)) when given, else it is the Philox draw of (seeds[b], step,
+ * stream 3) documented above.  final != 0: img_out = D and no noise is drawn.  d_out receives D and may equal d_prev;
+ * img_out may equal img.  seeds and noise are not both given. */
+int extdm_dpmpp_update(const float* img, const float* pred, const float* d_prev, const long long* seeds,
+                       const float* noise, int step, const float* s, float c_recip, float c_recipm1, float A,
+                       float B_coef, float C_coef, float N, int final, float* img_out, float* d_out, int B, int n,
+                       void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Denoising-loss evaluation (GaussianDiffusion.denoising_loss: the forward of Diffusion.py p_losses, :286-319, under
