@@ -9,6 +9,8 @@
 // in the forward-diffusion kernel, and reduces the per-(video, frame) loss in a fixed order.
 // DPM-Solver++(2M) (GaussianDiffusion.dpm_solver_sample) reuses the DDIM threshold and x_start math, and draws the noise
 // of its stochastic variant from that generator too (stream 3).
+// Interpolation between two futures (GaussianDiffusion.interpolate) mixes their forward diffusions in one kernel, with
+// each endpoint's epsilon from that generator (streams 4 and 5), then runs the DDIM or ancestral loop above.
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -335,6 +337,46 @@ __global__ void __launch_bounds__(256) q_sample_kernel(const float* __restrict__
   }
 }
 
+// ------------------------------------------------------------------------------------------------ interpolation
+// Philox counter word 2 of the two endpoints' epsilon in GaussianDiffusion.interpolate; word 1 is the mix timestep t
+constexpr unsigned int kStreamInterp1 = 4u, kStreamInterp2 = 5u;
+
+// x_t = c1 * q(x1, eps1) + c2 * q(x2, eps2) at one timestep t shared by the batch, q as q_sample_of; every product
+// rounded on its own and each sum of two (no FMA), as torch evaluates `(1 - lam) * (...) + lam * (...)` in fp32.
+// eps1, eps2 are noise[i] and noise[total4 + i] when noise is given, else the Philox draws of streams 4 and 5.
+__global__ void __launch_bounds__(256) q_interpolate_kernel(const float* __restrict__ x1, const float* __restrict__ x2,
+                                                            int t, const long long* __restrict__ seeds,
+                                                            const float* __restrict__ noise,
+                                                            const float* __restrict__ sqrt_acp,
+                                                            const float* __restrict__ sqrt_1m_acp, float c1, float c2,
+                                                            float* __restrict__ x_t, int n4_per_sample,
+                                                            long long total4) {
+  const float a = __ldg(sqrt_acp + t), c = __ldg(sqrt_1m_acp + t);
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    float4 e1, e2;
+    if (noise) {
+      e1 = reinterpret_cast<const float4*>(noise)[i];
+      e2 = reinterpret_cast<const float4*>(noise)[total4 + i];
+    } else {
+      const long long b = i / n4_per_sample;
+      const long long sd = __ldg(seeds + b);
+      const unsigned int quad = static_cast<unsigned int>(i - b * n4_per_sample);
+      e1 = normal4(sd, quad, static_cast<unsigned int>(t), kStreamInterp1);
+      e2 = normal4(sd, quad, static_cast<unsigned int>(t), kStreamInterp2);
+    }
+    const float4 u = reinterpret_cast<const float4*>(x1)[i], v = reinterpret_cast<const float4*>(x2)[i];
+    const float uv[4] = {u.x, u.y, u.z, u.w}, vv[4] = {v.x, v.y, v.z, v.w};
+    const float e1v[4] = {e1.x, e1.y, e1.z, e1.w}, e2v[4] = {e2.x, e2.y, e2.z, e2.w};
+    float o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      o[j] = __fadd_rn(__fmul_rn(c1, q_sample_of(uv[j], e1v[j], a, c)),
+                       __fmul_rn(c2, q_sample_of(vv[j], e2v[j], a, c)));
+    reinterpret_cast<float4*>(x_t)[i] = make_float4(o[0], o[1], o[2], o[3]);
+  }
+}
+
 // One block per (video b, frame f) of (B, 3, tp, hw) tensors: out[b, f] = mean over (3, hw) of (eps - pred)^2 (or
 // |eps - pred|).  The difference of two floats is exact in double, so the terms are exact and the sum is in fp64; each
 // thread sums a fixed strided subset in order, then a fixed shared-memory tree: the result depends on the (b, f) slice
@@ -510,6 +552,21 @@ extern "C" int extdm_q_sample(const float* x_start, const long long* t, const lo
   const long long total4 = static_cast<long long>(B) * n / 4;
   q_sample_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t_out, eps_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_q_interpolate(const float* x1, const float* x2, int t, const long long* seeds, const float* noise,
+                                   const float* sqrt_acp, const float* sqrt_1m_acp, float c1, float c2, float* x_t_out,
+                                   int B, int n, void* stream) {
+  if (n % 4 || n < 4 || B < 1 || t < 0 || !x1 || !x2 || (!noise == !seeds) || !sqrt_acp || !sqrt_1m_acp || !x_t_out) {
+    extdm_set_error("q_interpolate: need n % 4 == 0, B >= 1, t >= 0, both endpoints, exactly one of seeds and noise, "
+                    "both tables and the output", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const long long total4 = static_cast<long long>(B) * n / 4;
+  q_interpolate_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      x1, x2, t, seeds, noise, sqrt_acp, sqrt_1m_acp, c1, c2, x_t_out, n / 4, total4);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

@@ -12,9 +12,12 @@ iteration is captured and replayed timesteps times, with its per-step values on 
 evaluations on DDIM's timestep grid, the whole loop captured as one CUDA graph as for DDIM.
 `denoising_loss()` evaluates the training objective of p_losses (Diffusion.py:286-319) forward-only, under no_grad:
 forward diffusion to one timestep per video, one UNet forward, the per-(video, frame) loss, as one CUDA graph.
+`interpolate()` (Diffusion.py:261-274) mixes the forward diffusions of two futures at one timestep and denoises the
+mix with the DDIM or the ancestral loop.
 Training itself (gradients, optimisers) is out of scope.
 """
 import math
+import numbers
 import struct
 
 import torch
@@ -131,9 +134,13 @@ class GaussianDiffusion(nn.Module):
     def ddim_schedule(self):
         """[(time, time_next, c_recip, c_recipm1, sqrt_alpha_next, c, sigma)], evaluated with the same fp32 torch
         scalar ops as Diffusion.py:214-216, 221-222, 248-249 (note the alphas_cumprod_*prev* indexing)."""
-        total, n, eta = self.num_timesteps, self.sampling_timesteps, self.ddim_sampling_eta
+        total, n = self.num_timesteps, self.sampling_timesteps
         times = torch.linspace(0.0, total, steps=n + 2)[:-1]
-        times = list(reversed(times.int().tolist()))
+        return self._ddim_rows(list(reversed(times.int().tolist())))
+
+    def _ddim_rows(self, times):
+        """ddim_schedule's rows for the consecutive pairs (time, time_next) of `times`."""
+        eta = self.ddim_sampling_eta
         prev = self.alphas_cumprod_prev.detach().cpu()
         recip = self.sqrt_recip_alphas_cumprod.detach().cpu()
         recipm1 = self.sqrt_recipm1_alphas_cumprod.detach().cpu()
@@ -244,12 +251,17 @@ class GaussianDiffusion(nn.Module):
             r.set_conditioning(x_cond.float(), cond_fea.float())
         s = st["s"] if st is not None else torch.zeros(r.B, device=r.dev)
         seeds = st.get("seeds") if st is not None else None
-        rec = ops.IMMEDIATE
         r.run_prologue()
         if seeds is not None:
-            ops.ddpm_fill_normal(rec, seeds, r.x)
+            ops.ddpm_fill_normal(ops.IMMEDIATE, seeds, r.x)
         else:
             r.x.copy_(noise[0])
+        return self._ddim_steps(r, sched, None if noise is None else noise[1:], seeds, s, trace)
+
+    def _ddim_steps(self, r, sched, noise, seeds, s, trace=None):
+        """The DDIM iterations of sched from r.x (after the UNet prologue): the noise of iteration i is noise[i], or,
+        with seeds, the Philox draw of (seeds[b], i, stream 0)."""
+        rec = ops.IMMEDIATE
         q = float(self.dynamic_thres_percentile)
         ss = r.ss_for_times([s_[0] for s_ in sched])       # evaluated once per schedule, outside the captured loop
         for i, (time, time_next, c_recip, c_recipm1, san, c, sigma) in enumerate(sched):
@@ -257,7 +269,7 @@ class GaussianDiffusion(nn.Module):
             ops.ddim_threshold(rec, r.x, r.out, c_recip, c_recipm1, q, s)
             nz = None
             if seeds is None:
-                nz = noise[i + 1] if (time_next > 0 and i + 1 < noise.shape[0]) else None
+                nz = noise[i] if (time_next > 0 and i < noise.shape[0]) else None
                 if time_next > 0 and nz is None:
                     raise ValueError("ddim_sample: not enough noise tensors supplied")
             xs = torch.empty_like(r.x) if trace is not None else None
@@ -317,25 +329,30 @@ class GaussianDiffusion(nn.Module):
             for _ in range(T):
                 self._ddpm_iteration(r, st, trace)
             return r.x.clone()
+        g, st = self._ddpm_graph(r, shape, noise is not None,
+                                 lambda st: self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise))
+        self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
+        for _ in range(T):
+            g.replay()
+        return r.x.clone()
+
+    def _ddpm_graph(self, r, shape, injected, start):
+        """(graph, state) of one captured ancestral iteration.  start(st) sets up a round for the warm-up run."""
         # One iteration (time-MLP rows, UNet step, threshold, update, advance) is captured; its per-step values come from
         # the device tables and step counter, so the same graph serves every timestep.  Like ddim_graphs it lives on the
         # runner, whose buffers it points into.
         graphs = r.ddpm_graphs
-        key = (tuple(shape), float(self.dynamic_thres_percentile), T, noise is not None)
+        key = (tuple(shape), float(self.dynamic_thres_percentile), self.num_timesteps, injected)
         if key not in graphs:
-            st = self._ddpm_state(r, noise is not None)
-            self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)           # warm-up (lazy inits)
+            st = self._ddpm_state(r, injected)
+            start(st)                                                          # warm-up (lazy inits)
             self._ddpm_iteration(r, st)
             torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
                 self._ddpm_iteration(r, st)
             graphs[key] = (g, st)
-        g, st = graphs[key]
-        self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
-        for _ in range(T):
-            g.replay()
-        return r.x.clone()
+        return graphs[key]
 
     def _ddpm_state(self, r, injected):
         """Device state of the loop: schedule table, time-MLP rows per step, step counter, per-video seeds,
@@ -356,8 +373,12 @@ class GaussianDiffusion(nn.Module):
         else:
             r.x.copy_(noise[0])
             st["noise"].copy_(noise[1:])
-        st["step"].zero_()
-        r.time.fill_(self.num_timesteps - 1)
+        self._ddpm_start(r, st, 0)
+
+    def _ddpm_start(self, r, st, row):
+        """Point the loop at row `row` of ddpm_schedule (time num_timesteps - 1 - row): step counter and time."""
+        st["step"].fill_(row)
+        r.time.fill_(self.num_timesteps - 1 - row)
 
     def _ddpm_iteration(self, r, st, trace=None):
         rec = ops.IMMEDIATE
@@ -615,3 +636,155 @@ class GaussianDiffusion(nn.Module):
         ops.q_sample(rec, st["x_start"], r.time, st["seeds"], st["noise"], st["acp"], st["a1m"], r.x, st["eps"])
         r.run_step()
         ops.denoise_loss(rec, st["eps"], r.out, st["lpf"], l1)
+
+    # ------------------------------------------------------------------ interpolation between two futures
+    def interp_times(self, t):
+        """tau_0 = t > ... > tau_S = 0, the DDIM-mode grid of interpolate: torch.linspace(0, t, S + 1).int() reversed,
+        S = sampling_timesteps (host only).  ValueError when it is not strictly decreasing (t < S)."""
+        S = int(self.sampling_timesteps)
+        times = list(reversed(torch.linspace(0, t, S + 1).int().tolist())) if S >= 1 else []
+        if S < 1 or any(a <= b for a, b in zip(times, times[1:])):
+            raise ValueError(f"interpolate: the grid of {S} steps from t = {t} is not strictly decreasing (need "
+                             f"sampling_timesteps <= t): {times}")
+        return times
+
+    def interp_args(self, x1, x2, tc, t=None, lam=0.5, seeds=None, noise=None, who="interpolate"):
+        """Check the arguments of interpolate for tc conditioning frames on the host, before anything is launched.
+        Returns (t, lams, sweep, seeds, times): lams the list of lambda values, sweep whether lam was a list, times
+        the DDIM-mode grid (interp_times) or None in ancestral mode."""
+        if self.solver is not None:
+            raise ValueError(f"{who}: interpolation runs the DDIM or the ancestral loop, not {self.solver!r}")
+        for name, v in (("x1", x1), ("x2", x2)):
+            if not torch.is_tensor(v) or v.dim() != 5 or v.dtype != torch.float32:
+                raise ValueError(f"{who}: {name} must be a (B, 3, tp, h, w) float32 tensor")
+        if x1.shape != x2.shape:
+            raise ValueError(f"{who}: x1 {tuple(x1.shape)} and x2 {tuple(x2.shape)} differ in shape")
+        B, C, tp = x1.shape[:3]
+        if B < 1 or C != 3 or tc + tp != self.num_frames:
+            raise ValueError(f"{who}: x1 {tuple(x1.shape)}: expected (B >= 1, 3, {self.num_frames - tc}, h, w)")
+        T = self.num_timesteps
+        t = T - 1 if t is None else t
+        if isinstance(t, bool) or not isinstance(t, numbers.Integral) or not 0 <= t < T:
+            raise ValueError(f"{who}: t must be an int in [0, {T}), got {t!r}")
+        t = int(t)
+        sweep = isinstance(lam, (list, tuple))
+        lams = list(lam) if sweep else [lam]
+        if not lams or any(isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v)
+                           for v in lams):
+            raise ValueError(f"{who}: lam must be a finite float or a non-empty list of them, got {lam!r}")
+        seeds = _seed_vector(seeds, noise, B, who)
+        times = self.interp_times(t) if self.is_ddim_sampling else None
+        n_loop = t if times is None else len(times) - 2
+        if noise is not None and (not torch.is_tensor(noise) or noise.dtype != torch.float32
+                                  or tuple(noise.shape) != (2 + n_loop, *x1.shape)):
+            raise ValueError(f"{who}: noise must be a float32 tensor of shape {(2 + n_loop, *x1.shape)}, got "
+                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
+        return t, [float(v) for v in lams], sweep, seeds, times
+
+    @torch.no_grad()
+    def interpolate(self, x1, x2, x_cond, cond_fea, t=None, lam=0.5, seeds=None, noise=None):
+        """Diffusion.py:261-274 with x_cond and cond_fea passed to the denoiser by keyword (DESIGN.md section 1): mix the
+        forward diffusions of two futures x1, x2 (B, 3, tp, h, w) at timestep t (default num_timesteps - 1),
+
+            x_t = (1 - lam) * (sqrt_alphas_cumprod[t] * x1 + sqrt_one_minus_alphas_cumprod[t] * eps1)
+                + lam * (sqrt_alphas_cumprod[t] * x2 + sqrt_one_minus_alphas_cumprod[t] * eps2)       (fp32, no FMA)
+
+        then denoise it to time 0 with the loop sample() would pick (a solver is a ValueError):
+          * ancestral (sampling_timesteps == timesteps): p_sample at i = t-1, ..., 0, as the reference; the first step
+            treats x_t, mixed at t, as a sample at t - 1.  The captured iteration of p_sample_loop, started at row T - t
+            of ddpm_schedule; t = 0 returns the mix.
+          * DDIM (S = sampling_timesteps < timesteps): S DDIM steps over the pairs of interp_times(t), read as
+            ddim_schedule reads the schedule (alphas_cumprod_prev indexing), with ddim_sampling_eta.
+
+        lam: a float, or a list of K floats (a sweep): one conditioning pass and UNet prologue, one loop per value, all
+        with the same eps1, eps2 and loop noise; the result is then (K, B, 3, tp, h, w), else (B, 3, tp, h, w).
+        seeds: optional (B,) int64 tensor or list; eps1, eps2 of video b are the Philox draws of (seeds[b], t, streams
+        4 and 5) and its loop noise stream 0 keyed as in p_sample_loop (the ddpm_schedule row) or ddim_sample (the
+        iteration) (include/extdm_b200.h); default: seeds drawn from torch's default generator.  noise: optional
+        (2 + n_loop, B, 3, tp, h, w) instead of seeds: eps1, eps2, then the noise of the loop's steps (n_loop = t
+        ancestral, S - 1 DDIM: the last DDIM step adds none).
+
+        The mix is one kernel launch per value; the loop replays a CUDA graph kept on the UNet runner (the ancestral
+        iteration of ddpm_graphs, or the whole DDIM loop in interp_graphs, one per shape, t, S, eta, percentile and
+        injected-or-not).  Argument errors raise ValueError before anything runs; CPU tensors then RuntimeError."""
+        if not all(torch.is_tensor(v) and v.dim() == 5 for v in (x_cond, cond_fea)):
+            raise ValueError("interpolate: x_cond and cond_fea must be 5-D tensors")
+        tc = x_cond.shape[2]
+        t, lams, sweep, seeds, times = self.interp_args(x1, x2, tc, t, lam, seeds, noise)
+        B, _, _, h, w = x1.shape
+        if tuple(x_cond.shape) != (B, 3, tc, h, w) or cond_fea.shape[0] != B:
+            raise ValueError(f"interpolate: x_cond {tuple(x_cond.shape)}, cond_fea {tuple(cond_fea.shape)}: expected "
+                             f"({B}, 3, {tc}, {h}, {w}) and ({B}, ...)")
+        if not self.use_dynamic_thres:
+            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
+        if x1.device.type != "cuda":
+            raise RuntimeError("interpolate runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        if noise is None and seeds is None:
+            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        r = self.denoise_fn.runner(B, h, w, cond_fea.shape[-1])
+        x1, x2 = x1.to(r.dev).contiguous(), x2.to(r.dev).contiguous()
+        eps = noise[:2].to(r.dev).contiguous() if noise is not None else None
+        acp, a1m = self.sqrt_alphas_cumprod.to(r.dev), self.sqrt_one_minus_alphas_cumprod.to(r.dev)
+        T = self.num_timesteps
+
+        def begin(st):
+            """Once per call: conditioning, UNet prologue, the seeds or the loop noise."""
+            r.set_conditioning(x_cond.float(), cond_fea.float())
+            r.run_prologue()
+            if noise is None:
+                _load_seeds(st["seeds"], seeds)                          # no host sync before the launches / replays
+            elif noise.shape[0] > 2:
+                st["noise"][st["noise"].shape[0] - (noise.shape[0] - 2):].copy_(noise[2:])
+
+        def mix(st, v):
+            ops.q_interpolate(ops.IMMEDIATE, x1, x2, t, st["seeds"] if noise is None else None, eps, acp, a1m,
+                              _f32(1.0 - v), _f32(v), r.x)
+            if times is None and t > 0:
+                self._ddpm_start(r, st, T - t)
+
+        if times is None:                                               # ancestral: replays of one iteration
+            def loop():
+                for _ in range(t):
+                    run()
+            if t == 0:
+                st, run = dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev), noise=None), None
+            elif self.use_cuda_graph:
+                g, st = self._ddpm_graph(r, x1.shape, noise is not None, lambda st: (begin(st), mix(st, lams[0])))
+                run = g.replay
+            else:
+                st = self._ddpm_state(r, noise is not None)
+                run = lambda: self._ddpm_iteration(r, st)                 # noqa: E731
+        else:                                                           # DDIM: the whole loop
+            sched = self._ddim_rows(times)
+
+            def state():
+                return dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if noise is None else None,
+                            noise=torch.zeros(len(sched) - 1, *x1.shape, device=r.dev) if noise is not None else None,
+                            s=torch.zeros(B, device=r.dev))
+
+            def steps():
+                self._ddim_steps(r, sched, st["noise"], st["seeds"], st["s"])
+            if not self.use_cuda_graph:
+                st, loop = state(), steps
+            else:
+                # like ddim_graphs the graph points into the runner's buffers and bakes in the schedule scalars
+                key = self._ddim_key(x1.shape) + (t, noise is not None)
+                if key not in r.interp_graphs:
+                    st = state()
+                    begin(st)
+                    mix(st, lams[0])
+                    steps()                                             # warm-up (lazy inits)
+                    torch.cuda.synchronize()
+                    g = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(g):
+                        steps()
+                    r.interp_graphs[key] = (g, st)
+                g, st = r.interp_graphs[key]
+                loop = g.replay
+        begin(st)
+        outs = []
+        for v in lams:
+            mix(st, v)
+            loop()
+            outs.append(r.x.clone())
+        return torch.stack(outs) if sweep else outs[0]

@@ -17,6 +17,11 @@ The diffusion model's own training objective on held-out clips of tc + tp frames
 timestep):
 
     out = evaluate.denoising_loss_videos(model, real_vids, timesteps=[100, 500, 900], seed=0)
+
+Interpolation between two futures of the same past (e.g. the encoded ground truth and a sample), decoded to RGB:
+
+    x1 = model.encode_future(real_vids);  x2 = model.diffusion.sample(...)    # (B, 3, tp, h, w) latents
+    origin, result = evaluate.interpolate_videos(model, real_vids, x1, x2, lams=[0.0, 0.25, 0.5, 0.75, 1.0], seed=0)
 """
 import os
 
@@ -124,6 +129,30 @@ def denoising_loss_videos(model, real_vids, timesteps=None, seed=None, video_off
     if not curve:
         return {k: v.cpu() for k, v in outs[0].items()}
     return {k: torch.stack([o[k] for o in outs], dim=1).cpu() for k in outs[0]}
+
+
+@torch.no_grad()
+def interpolate_videos(model, real_vids, x1, x2, lams, t=None, seed=None, video_offset=0):
+    """FlowDiffusion.interpolate_one_video over real_vids (B, C, >= tc, H, W) in [0, 1] and the futures x1, x2 (B, 3,
+    tp, h, w) (any device) -> (origin, result) in the layout of sample_videos, both (B, K, T', C, H, W) on the CPU:
+    result[:, k] = the cond frames followed by the tp frames decoded from the interpolation at lams[k] (lams: a list
+    of K floats, or one float for K = 1), origin[:, k] = real_vids.  psnr_videos / ssim_videos / summarize /
+    save_results apply unchanged.  t: as GaussianDiffusion.interpolate.
+
+    seed: optional int.  Then video b, whose *global* index is g = video_offset + b, is interpolated with the seed
+    sharding.video_seeds(seed, g, 2), so a sharded evaluation that passes video_offset = lo of sharding.shard_range
+    equals a single-GPU run.  Default: seeds from torch's default generator."""
+    from .sharding import video_seeds
+    B, tc = real_vids.shape[0], model.cond_frame_num
+    lams = list(lams) if isinstance(lams, (list, tuple)) else [lams]
+    seeds = video_seeds(seed, torch.arange(B) + video_offset, 2) if seed is not None else None
+    dev = next(model.parameters()).device
+    out = model.interpolate_one_video(real_vids.to(dev).float(), x1.to(dev), x2.to(dev), t=t, lam=lams, seeds=seeds)
+    pred = out["sample_out_vid"][:, :, :, tc:].cpu()                               # (K, B, 3, tp, H, W)
+    cond = real_vids[:, :, :tc].cpu().float()
+    res = torch.cat([cond.expand(len(lams), *cond.shape), pred], dim=3)
+    origin = real_vids.cpu().float().permute(0, 2, 1, 3, 4).unsqueeze(1)          # 'b c t h w -> b 1 t c h w'
+    return origin.expand(B, len(lams), *origin.shape[2:]).contiguous(), res.permute(1, 0, 3, 2, 4, 5).contiguous()
 
 
 def save_results(log_dir, origin_videos, result_videos, best_videos=None):

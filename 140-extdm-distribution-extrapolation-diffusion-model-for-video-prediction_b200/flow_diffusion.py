@@ -4,6 +4,7 @@ VideoFlowDiffusion_multi1248.py, VideoFlowDiffusion_multi.py) with the same cons
 
   (A) conditioning  : torch (RegionPredictor / BGMotionPredictor / Generator.forward), batched over the tc frames
   (B) denoise       : GaussianDiffusion.sample  -> CUDA-graphed UNet3D + DDIM kernels
+                      (interpolate_one_video: GaussianDiffusion.interpolate between two given futures)
   (C) decode        : Generator.decode_video    -> CUDA warp / blend / conv kernels
 """
 import torch
@@ -178,6 +179,12 @@ class FlowDiffusion(nn.Module):
         ret, x_cond, cond_fea, ref = self.condition(real_vid)
         pred = self.diffusion.sample(x_cond, cond_fea=cond_fea, batch_size=1, cond_scale=cond_scale, noise=noise,
                                      seeds=seeds)
+        ret.update(self._decode_sample(ret, ref, pred))
+        return ret
+
+    def _decode_sample(self, ret, ref, pred):
+        """sample_one_video's post-processing and decode of a sampled x (B, 3, tp, h, w) after condition()'s ret and
+        ref: the 'sample_*' entries of the result and the decoded conditioning frames."""
         tc = self.cond_frame_num
         grid, conf = x_start_to_flow(pred, self.use_residual_flow, self.estimate_occlusion_map)
         sample_vid_grid = torch.cat([ret["real_vid_grid"][:, :, :tc], grid], dim=2)
@@ -185,13 +192,48 @@ class FlowDiffusion(nn.Module):
         if self.estimate_occlusion_map:
             sample_vid_conf = torch.cat([ret["real_vid_conf"][:, :, :tc], conf], dim=2)
         out, warped = self.generator.decode_video(ref, sample_vid_grid, sample_vid_conf)
-        ret["sample_vid_grid"] = sample_vid_grid
+        res = {"sample_vid_grid": sample_vid_grid}
         if sample_vid_conf is not None:
-            ret["sample_vid_conf"] = sample_vid_conf
-        ret["sample_out_vid"] = out
-        ret["sample_warped_vid"] = warped
-        ret["real_out_vid"] = out[:, :, :tc]
-        ret["real_warped_vid"] = warped[:, :, :tc]
+            res["sample_vid_conf"] = sample_vid_conf
+        res["sample_out_vid"] = out
+        res["sample_warped_vid"] = warped
+        res["real_out_vid"] = out[:, :, :tc]
+        res["real_warped_vid"] = warped[:, :, :tc]
+        return res
+
+    # ------------------------------------------------------------------ interpolation between two futures
+    @torch.no_grad()
+    def encode_future(self, real_vid):
+        """The latent of the tp future frames of real_vid (B, 3, tc + tp, H, W) in [0, 1]: loss_inputs(real_vid)'s
+        x_start (B, 3, tp, h, w), in the space of what sample() returns.  Decoding it as sample_one_video decodes a
+        sample gives the LFAE reconstruction of those frames from source frame tc - 1."""
+        return self.loss_inputs(real_vid)[0]
+
+    @torch.no_grad()
+    def interpolate_one_video(self, real_vid, x1, x2, t=None, lam=0.5, seeds=None, noise=None):
+        """Condition on the first tc frames of real_vid (B, 3, >= tc, H, W) in [0, 1], interpolate between the futures
+        x1 and x2 (B, 3, tp, h, w; e.g. encode_future of a clip, or a sample) with GaussianDiffusion.interpolate (t,
+        lam, seeds, noise as there), then post-process and decode as sample_one_video.  Returns sample_one_video's
+        dict; when lam is a list of K values its 'sample_*' entries carry a leading K axis (the decoded conditioning
+        frames 'real_out_vid' / 'real_warped_vid' do not depend on lam).  Argument errors raise ValueError before
+        anything runs."""
+        tc = self.cond_frame_num
+        if not torch.is_tensor(real_vid) or real_vid.dim() != 5 or real_vid.shape[1] != 3 or real_vid.shape[2] < tc:
+            raise ValueError(f"interpolate_one_video: real_vid must be a (B, 3, >= {tc}, H, W) tensor")
+        self.diffusion.interp_args(x1, x2, tc, t, lam, seeds, noise, who="interpolate_one_video")
+        st = int(round(1 / self.region_predictor.scale_factor))
+        B, _, _, H, W = real_vid.shape
+        if tuple(x1.shape) != (B, 3, self.pred_frame_num, H // st, W // st):
+            raise ValueError(f"interpolate_one_video: x1 {tuple(x1.shape)} does not fit real_vid "
+                             f"{tuple(real_vid.shape)}: expected {(B, 3, self.pred_frame_num, H // st, W // st)}")
+        ret, x_cond, cond_fea, ref = self.condition(real_vid[:, :, :tc].contiguous())
+        pred = self.diffusion.interpolate(x1, x2, x_cond, cond_fea, t=t, lam=lam, seeds=seeds, noise=noise)
+        if not isinstance(lam, (list, tuple)):
+            ret.update(self._decode_sample(ret, ref, pred))
+            return ret
+        parts = [self._decode_sample(ret, ref, p) for p in pred]
+        for k in parts[0]:
+            ret[k] = parts[0][k] if k.startswith("real_") else torch.stack([d[k] for d in parts])
         return ret
 
     # ------------------------------------------------------------------ denoising loss (forward-only training objective)

@@ -660,6 +660,37 @@ def q_sample(rec, x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t, eps):
              keep=(x_start, t, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t, eps))
 
 
+def q_interpolate(rec, x1, x2, t, seeds, noise, sqrt_acp, sqrt_1m_acp, c1, c2, x_t):
+    """x_t = c1 * (sqrt_acp[t] * x1 + sqrt_1m_acp[t] * eps1) + c2 * (sqrt_acp[t] * x2 + sqrt_1m_acp[t] * eps2) with one
+    int t for the batch; (eps1, eps2) = noise (2, *x1.shape) when given, else the Philox draws of (seeds[b], t, streams
+    4 and 5)."""
+    for v, name in ((x1, "x1"), (x2, "x2"), (x_t, "x_t"), (sqrt_acp, "sqrt_acp"), (sqrt_1m_acp, "sqrt_1m_acp")):
+        if v is None:
+            raise ValueError(f"q_interpolate: {name} is required")
+        _chk(v, torch.float32, name)
+    _chk(seeds, torch.int64, "seeds")
+    _chk(noise, torch.float32, "noise")
+    B = x1.shape[0]
+    if (seeds is None) == (noise is None):
+        raise ValueError("q_interpolate: pass exactly one of seeds and noise")
+    if seeds is not None and (seeds.numel() != B or seeds.device != x1.device):
+        raise ValueError(f"q_interpolate: seeds must be {B} int64 on {x1.device}, got {seeds.numel()} on "
+                         f"{seeds.device}")
+    for v, name in ((x2, "x2"), (x_t, "x_t")):
+        if v.shape != x1.shape:
+            raise ValueError(f"q_interpolate: {name} {tuple(v.shape)} != x1 {tuple(x1.shape)}")
+    if noise is not None and tuple(noise.shape) != (2, *x1.shape):
+        raise ValueError(f"q_interpolate: noise must be {(2, *x1.shape)}, got {tuple(noise.shape)}")
+    if sqrt_acp.numel() != sqrt_1m_acp.numel() or not 0 <= int(t) < sqrt_acp.numel():
+        raise ValueError(f"q_interpolate: t = {t} outside the schedule tables ({sqrt_acp.numel()}, "
+                         f"{sqrt_1m_acp.numel()})")
+    if (x1.numel() // B) % 4:
+        raise ValueError("q_interpolate: elements per sample must be a multiple of 4")
+    rec.emit("extdm_q_interpolate", (_p(x1), _p(x2), int(t), _p(seeds), _p(noise), _p(sqrt_acp), _p(sqrt_1m_acp),
+                                     C.c_float(c1), C.c_float(c2), _p(x_t), B, x1.numel() // B),
+             keep=(x1, x2, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t))
+
+
 def denoise_loss(rec, eps, pred, out, l1=False):
     """out (B, tp) = mean over (3, h, w) of (eps - pred)^2, or |eps - pred| with l1, per (video, frame) of eps, pred
     (B, 3, tp, h, w)."""

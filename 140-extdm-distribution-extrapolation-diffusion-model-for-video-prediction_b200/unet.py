@@ -177,6 +177,7 @@ class UnetRunner:
         self.ddpm_graphs = {}               # CUDA graphs of one ancestral-sampler iteration (GaussianDiffusion)
         self.loss_graphs = {}               # CUDA graphs of the denoising-loss evaluation (GaussianDiffusion)
         self.solver_graphs = {}             # CUDA graphs of the DPM-Solver++(2M) sampling loop (GaussianDiffusion)
+        self.interp_graphs = {}             # CUDA graphs of the DDIM loop of GaussianDiffusion.interpolate
         self._build()
 
     # ------------------------------------------------------------------ helpers

@@ -303,6 +303,8 @@ int extdm_ddim_update_seeded(const float* img, const float* pred, const long lon
  * counter (element index / 4 within the video, t[b], 2, 0), so a video's epsilon depends on its seed and its timestep
  * only, and every timestep of a loss curve draws its own.  Stream 3 is the noise of the stochastic DPM-Solver++(2M)
  * (extdm_dpmpp_update): iteration i draws counter (element index / 4 within the video, i, 3, 0); its x_T is stream 1.
+ * Streams 4 and 5 are the epsilons of the two endpoints of an interpolation (extdm_q_interpolate): counter (element
+ * index / 4 within the video, t, 4 or 5, 0), t the mix timestep; its loop noise is stream 0 as above.
  */
 
 /* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
@@ -359,6 +361,22 @@ int extdm_q_sample(const float* x_start, const long long* t, const long long* se
  * data only. */
 int extdm_denoise_loss(const float* eps, const float* pred, float* out, int B, int tp, int per_frame, int l1,
                        void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Interpolation between two futures (GaussianDiffusion.interpolate, Diffusion.py:261-274 with the keyword fix of
+ * SURVEY App. E10), fp32.  Added under ABI version 5 (backward compatible).
+ */
+
+/* The mix of two forward diffusions at one timestep t shared by the batch, a = sqrt_acp[t], b = sqrt_1m_acp[t]:
+ *   x_t_out = c1 * (a * x1 + b * eps1) + c2 * (a * x2 + b * eps2)       (each product rounded, no FMA)
+ * bit-exact against the torch fp32 expression with c1 = fp32(1 - lam), c2 = fp32(lam).  eps1, eps2 are noise[0] and
+ * noise[1] of noise ((2, B, n)) when noise != NULL, else the Philox draws of (seeds[b], t, stream 4) and (seeds[b], t,
+ * stream 5) documented above.  Exactly one of seeds ((B,) int64) and noise is given.  x1, x2, x_t_out: (B, n) fp32;
+ * t in [0, length of the tables) -- the caller checks the upper bound; sqrt_acp, sqrt_1m_acp: the fp32
+ * sqrt_alphas_cumprod / sqrt_one_minus_alphas_cumprod buffers. */
+int extdm_q_interpolate(const float* x1, const float* x2, int t, const long long* seeds, const float* noise,
+                        const float* sqrt_acp, const float* sqrt_1m_acp, float c1, float c2, float* x_t_out, int B,
+                        int n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * LFAE decode (Generator.forward_with_flow / deform_input / apply_optical, model/LFAE/generator.py:63-93,
