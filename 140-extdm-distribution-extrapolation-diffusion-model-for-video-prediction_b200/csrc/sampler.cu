@@ -21,6 +21,12 @@ __device__ __forceinline__ float x_start_of(float img, float pred, float c_recip
   return __fsub_rn(__fmul_rn(c_recip, img), __fmul_rn(c_recipm1, pred));
 }
 
+// The thresholded x0 of every update: clamp(x_start, -s, s) / s, clamped then divided with one rounding, as the
+// reference evaluates `x_start.clamp(-s, s) / s`.
+__device__ __forceinline__ float clamped_x0(float img, float pred, float c_recip, float c_recipm1, float s) {
+  return __fdiv_rn(fminf(fmaxf(x_start_of(img, pred, c_recip, c_recipm1), -s), s), s);
+}
+
 // One CTA per sample: s_out[b] = max(1, quantile_q(|x_start[b]|)).  |x| >= 0 so the IEEE bit pattern orders like an
 // unsigned integer.  Shared by the DDIM kernel (coefficients as arguments) and the DDPM kernel (coefficients read from
 // the schedule table on the device), so both take the same select path.
@@ -105,8 +111,7 @@ __device__ __forceinline__ void ddim_quad(float4 x, float4 e, float4 z, bool wit
   float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, zv[4] = {z.x, z.y, z.z, z.w}, o[4], xs[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
-    float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
-    v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+    const float v = clamped_x0(xv[j], ev[j], c_recip, c_recipm1, sb);
     xs[j] = v;
     float r = __fadd_rn(__fmul_rn(v, sqrt_alpha_next), __fmul_rn(c, ev[j]));
     if (with_noise) r = __fadd_rn(r, __fmul_rn(sigma, zv[j]));
@@ -211,8 +216,7 @@ __global__ void __launch_bounds__(256) ddpm_update_kernel(const float* __restric
     float xv[4] = {x.x, x.y, x.z, x.w}, ev[4] = {e.x, e.y, e.z, e.w}, zv[4] = {z.x, z.y, z.z, z.w}, o[4], xs[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
-      v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+      const float v = clamped_x0(xv[j], ev[j], c_recip, c_recipm1, sb);
       xs[j] = v;
       const float mean = __fadd_rn(__fmul_rn(c1, v), __fmul_rn(c2, xv[j]));
       o[j] = __fadd_rn(mean, __fmul_rn(sig, zv[j]));       // added at t = 0 too (sig = 0): torch's signed zeros
@@ -290,8 +294,7 @@ __global__ void __launch_bounds__(256) dpmpp_update_kernel(const float* __restri
           zv[4] = {z.x, z.y, z.z, z.w}, o[4], dv[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      float v = x_start_of(xv[j], ev[j], c_recip, c_recipm1);
-      v = __fdiv_rn(fminf(fmaxf(v, -sb), sb), sb);
+      const float v = clamped_x0(xv[j], ev[j], c_recip, c_recipm1, sb);
       dv[j] = v;
       float r = __fadd_rn(__fmul_rn(A, xv[j]), __fmul_rn(B, v));
       if (d_prev) r = __fadd_rn(r, __fmul_rn(C, pv[j]));
@@ -429,6 +432,11 @@ __global__ void __launch_bounds__(256) ddpm_advance_kernel(int* __restrict__ ste
 
 using namespace extdm;
 
+static int ddpm_grid(long long total4) {
+  long long g = (total4 + 255) / 256;
+  return static_cast<int>(g > 148 * 8 ? 148 * 8 : g);
+}
+
 extern "C" int extdm_ddim_threshold(const float* img, const float* pred, float c_recip, float c_recipm1, float q,
                                     float* s, int B, int n, void* stream) {
   if (n < 2 || B < 1) {
@@ -448,17 +456,10 @@ extern "C" int extdm_ddim_update(const float* img, const float* pred, const floa
     return EXTDM_ERR_ARG;
   }
   const long long total4 = static_cast<long long>(B) * n / 4;
-  long long g = (total4 + 255) / 256;
-  if (g > 148 * 8) g = 148 * 8;
-  ddim_update_kernel<<<static_cast<int>(g), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+  ddim_update_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       img, pred, noise, s, c_recip, c_recipm1, sqrt_alpha_next, c, sigma, img_out, x_start_out, n / 4, total4);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
-}
-
-static int ddpm_grid(long long total4) {
-  long long g = (total4 + 255) / 256;
-  return static_cast<int>(g > 148 * 8 ? 148 * 8 : g);
 }
 
 extern "C" int extdm_ddim_update_seeded(const float* img, const float* pred, const long long* seeds, int step,

@@ -34,22 +34,27 @@ def _f32(v):
     return struct.unpack("f", struct.pack("f", v))[0]
 
 
+def _int64_vector(v, B, what, who):
+    """v, a (B,) int64 tensor (any device) or a list of ints, as a tensor: one `what` (e.g. "seed") per video."""
+    if not torch.is_tensor(v):
+        try:
+            v = torch.tensor(list(v))
+        except (TypeError, RuntimeError, OverflowError) as e:
+            raise ValueError(f"{who}: {what}s must be int64 values ({e})") from None
+    if v.dtype != torch.int64:
+        raise ValueError(f"{who}: {what}s must be int64, got {v.dtype}")
+    if tuple(v.shape) != (B,):
+        raise ValueError(f"{who}: need one {what} per video, shape ({B},), got {tuple(v.shape)}")
+    return v
+
+
 def _seed_vector(seeds, noise, B, who):
     """Validate the per-video seeds of a sampler call: None, or a (B,) int64 tensor (any device) or a list of ints."""
     if seeds is None:
         return None
     if noise is not None:
         raise ValueError(f"{who}: pass noise or seeds, not both")
-    if not torch.is_tensor(seeds):
-        try:
-            seeds = torch.tensor(list(seeds))
-        except (TypeError, RuntimeError, OverflowError) as e:
-            raise ValueError(f"{who}: seeds must be int64 values ({e})") from None
-    if seeds.dtype != torch.int64:
-        raise ValueError(f"{who}: seeds must be int64, got {seeds.dtype}")
-    if tuple(seeds.shape) != (B,):
-        raise ValueError(f"{who}: need one seed per video, shape ({B},), got {tuple(seeds.shape)}")
-    return seeds
+    return _int64_vector(seeds, B, "seed", who)
 
 
 def _timestep_vector(timesteps, B, num_timesteps, who):
@@ -58,19 +63,36 @@ def _timestep_vector(timesteps, B, num_timesteps, who):
     the forward-diffusion kernel indexes the schedule tables with these values."""
     if timesteps is None:
         return None
-    if not torch.is_tensor(timesteps):
-        try:
-            timesteps = torch.tensor(list(timesteps))
-        except (TypeError, RuntimeError, OverflowError) as e:
-            raise ValueError(f"{who}: timesteps must be int64 values ({e})") from None
-    if timesteps.dtype != torch.int64:
-        raise ValueError(f"{who}: timesteps must be int64, got {timesteps.dtype}")
-    if tuple(timesteps.shape) != (B,):
-        raise ValueError(f"{who}: need one timestep per video, shape ({B},), got {tuple(timesteps.shape)}")
+    timesteps = _int64_vector(timesteps, B, "timestep", who)
     host = timesteps.cpu()
     if B and (int(host.min()) < 0 or int(host.max()) >= num_timesteps):
         raise ValueError(f"{who}: timesteps must lie in [0, {num_timesteps}), got {host.tolist()}")
     return timesteps
+
+
+def _check_noise(noise, shape, who, dtype=None):
+    """ValueError unless noise is None or a tensor of `shape`; dtype "float" also requires a floating-point tensor,
+    "float32" an fp32 one."""
+    if noise is None:
+        return
+    if (not torch.is_tensor(noise) or tuple(noise.shape) != tuple(shape)
+            or (dtype == "float" and not noise.is_floating_point())
+            or (dtype == "float32" and noise.dtype != torch.float32)):
+        got = f"{noise.dtype} {tuple(noise.shape)}" if torch.is_tensor(noise) else type(noise).__name__
+        raise ValueError(f"{who}: noise must be a {dtype + ' ' if dtype else ''}tensor of shape {tuple(shape)}, "
+                         f"got {got}")
+
+
+def _default_seeds(seeds, noise, B):
+    """seeds, or B seeds drawn from torch's default generator when neither seeds nor noise is given."""
+    if noise is None and seeds is None:
+        return torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+    return seeds
+
+
+def _require_cuda(x, who):
+    if x.device.type != "cuda":
+        raise RuntimeError(f"{who} runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
 
 
 def _load_seeds(dst, seeds):
@@ -130,13 +152,39 @@ class GaussianDiffusion(nn.Module):
             raise ValueError(f"solver must be None or one of {SOLVERS}, got {value!r}")
         self._solver = value
 
+    def _check_thresholding(self, clip_denoised=True):
+        if not clip_denoised or not self.use_dynamic_thres:
+            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
+
+    def _graph(self, r, key, make_state, prepare, body, trace=None):
+        """(state, run) of the launch sequence body(state) on the runner r.
+
+        With use_cuda_graph and no trace, the first call for `key` makes the state, prepare(state)s it (stages a call's
+        inputs), runs body once eagerly and captures it (ops.capture_graph); run replays that graph, on the same state,
+        for every later call with this key.  Otherwise run calls body on a fresh state.  Captured graphs hold raw
+        pointers into the runner's weight and activation buffers, so they live ON the runner, in r.graphs:
+        Unet3D.invalidate() (load_state_dict, device move) drops runner and graphs together.  The key starts with the
+        kind of loop ("ddim", "ddpm", "solver", "loss", "interp") and holds everything the capture bakes in."""
+        if trace is not None or not self.use_cuda_graph:
+            st = make_state()
+            return st, lambda: body(st)
+        if key not in r.graphs:
+            st = make_state()
+            prepare(st)
+            r.graphs[key] = (ops.capture_graph(lambda: body(st)), st)
+        g, st = r.graphs[key]
+        return st, g.replay
+
     # ------------------------------------------------------------------ schedule scalars (host, fp32)
+    def _ddim_times(self, S):
+        """t_0 > ... > t_S = 0, the DDIM grid of S steps: torch.linspace(0, num_timesteps, S + 2)[:-1].int() reversed
+        (host only)."""
+        return list(reversed(torch.linspace(0.0, self.num_timesteps, steps=S + 2)[:-1].int().tolist()))
+
     def ddim_schedule(self):
         """[(time, time_next, c_recip, c_recipm1, sqrt_alpha_next, c, sigma)], evaluated with the same fp32 torch
         scalar ops as Diffusion.py:214-216, 221-222, 248-249 (note the alphas_cumprod_*prev* indexing)."""
-        total, n = self.num_timesteps, self.sampling_timesteps
-        times = torch.linspace(0.0, total, steps=n + 2)[:-1]
-        return self._ddim_rows(list(reversed(times.int().tolist())))
+        return self._ddim_rows(self._ddim_times(self.sampling_timesteps))
 
     def _ddim_rows(self, times):
         """ddim_schedule's rows for the consecutive pairs (time, time_next) of `times`."""
@@ -175,88 +223,55 @@ class GaussianDiffusion(nn.Module):
         device, in the reference's draw order.  seeds: optional (B,) int64 tensor or list, one per video, instead of
         noise: x_T and the noise of iteration i are the Philox draws of the video's seed (stream 1, and step i of
         stream 0: include/extdm_b200.h), made inside the kernels, so video b's sample depends on seeds[b] only and
-        no noise tensor is stored.  trace: list that receives per-step tensors (tests)."""
+        no noise tensor is stored.  trace: list that receives per-step tensors (tests).
+
+        The whole loop is one CUDA graph per shape, schedule and seeded-or-not (_graph, key "ddim"); the noise or the
+        seeds are copied into its state before each replay, the seeds without a host synchronisation."""
         B = shape[0]
         seeds = _seed_vector(seeds, noise, B, "ddim_sample")
-        if not clip_denoised or not self.use_dynamic_thres:
-            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
-        unet = self.denoise_fn
+        self._check_thresholding(clip_denoised)
         dev = x_cond.device
         sched = self.ddim_schedule()
-        r = unet.runner(B, shape[3], shape[4], cond_fea.shape[-1])
-        if seeds is not None:
-            return self._ddim_seeded(r, sched, shape, x_cond, cond_fea, seeds, trace)
-        if noise is None:
+        r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
+        if noise is None and seeds is None:
             noise = torch.empty(len(sched), *shape, device=dev)
             noise[0] = torch.randn(shape, device=dev)
             for i in range(1, len(sched)):
                 noise[i] = torch.randn(shape, device=dev)
-        if trace is not None or not self.use_cuda_graph:
-            return self._run_loop(r, sched, x_cond, cond_fea, noise, trace).clone()
-        # Captured graphs hold raw pointers into the runner's weight and activation buffers, so they live ON the runner:
-        # Unet3D.invalidate() (load_state_dict, device move) drops runner and graphs together.  The schedule scalars are
-        # baked into the capture, hence part of the key.
-        graphs = r.ddim_graphs
-        key = self._ddim_key(shape)
-        if key not in graphs:
-            st = dict(noise=torch.zeros_like(noise), s=torch.zeros(B, device=dev))
-            st["x_cond"], st["cond_fea"] = r.cond_frames, r.cond_fea
-            self._run_loop(r, sched, x_cond, cond_fea, noise, None, st)          # warm-up (lazy inits)
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._run_loop(r, sched, None, None, st["noise"], None, st)
-            graphs[key] = (g, st)
-        g, st = graphs[key]
-        r.set_conditioning(x_cond.float(), cond_fea.float())
-        st["noise"].copy_(noise)
-        g.replay()
+
+        def state():
+            return dict(s=torch.zeros(B, device=r.dev),
+                        seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if seeds is not None else None,
+                        noise=torch.zeros_like(noise) if noise is not None else None)
+
+        def stage(st):
+            r.set_conditioning(x_cond.float(), cond_fea.float())
+            if seeds is None:
+                st["noise"].copy_(noise)
+            else:
+                _load_seeds(st["seeds"], seeds)                                   # no host sync before the replay
+
+        # the schedule scalars are baked into the capture, hence part of the key
+        key = self._ddim_key("ddim", shape) + ((("seeded", True),) if seeds is not None else ())
+        st, run = self._graph(r, key, state, stage, lambda st: self._ddim_loop(r, sched, st, trace), trace)
+        stage(st)
+        run()
         return r.x.clone()
 
-    def _ddim_key(self, shape):
-        return (tuple(shape), float(self.ddim_sampling_eta), float(self.dynamic_thres_percentile),
+    def _ddim_key(self, kind, shape):
+        return (kind, tuple(shape), float(self.ddim_sampling_eta), float(self.dynamic_thres_percentile),
                 int(self.sampling_timesteps), int(self.num_timesteps))
 
-    def _ddim_seeded(self, r, sched, shape, x_cond, cond_fea, seeds, trace):
-        """ddim_sample with per-video seeds.  The graph reads the seeds from a device buffer of its state (there is
-        no noise buffer), so one capture serves every seed vector; each call only copies the seeds in."""
-        def state():
-            return dict(seeds=torch.zeros(r.B, dtype=torch.long, device=r.dev), s=torch.zeros(r.B, device=r.dev))
-        if trace is not None or not self.use_cuda_graph:
-            st = state()
-            _load_seeds(st["seeds"], seeds)
-            return self._run_loop(r, sched, x_cond, cond_fea, None, trace, st).clone()
-        graphs = r.ddim_graphs
-        key = self._ddim_key(shape) + (("seeded", True),)
-        if key not in graphs:
-            st = state()
-            _load_seeds(st["seeds"], seeds)
-            st["x_cond"], st["cond_fea"] = r.cond_frames, r.cond_fea
-            self._run_loop(r, sched, x_cond, cond_fea, None, None, st)            # warm-up (lazy inits)
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._run_loop(r, sched, None, None, None, None, st)
-            graphs[key] = (g, st)
-        g, st = graphs[key]
-        r.set_conditioning(x_cond.float(), cond_fea.float())
-        _load_seeds(st["seeds"], seeds)                                           # no host sync before the replay
-        g.replay()
-        return r.x.clone()
-
-    def _run_loop(self, r, sched, x_cond, cond_fea, noise, trace, st=None):
-        """The DDIM loop.  Its noise is noise[0] (x_T) and noise[i + 1] (iteration i), or, when st holds "seeds", the
-        Philox draws of those seeds."""
-        if x_cond is not None:
-            r.set_conditioning(x_cond.float(), cond_fea.float())
-        s = st["s"] if st is not None else torch.zeros(r.B, device=r.dev)
-        seeds = st.get("seeds") if st is not None else None
+    def _ddim_loop(self, r, sched, st, trace=None):
+        """UNet prologue, x_T, then the DDIM iterations.  The noise is st["noise"][0] (x_T) and st["noise"][i + 1]
+        (iteration i), or, when st holds "seeds", the Philox draws of those seeds."""
         r.run_prologue()
-        if seeds is not None:
-            ops.ddpm_fill_normal(ops.IMMEDIATE, seeds, r.x)
+        if st["seeds"] is not None:
+            ops.ddpm_fill_normal(ops.IMMEDIATE, st["seeds"], r.x)
         else:
-            r.x.copy_(noise[0])
-        return self._ddim_steps(r, sched, None if noise is None else noise[1:], seeds, s, trace)
+            r.x.copy_(st["noise"][0])
+        return self._ddim_steps(r, sched, None if st["noise"] is None else st["noise"][1:], st["seeds"], st["s"],
+                                trace)
 
     def _ddim_steps(self, r, sched, noise, seeds, s, trace=None):
         """The DDIM iterations of sched from r.x (after the UNet prologue): the noise of iteration i is noise[i], or,
@@ -311,48 +326,31 @@ class GaussianDiffusion(nn.Module):
         iteration i.  Default: Philox4x32-10 noise drawn inside the kernels, keyed by one seed per video that is taken
         from torch's default generator on every call (so torch.manual_seed reproduces a run, and a video's noise
         does not depend on its batch neighbours).  seeds: optional (B,) int64 tensor or list that replaces those
-        drawn seeds.  trace: list that receives per-step tensors (tests)."""
+        drawn seeds.  trace: list that receives per-step tensors (tests).
+
+        One iteration (time-MLP rows, UNet step, threshold, update, advance) is captured (_graph, _ddpm_key); its
+        per-step values come from the device tables and step counter, so the same graph serves every timestep."""
         seeds = _seed_vector(seeds, noise, shape[0], "p_sample_loop")
-        if not self.use_dynamic_thres:
-            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
-        if x_cond.device.type != "cuda":
-            raise RuntimeError("p_sample_loop runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
-        T, B, dev = self.num_timesteps, shape[0], x_cond.device
-        if noise is not None and tuple(noise.shape) != (T + 1, *shape):
-            raise ValueError(f"p_sample_loop: noise must have shape {(T + 1, *shape)}, got {tuple(noise.shape)}")
+        self._check_thresholding()
+        _require_cuda(x_cond, "p_sample_loop")
+        T, B = self.num_timesteps, shape[0]
+        _check_noise(noise, (T + 1, *shape), "p_sample_loop")
         r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
-        if noise is None and seeds is None:
-            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
-        if trace is not None or not self.use_cuda_graph:
-            st = self._ddpm_state(r, noise is not None)
+        seeds = _default_seeds(seeds, noise, B)
+        injected = noise is not None
+
+        def start(st):
             self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
-            for _ in range(T):
-                self._ddpm_iteration(r, st, trace)
-            return r.x.clone()
-        g, st = self._ddpm_graph(r, shape, noise is not None,
-                                 lambda st: self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise))
-        self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise)
+        st, run = self._graph(r, self._ddpm_key(shape, injected), lambda: self._ddpm_state(r, injected), start,
+                              lambda st: self._ddpm_iteration(r, st, trace), trace)
+        start(st)
         for _ in range(T):
-            g.replay()
+            run()
         return r.x.clone()
 
-    def _ddpm_graph(self, r, shape, injected, start):
-        """(graph, state) of one captured ancestral iteration.  start(st) sets up a round for the warm-up run."""
-        # One iteration (time-MLP rows, UNet step, threshold, update, advance) is captured; its per-step values come from
-        # the device tables and step counter, so the same graph serves every timestep.  Like ddim_graphs it lives on the
-        # runner, whose buffers it points into.
-        graphs = r.ddpm_graphs
-        key = (tuple(shape), float(self.dynamic_thres_percentile), self.num_timesteps, injected)
-        if key not in graphs:
-            st = self._ddpm_state(r, injected)
-            start(st)                                                          # warm-up (lazy inits)
-            self._ddpm_iteration(r, st)
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._ddpm_iteration(r, st)
-            graphs[key] = (g, st)
-        return graphs[key]
+    def _ddpm_key(self, shape, injected):
+        """The key of the captured ancestral iteration, shared by p_sample_loop and interpolate."""
+        return ("ddpm", tuple(shape), float(self.dynamic_thres_percentile), self.num_timesteps, injected)
 
     def _ddpm_state(self, r, injected):
         """Device state of the loop: schedule table, time-MLP rows per step, step counter, per-video seeds,
@@ -401,7 +399,7 @@ class GaussianDiffusion(nn.Module):
         if self.solver is None:
             raise ValueError("solver_schedule: no solver is selected")
         T, S = self.num_timesteps, int(self.sampling_timesteps)
-        times = list(reversed(torch.linspace(0.0, T, steps=S + 2)[:-1].int().tolist())) if S >= 1 else []
+        times = self._ddim_times(S) if S >= 1 else []
         if S < 1 or any(a <= b for a, b in zip(times, times[1:])):
             raise ValueError(f"{self.solver}: the grid of {S} steps over {T} timesteps is not strictly decreasing "
                              f"(need 1 <= sampling_timesteps < timesteps, and well below it): {times}")
@@ -460,27 +458,23 @@ class GaussianDiffusion(nn.Module):
         trace: list that receives per-step tensors (tests).
 
         The whole loop (UNet prologue, x_T, S x (UNet step, threshold, update)) is one CUDA graph per shape, solver, S,
-        T, percentile and injected-or-not, kept on the UNet runner (solver_graphs); the seeds (or the noise) are
-        copied in before each replay without a host synchronisation, so one capture serves every seed vector."""
+        T, percentile and injected-or-not (_graph, key "solver"); the seeds (or the noise) are copied in before each
+        replay without a host synchronisation, so one capture serves every seed vector."""
         B = shape[0]
         seeds = _seed_vector(seeds, noise, B, "dpm_solver_sample")
         S = len(self._solver_times()) - 1
-        if noise is not None and (not torch.is_tensor(noise) or not noise.is_floating_point()
-                                  or tuple(noise.shape) != (S, *shape)):
-            raise ValueError(f"dpm_solver_sample: noise must be a float tensor of shape {(S, *shape)}, got "
-                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
-        if not self.use_dynamic_thres:
-            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
-        if x_cond.device.type != "cuda":
-            raise RuntimeError("dpm_solver_sample runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
-        if noise is None and seeds is None:
-            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        _check_noise(noise, (S, *shape), "dpm_solver_sample", "float")
+        self._check_thresholding()
+        _require_cuda(x_cond, "dpm_solver_sample")
+        seeds = _default_seeds(seeds, noise, B)
         r = self.denoise_fn.runner(B, shape[3], shape[4], cond_fea.shape[-1])
 
         def state():
+            # the coefficients read the buffers on the host: only when capturing (or running eagerly)
             return dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if noise is None else None,
                         noise=torch.zeros(S, *shape, device=r.dev) if noise is not None else None,
-                        s=torch.zeros(B, device=r.dev), d=torch.zeros(shape, device=r.dev))
+                        s=torch.zeros(B, device=r.dev), d=torch.zeros(shape, device=r.dev),
+                        sched=self.solver_schedule())
 
         def stage(st):
             r.set_conditioning(x_cond.float(), cond_fea.float())
@@ -489,31 +483,16 @@ class GaussianDiffusion(nn.Module):
             else:
                 st["noise"].copy_(noise)
 
-        if trace is not None or not self.use_cuda_graph:
-            st = state()
-            stage(st)
-            return self._solver_loop(r, self.solver_schedule(), st, trace).clone()
-        # like ddim_graphs the graph points into the runner's buffers (and bakes in the coefficients), so it lives on
-        # the runner and its key holds what selects the coefficients
-        key = (tuple(shape), self.solver, S, self.num_timesteps, float(self.dynamic_thres_percentile),
+        key = ("solver", tuple(shape), self.solver, S, self.num_timesteps, float(self.dynamic_thres_percentile),
                noise is not None)
-        if key not in r.solver_graphs:
-            sched = self.solver_schedule()               # reads the buffers on the host: only when capturing
-            st = state()
-            stage(st)
-            self._solver_loop(r, sched, st)                                 # warm-up (lazy inits)
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._solver_loop(r, sched, st)
-            r.solver_graphs[key] = (g, st)
-        g, st = r.solver_graphs[key]
+        st, run = self._graph(r, key, state, stage, lambda st: self._solver_loop(r, st, trace), trace)
         stage(st)
-        g.replay()
+        run()
         return r.x.clone()
 
-    def _solver_loop(self, r, sched, st, trace=None):
-        """UNet prologue, x_T, then per step: UNet step, threshold, dpmpp_update (D kept in st["d"] for the next)."""
+    def _solver_loop(self, r, st, trace=None):
+        """UNet prologue, x_T, then per step of st["sched"]: UNet step, threshold, dpmpp_update (D kept in st["d"] for
+        the next)."""
         rec = ops.IMMEDIATE
         r.run_prologue()
         if st["noise"] is None:
@@ -522,6 +501,7 @@ class GaussianDiffusion(nn.Module):
             r.x.copy_(st["noise"][0])
         q = float(self.dynamic_thres_percentile)
         sde = self.solver == "dpmpp_2m_sde"
+        sched = st["sched"]
         ss = r.ss_for_times([row[0] for row in sched])       # evaluated once per schedule, outside the captured loop
         for i, (t, c_recip, c_recipm1, A, Bc, Cc, N, final) in enumerate(sched):
             r.run_step(ss[i])
@@ -545,9 +525,7 @@ class GaussianDiffusion(nn.Module):
         if self.loss_type not in ("l1", "l2"):
             raise ValueError(f"{who}: loss_type {self.loss_type!r} is not 'l1' or 'l2'")
         seeds = _seed_vector(seeds, noise, B, who)
-        if noise is not None and (not torch.is_tensor(noise) or tuple(noise.shape) != tuple(shape)):
-            raise ValueError(f"{who}: noise must have shape {tuple(shape)}, got "
-                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
+        _check_noise(noise, shape, who)
         return _timestep_vector(timesteps, B, self.num_timesteps, who), seeds
 
     @torch.no_grad()
@@ -580,12 +558,10 @@ class GaussianDiffusion(nn.Module):
                              f"{tuple(cond_fea.shape)}: expected (B, 3, tp, h, w), (B, 3, tc, h, w) and (B, ...) with "
                              f"tc + tp = {self.num_frames}")
         t, seeds = self.loss_args(B, x_start.shape, timesteps, seeds, noise)
-        if x_start.device.type != "cuda":
-            raise RuntimeError("denoising_loss runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
+        _require_cuda(x_start, "denoising_loss")
         if t is None:
             t = torch.randint(0, self.num_timesteps, (B,))
-        if noise is None and seeds is None:
-            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        seeds = _default_seeds(seeds, noise, B)
         r = self.denoise_fn.runner(B, h, w, cond_fea.shape[-1])
         l1 = self.loss_type == "l1"
 
@@ -607,25 +583,10 @@ class GaussianDiffusion(nn.Module):
                 _load_seeds(st["seeds"], seeds)
             _load_seeds(r.time, t)                                     # no host sync before the launches / replay
 
-        if not self.use_cuda_graph:
-            st = state()
-            stage(st)
-            self._loss_launch(r, st, l1)
-        else:
-            # like ddim_graphs the graph points into the runner's buffers, so it lives on the runner
-            key = (tuple(x_start.shape), self.loss_type, noise is not None, self.num_timesteps)
-            if key not in r.loss_graphs:
-                st = state()
-                stage(st)
-                self._loss_launch(r, st, l1)                           # warm-up (lazy inits)
-                torch.cuda.synchronize()
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    self._loss_launch(r, st, l1)
-                r.loss_graphs[key] = (g, st)
-            g, st = r.loss_graphs[key]
-            stage(st)
-            g.replay()
+        key = ("loss", tuple(x_start.shape), self.loss_type, noise is not None, self.num_timesteps)
+        st, run = self._graph(r, key, state, stage, lambda st: self._loss_launch(r, st, l1))
+        stage(st)
+        run()
         lpf = st["lpf"].clone()           # a copy: the next call of the same shape rewrites the state
         return {"loss": lpf.mean(dim=1), "loss_per_frame": lpf, "timesteps": r.time.clone()}
 
@@ -675,10 +636,7 @@ class GaussianDiffusion(nn.Module):
         seeds = _seed_vector(seeds, noise, B, who)
         times = self.interp_times(t) if self.is_ddim_sampling else None
         n_loop = t if times is None else len(times) - 2
-        if noise is not None and (not torch.is_tensor(noise) or noise.dtype != torch.float32
-                                  or tuple(noise.shape) != (2 + n_loop, *x1.shape)):
-            raise ValueError(f"{who}: noise must be a float32 tensor of shape {(2 + n_loop, *x1.shape)}, got "
-                             f"{tuple(noise.shape) if torch.is_tensor(noise) else type(noise).__name__}")
+        _check_noise(noise, (2 + n_loop, *x1.shape), who, "float32")
         return t, [float(v) for v in lams], sweep, seeds, times
 
     @torch.no_grad()
@@ -704,9 +662,9 @@ class GaussianDiffusion(nn.Module):
         (2 + n_loop, B, 3, tp, h, w) instead of seeds: eps1, eps2, then the noise of the loop's steps (n_loop = t
         ancestral, S - 1 DDIM: the last DDIM step adds none).
 
-        The mix is one kernel launch per value; the loop replays a CUDA graph kept on the UNet runner (the ancestral
-        iteration of ddpm_graphs, or the whole DDIM loop in interp_graphs, one per shape, t, S, eta, percentile and
-        injected-or-not).  Argument errors raise ValueError before anything runs; CPU tensors then RuntimeError."""
+        The mix is one kernel launch per value; the loop replays a CUDA graph kept on the UNet runner (_graph: the
+        ancestral iteration of p_sample_loop, key "ddpm", or the whole DDIM loop, key "interp", one per shape, t, S,
+        eta, percentile and injected-or-not).  Argument errors raise ValueError before anything runs; CPU tensors then RuntimeError."""
         if not all(torch.is_tensor(v) and v.dim() == 5 for v in (x_cond, cond_fea)):
             raise ValueError("interpolate: x_cond and cond_fea must be 5-D tensors")
         tc = x_cond.shape[2]
@@ -715,12 +673,9 @@ class GaussianDiffusion(nn.Module):
         if tuple(x_cond.shape) != (B, 3, tc, h, w) or cond_fea.shape[0] != B:
             raise ValueError(f"interpolate: x_cond {tuple(x_cond.shape)}, cond_fea {tuple(cond_fea.shape)}: expected "
                              f"({B}, 3, {tc}, {h}, {w}) and ({B}, ...)")
-        if not self.use_dynamic_thres:
-            raise NotImplementedError("only clip_denoised=True with dynamic thresholding (the shipped setting)")
-        if x1.device.type != "cuda":
-            raise RuntimeError("interpolate runs on CUDA only (hand-written sm_100a kernels, no CPU fallback)")
-        if noise is None and seeds is None:
-            seeds = torch.randint(0, 2 ** 62, (B,), dtype=torch.long)
+        self._check_thresholding()
+        _require_cuda(x1, "interpolate")
+        seeds = _default_seeds(seeds, noise, B)
         r = self.denoise_fn.runner(B, h, w, cond_fea.shape[-1])
         x1, x2 = x1.to(r.dev).contiguous(), x2.to(r.dev).contiguous()
         eps = noise[:2].to(r.dev).contiguous() if noise is not None else None
@@ -742,49 +697,34 @@ class GaussianDiffusion(nn.Module):
             if times is None and t > 0:
                 self._ddpm_start(r, st, T - t)
 
-        if times is None:                                               # ancestral: replays of one iteration
-            def loop():
-                for _ in range(t):
-                    run()
+        def prepare(st):
+            begin(st)
+            mix(st, lams[0])
+
+        injected = noise is not None
+        if times is None:                                               # ancestral: t replays of one iteration
+            n_runs = t
             if t == 0:
                 st, run = dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev), noise=None), None
-            elif self.use_cuda_graph:
-                g, st = self._ddpm_graph(r, x1.shape, noise is not None, lambda st: (begin(st), mix(st, lams[0])))
-                run = g.replay
             else:
-                st = self._ddpm_state(r, noise is not None)
-                run = lambda: self._ddpm_iteration(r, st)                 # noqa: E731
-        else:                                                           # DDIM: the whole loop
+                st, run = self._graph(r, self._ddpm_key(x1.shape, injected), lambda: self._ddpm_state(r, injected),
+                                      prepare, lambda st: self._ddpm_iteration(r, st))
+        else:                                                           # DDIM: the whole loop, one run
+            n_runs = 1
             sched = self._ddim_rows(times)
 
             def state():
-                return dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if noise is None else None,
-                            noise=torch.zeros(len(sched) - 1, *x1.shape, device=r.dev) if noise is not None else None,
+                return dict(seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if not injected else None,
+                            noise=torch.zeros(len(sched) - 1, *x1.shape, device=r.dev) if injected else None,
                             s=torch.zeros(B, device=r.dev))
-
-            def steps():
-                self._ddim_steps(r, sched, st["noise"], st["seeds"], st["s"])
-            if not self.use_cuda_graph:
-                st, loop = state(), steps
-            else:
-                # like ddim_graphs the graph points into the runner's buffers and bakes in the schedule scalars
-                key = self._ddim_key(x1.shape) + (t, noise is not None)
-                if key not in r.interp_graphs:
-                    st = state()
-                    begin(st)
-                    mix(st, lams[0])
-                    steps()                                             # warm-up (lazy inits)
-                    torch.cuda.synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        steps()
-                    r.interp_graphs[key] = (g, st)
-                g, st = r.interp_graphs[key]
-                loop = g.replay
+            # the graph bakes in the schedule scalars of t's grid
+            st, run = self._graph(r, self._ddim_key("interp", x1.shape) + (t, injected), state, prepare,
+                                  lambda st: self._ddim_steps(r, sched, st["noise"], st["seeds"], st["s"]))
         begin(st)
         outs = []
         for v in lams:
             mix(st, v)
-            loop()
+            for _ in range(n_runs):
+                run()
             outs.append(r.x.clone())
         return torch.stack(outs) if sweep else outs[0]

@@ -724,20 +724,9 @@ class CondRunner:
             self.launch()
             return self.grid, self.conf
         if self._graph is None:                                # static buffers: the launch lists replay as one graph
-            self._graph = _capture(self.launch)
+            self._graph = ops.capture_graph(self.launch)
         self._graph.replay()
         return self.grid, self.conf
-
-
-def _capture(launch):
-    """One CUDA graph of `launch` (a function that issues kernels on the current stream), after one eager warm-up run
-    (lazy per-kernel attribute set-up)."""
-    launch()
-    torch.cuda.synchronize()
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        launch()
-    return g
 
 
 class ReconRunner:
@@ -776,7 +765,7 @@ class ReconRunner:
             self.launch()
         else:
             if self._graph is None:
-                self._graph = _capture(self.launch)
+                self._graph = ops.capture_graph(self.launch)
             self._graph.replay()
         per_video = lambda t: t.view(B, T, *t.shape[1:]).transpose(1, 2)
         out = {"prediction": per_video(self.dec.prediction), "deformed": per_video(self.dec.deformed),

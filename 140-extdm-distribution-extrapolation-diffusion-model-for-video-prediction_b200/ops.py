@@ -63,6 +63,17 @@ class Recorder:
 IMMEDIATE = Recorder(record=False)
 
 
+def capture_graph(launch):
+    """One CUDA graph of `launch` (a function that issues kernels on the current stream), after one eager warm-up run
+    (lazy per-kernel attribute set-up)."""
+    launch()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        launch()
+    return g
+
+
 def _p(t):
     return C.c_void_p(0 if t is None else t.data_ptr())
 

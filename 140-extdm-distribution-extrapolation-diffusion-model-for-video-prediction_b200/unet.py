@@ -173,11 +173,7 @@ class UnetRunner:
         self._ss_tables = {}
         self._ss_rows = {}
         self.taps = {}                      # name -> buffer, for layer-by-layer parity tests
-        self.ddim_graphs = {}               # CUDA graphs of the sampling loop over these buffers (GaussianDiffusion)
-        self.ddpm_graphs = {}               # CUDA graphs of one ancestral-sampler iteration (GaussianDiffusion)
-        self.loss_graphs = {}               # CUDA graphs of the denoising-loss evaluation (GaussianDiffusion)
-        self.solver_graphs = {}             # CUDA graphs of the DPM-Solver++(2M) sampling loop (GaussianDiffusion)
-        self.interp_graphs = {}             # CUDA graphs of the DDIM loop of GaussianDiffusion.interpolate
+        self.graphs = {}                    # key -> (CUDA graph, state) over these buffers (GaussianDiffusion._graph)
         self._build()
 
     # ------------------------------------------------------------------ helpers

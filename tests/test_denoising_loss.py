@@ -36,6 +36,11 @@ def bits(t):
     return t.contiguous().view(torch.int32)
 
 
+def n_graphs(r, kind):
+    """The number of CUDA graphs of one kind (the first field of the key) on the UNet runner r."""
+    return sum(k[0] == kind for k in r.graphs)
+
+
 def _rnd(shape, seed, scale=1.0):
     return torch.randn(shape, generator=torch.Generator().manual_seed(seed)) * scale
 
@@ -304,7 +309,7 @@ def _mini():
 
 
 @pytest.mark.gpu
-def test_denoising_loss_mini_unet():
+def test_denoising_loss_mini_unet_graph_cache():
     from oracle import extdm_oracle as O
     torch.set_num_threads(8)
     u, sd, fx, diff, x_start, x_cond, fea = _mini()
@@ -338,7 +343,7 @@ def test_denoising_loss_mini_unet():
     diff.use_cuda_graph = True
     g1 = diff.denoising_loss(x_start, x_cond, fea, timesteps=t, seeds=seeds)
     assert torch.equal(bits(g1["loss_per_frame"]), bits(eager["loss_per_frame"]))
-    assert len(r.loss_graphs) == 1
+    assert n_graphs(r, "loss") == 1
     for t2, s2 in ((torch.tensor([999, 0]), torch.tensor([-3, 2 ** 62 + 1])), ([1, 1], [9, 9])):
         g2 = diff.denoising_loss(x_start, x_cond, fea, timesteps=t2, seeds=s2)
         diff.use_cuda_graph = False
@@ -346,12 +351,12 @@ def test_denoising_loss_mini_unet():
         diff.use_cuda_graph = True
         assert torch.equal(bits(g2["loss_per_frame"]), bits(e2["loss_per_frame"]))
         assert not torch.equal(g2["loss"], g1["loss"])
-    assert len(r.loss_graphs) == 1
+    assert n_graphs(r, "loss") == 1
     dev_t = diff.denoising_loss(x_start, x_cond, fea, timesteps=t.cuda(), seeds=seeds.cuda())
     assert torch.equal(bits(dev_t["loss_per_frame"]), bits(eager["loss_per_frame"]))
     # injected noise: its own graph, equal to the seeded evaluation fed the same eps
     inj = diff.denoising_loss(x_start, x_cond, fea, timesteps=t, noise=eps)
-    assert torch.equal(bits(inj["loss_per_frame"]), bits(eager["loss_per_frame"])) and len(r.loss_graphs) == 2
+    assert torch.equal(bits(inj["loss_per_frame"]), bits(eager["loss_per_frame"])) and n_graphs(r, "loss") == 2
     # drawn t and seeds: torch.randint from the default generator, t first
     torch.manual_seed(3)
     drawn = diff.denoising_loss(x_start, x_cond, fea)

@@ -396,7 +396,7 @@ def test_solver_mini_unet_matches_oracle(solver):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("solver", SOLVERS)
-def test_solver_seeds(solver):
+def test_solver_seeds_graph_cache(solver):
     """Seeds against the injected noise they stand for, batch independence (video b alone vs in a batch of 4), one
     graph for two seed vectors, default seeds from torch's generator."""
     u, _, fx = _mini()
@@ -419,9 +419,9 @@ def test_solver_seeds(solver):
     graphed = diff.dpm_solver_sample(x, shape, fea, seeds=seeds)
     assert torch.equal(graphed, ref)
     r = u.runner(4, 32, 32, fea.shape[-1])
-    n_graphs = len(r.solver_graphs)
+    n_graphs = sum(k[0] == "solver" for k in r.graphs)
     again = diff.dpm_solver_sample(x, shape, fea, seeds=(seeds + 1).cuda())
-    assert len(r.solver_graphs) == n_graphs and not torch.equal(again, graphed)
+    assert sum(k[0] == "solver" for k in r.graphs) == n_graphs and not torch.equal(again, graphed)
     diff.use_cuda_graph = False
     assert torch.equal(diff.dpm_solver_sample(x, shape, fea, seeds=seeds + 1), again)
     k = 2
@@ -519,7 +519,7 @@ def test_solver_full_size_bair():
 
 
 @pytest.mark.gpu
-def test_default_sampler_untouched():
+def test_default_sampler_untouched_no_solver_graph():
     """solver=None: DDIM output bit-identical to a model constructed without the argument."""
     u, _, fx = _mini()
     x, fea, shape = _inputs(fx)
@@ -533,4 +533,4 @@ def test_default_sampler_untouched():
     b = without.sample(x.cuda(), cond_fea=fea.cuda(), seeds=seeds)
     assert torch.equal(a, b)
     r = u.runner(fx["B"], 32, 32, fea.shape[-1])
-    assert not r.solver_graphs
+    assert not any(k[0] == "solver" for k in r.graphs)

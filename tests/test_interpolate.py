@@ -286,7 +286,7 @@ def test_interp_ancestral_matches_reference():
 
 
 @pytest.mark.gpu
-def test_interp_ancestral_shares_p_sample_loop_noise():
+def test_interp_ancestral_shares_p_sample_loop_graph_and_noise():
     """Seeded ancestral interpolation replays p_sample_loop's captured iteration from row T - t, and its loop noise at
     timestep tau is p_sample_loop's with the same seed: feeding the same draws as injected noise gives the same output.
     p_sample_loop is unchanged around it."""
@@ -297,9 +297,9 @@ def test_interp_ancestral_shares_p_sample_loop_noise():
     seeds = torch.tensor([17, 2 ** 50 + 5][:B])
     before = d.p_sample_loop(x, shape, fea, seeds=seeds)
     r = d.denoise_fn.runner(B, 32, 32, fea.shape[-1])
-    n_graphs = len(r.ddpm_graphs)
+    n_graphs = sum(k[0] == "ddpm" for k in r.graphs)
     got = d.interpolate(x1, x2, x, fea, t=t, lam=0.6, seeds=seeds)
-    assert len(r.ddpm_graphs) == n_graphs                       # the same captured iteration
+    assert sum(k[0] == "ddpm" for k in r.graphs) == n_graphs      # the same captured iteration
     from test_ddpm import _draws
     n = math.prod(shape[1:])
     e1, e2 = _interp_eps(seeds, shape, t, T)
@@ -349,7 +349,7 @@ def test_interp_ddim_matches_reference():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("S", [5, 20])
-def test_interp_seeds(S):
+def test_interp_seeds_graph_cache(S):
     """Seeds: graph == eager, one capture for two seed vectors, a sweep equals single calls, video b alone against the
     batch of 3 within the batch-independence gate, default seeds from torch's generator."""
     T = 1000 if S < 20 else 20
@@ -362,10 +362,10 @@ def test_interp_seeds(S):
     d.use_cuda_graph = True
     assert torch.equal(d.interpolate(x1, x2, x, fea, t=t, lam=0.4, seeds=seeds), eager)
     r = d.denoise_fn.runner(3, 32, 32, fea.shape[-1])
-    graphs = r.interp_graphs if S < 20 else r.ddpm_graphs
-    n_graphs = len(graphs)
+    kind = "interp" if S < 20 else "ddpm"
+    n_graphs = sum(k[0] == kind for k in r.graphs)
     again = d.interpolate(x1, x2, x, fea, t=t, lam=0.4, seeds=(seeds + 1).cuda())
-    assert len(graphs) == n_graphs and not torch.equal(again, eager)
+    assert sum(k[0] == kind for k in r.graphs) == n_graphs and not torch.equal(again, eager)
     sweep = d.interpolate(x1, x2, x, fea, t=t, lam=[0.4, 0.9], seeds=seeds)
     assert torch.equal(sweep[0], eager)
     assert torch.equal(sweep[1], d.interpolate(x1, x2, x, fea, t=t, lam=0.9, seeds=seeds))

@@ -12,7 +12,6 @@ limit.  Prints one JSON line.  --profile DIR writes a torch.profiler chrome trac
 import argparse
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,28 +19,9 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs, ops  # noqa: E402
+from benchlib import event_ms, power_limit  # noqa: E402
 
 DDIM_STEPS, DDPM_STEPS = 10, 1000
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn, n=1):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    for _ in range(n):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / n
 
 
 def use(diff, steps):
@@ -87,7 +67,7 @@ def bench(name, B, repeats, profile_dir):
     r.set_conditioning(x_cond.float(), cond_fea.float())
     prologue = graph_ms(r.run_prologue, 10)
     time_mlp = graph_ms(r.time_rec.run, 50)
-    _, st = next(iter(r.ddpm_graphs.values()))
+    _, st = next(v for k, v in r.graphs.items() if k[0] == "ddpm")
     broadcast = graph_ms(lambda: ops.ddpm_broadcast_row(ops.IMMEDIATE, st["ss_rows"], st["step"], r.ss), 50)
     ddim_round, ddpm_round = min(t["ddim"]), min(t["ddpm"])
     ddim_step = (ddim_round - prologue) / DDIM_STEPS
@@ -97,7 +77,7 @@ def bench(name, B, repeats, profile_dir):
         from torch.profiler import ProfilerActivity, profile
         os.makedirs(profile_dir, exist_ok=True)
         use(diff, DDPM_STEPS)
-        g, st = next(iter(r.ddpm_graphs.values()))
+        g, st = next(v for k, v in r.graphs.items() if k[0] == "ddpm")
         st["step"].zero_()                          # replay from the first step, as a round does
         r.time.fill_(DDPM_STEPS - 1)
         with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:

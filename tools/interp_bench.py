@@ -16,7 +16,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -24,32 +23,7 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs, ops  # noqa: E402
-
-HBM_BYTES_PER_S = 7.7e12
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn, reps=1):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    for _ in range(reps):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / reps
-
-
-def spread(xs):
-    return {"median": round(statistics.median(xs), 3), "min": round(min(xs), 3), "max": round(max(xs), 3)}
+from benchlib import HBM_BYTES_PER_S, event_ms, power_limit, spread  # noqa: E402
 
 
 def kernel_time(diff, B, n, injected):

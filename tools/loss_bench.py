@@ -21,7 +21,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -29,33 +28,9 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs, ops  # noqa: E402
+from benchlib import HBM_BYTES_PER_S, event_ms, power_limit, spread  # noqa: E402
 
-HBM_BYTES_PER_S = 7.7e12
 KERNEL_REPS = 200
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn, reps=1):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    for _ in range(reps):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / reps
-
-
-def spread(xs):
-    return {"median": round(statistics.median(xs), 3), "min": round(min(xs), 3), "max": round(max(xs), 3)}
 
 
 def bench(name, B, rounds):
@@ -90,7 +65,7 @@ def bench(name, B, rounds):
     # the new kernels alone, on the graph's buffers
     x_start = inputs[0]
     r = diff.denoise_fn.runner(B, x_start.shape[3], x_start.shape[4], inputs[2].shape[-1])
-    g, st = next(v for k, v in r.loss_graphs.items() if k[0] == tuple(x_start.shape))
+    g, st = next(v for k, v in r.graphs.items() if k[:2] == ("loss", tuple(x_start.shape)))
     R = ops.IMMEDIATE
     q_ms = event_ms(lambda: ops.q_sample(R, st["x_start"], r.time, st["seeds"], None, st["acp"], st["a1m"], r.x,
                                          st["eps"]), KERNEL_REPS)

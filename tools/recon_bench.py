@@ -18,7 +18,6 @@ import json
 import math
 import os
 import statistics
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -28,29 +27,7 @@ import torch.nn.functional as F  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs  # noqa: E402
 from extdm_b200.flow_autoenc import FlowAE  # noqa: E402
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    out = fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b), out
-
-
-def spread(xs):
-    return {"median": round(statistics.median(xs), 1), "min": round(min(xs), 1), "max": round(max(xs), 1)}
+from benchlib import event_ms, power_limit, spread  # noqa: E402
 
 
 def bench(name, batch, rounds):
@@ -88,13 +65,11 @@ def bench(name, batch, rounds):
     times = {k: [] for k in arms}
     for _ in range(rounds):
         for k, fn in arms.items():
-            ms, out = event_ms(fn)
-            del out
-            times[k].append(ms)
+            times[k].append(event_ms(fn))
     frames = batch * T
     res = {"dataset": name, "batch": batch, "frames_per_video": T, "hw": hw}
     for k, ts in times.items():
-        res[f"{k}_frames_per_s"] = spread([frames / (t / 1e3) for t in ts])
+        res[f"{k}_frames_per_s"] = spread([frames / (t / 1e3) for t in ts], digits=1)
         res[f"{k}_ms"] = [round(t, 2) for t in ts]
     med = {k: statistics.median(ts) for k, ts in times.items()}
     res["speedup_vs_torch_default"] = round(med["torch_default"] / med["native_graph"], 2)

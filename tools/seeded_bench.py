@@ -14,7 +14,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -22,27 +21,9 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs  # noqa: E402
+from benchlib import event_ms, power_limit, spread  # noqa: E402
 
 STEPS = 10
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b)
 
 
 def noise_state_bytes(shape, steps, B):
@@ -52,10 +33,6 @@ def noise_state_bytes(shape, steps, B):
     for d in shape:
         n *= d
     return 2 * steps * n, 8 * B
-
-
-def spread(xs):
-    return {"median": round(statistics.median(xs), 3), "min": round(min(xs), 3), "max": round(max(xs), 3)}
 
 
 def bench(name, B, rounds):

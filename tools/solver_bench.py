@@ -17,7 +17,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -25,35 +24,11 @@ sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 import extdm_b200  # noqa: E402,F401
 from extdm_b200 import configs, ops  # noqa: E402
+from benchlib import HBM_BYTES_PER_S, event_ms, power_limit, spread  # noqa: E402
 
 ARMS = [("ddim", None, 10), ("dpmpp_2m", "dpmpp_2m", 5), ("dpmpp_2m", "dpmpp_2m", 10),
         ("dpmpp_2m_sde", "dpmpp_2m_sde", 10)]
-HBM_BYTES_PER_S = 7.7e12
 BYTES_PER_ELEMENT = 20
-
-
-def power_limit():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader",
-                              f"--id={torch.cuda.current_device()}"], capture_output=True, text=True, timeout=30)
-        return out.stdout.strip() or "unknown"
-    except (OSError, subprocess.SubprocessError):
-        return "unknown"
-
-
-def event_ms(fn, reps=1):
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    a.record()
-    for _ in range(reps):
-        fn()
-    b.record()
-    torch.cuda.synchronize()
-    return a.elapsed_time(b) / reps
-
-
-def spread(xs):
-    return {"median": round(statistics.median(xs), 3), "min": round(min(xs), 3), "max": round(max(xs), 3)}
 
 
 def kernel_time(B, n, sde):
