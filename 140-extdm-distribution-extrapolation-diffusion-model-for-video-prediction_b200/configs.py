@@ -73,14 +73,19 @@ def build_model(name, seed=1234, device="cuda"):
     return model.to(device), cfg
 
 
-def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None, seeds=None):
+def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None, seeds=None, keyframes=None):
     """Autoregressive rollout of scripts/DM/valid.py:167-172 -> (B, 3, total_pred, H, W).
     host_buffers=None keeps every round on the device (SURVEY.md section 8f-2).  With
     host_buffers=(pinned_in, pinned_out) each round copies its conditioning clip host->device and its
     sample_out_vid device->host exactly like the reference driver (`.cuda()` / `.cpu()` per round).
     seeds: optional per-video base seeds ((B,) int64 tensor or list); round r samples video b with the seed
     sharding.video_seeds(seeds[b], 0, r), so every round draws fresh noise and a video's rollout depends on its own
-    base seed only."""
+    base seed only.
+    keyframes: optional (frames (B, 3, total_pred, H, W) in [0, 1], mask (B, total_pred) bool): predicted frame j of
+    video b is known to be frames[b, :, j] where mask[b, j].  Round r imposes the known frames of its window
+    [r*tp, (r+1)*tp) with FlowDiffusion.sample_with_keyframes, encoded against that round's source frame (a predicted
+    frame after round 0); a round without a known frame calls sample_one_video as without keyframes.  Keyframes take
+    seeds or the default noise, not noise_fn."""
     import math
     import torch
     from .sharding import video_seeds
@@ -89,18 +94,38 @@ def rollout(model, clip, total_pred, host_buffers=None, noise_fn=None, seeds=Non
     if seeds is not None and len(seeds) != clip.shape[0]:
         raise ValueError(f"rollout: {len(seeds)} seeds for {clip.shape[0]} videos")
     tc, tp = model.cond_frame_num, model.pred_frame_num
+    n_rounds = math.ceil(total_pred / tp)
+    if keyframes is not None:
+        if noise_fn is not None:
+            raise ValueError("rollout: keyframes take seeds or the default noise, not noise_fn")
+        kf_frames, kf_mask = keyframes
+        B, _, _, H, W = clip.shape
+        if not torch.is_tensor(kf_frames) or tuple(kf_frames.shape) != (B, 3, total_pred, H, W):
+            raise ValueError(f"rollout: keyframe frames must be a ({B}, 3, {total_pred}, {H}, {W}) tensor")
+        if not torch.is_tensor(kf_mask) or kf_mask.dtype != torch.bool or tuple(kf_mask.shape) != (B, total_pred):
+            raise ValueError(f"rollout: the keyframe mask must be a ({B}, {total_pred}) bool tensor")
+        pad = n_rounds * tp - total_pred                         # the last round's window may reach past total_pred
+        kf_mask = torch.cat([kf_mask.cpu(), torch.zeros(B, pad, dtype=torch.bool)], dim=1)
+        kf_frames = torch.cat([kf_frames, kf_frames.new_zeros(B, 3, pad, H, W)], dim=2)
     preds = []
     cond = clip
-    for r in range(math.ceil(total_pred / tp)):
+    for r in range(n_rounds):
         if host_buffers is not None:
             pin_in, pin_out = host_buffers
             pin_in.copy_(cond)                                   # host -> pinned staging (host memcpy)
             dev_in = pin_in.to("cuda", non_blocking=True)
         else:
             dev_in = cond
-        out = model.sample_one_video(cond_scale=1.0, real_vid=dev_in,
-                                     noise=None if noise_fn is None else noise_fn(),
-                                     seeds=None if seeds is None else video_seeds(seeds, 0, r))["sample_out_vid"]
+        round_seeds = None if seeds is None else video_seeds(seeds, 0, r)
+        window = slice(r * tp, (r + 1) * tp)
+        if keyframes is not None and bool(kf_mask[:, window].any()):
+            real_vid = torch.cat([dev_in, kf_frames[:, :, window].to(dev_in.device, dev_in.dtype)], dim=2)
+            out = model.sample_with_keyframes(real_vid, kf_mask[:, window].contiguous(),
+                                              seeds=round_seeds)["sample_out_vid"]
+        else:
+            out = model.sample_one_video(cond_scale=1.0, real_vid=dev_in,
+                                         noise=None if noise_fn is None else noise_fn(),
+                                         seeds=round_seeds)["sample_out_vid"]
         if host_buffers is not None:
             pin_out.copy_(out, non_blocking=True)
             torch.cuda.current_stream().synchronize()

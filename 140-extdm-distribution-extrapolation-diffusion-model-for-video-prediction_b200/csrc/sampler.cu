@@ -11,6 +11,8 @@
 // of its stochastic variant from that generator too (stream 3).
 // Interpolation between two futures (GaussianDiffusion.interpolate) mixes their forward diffusions in one kernel, with
 // each endpoint's epsilon from that generator (streams 4 and 5), then runs the DDIM or ancestral loop above.
+// Keyframe-conditioned sampling (GaussianDiffusion.sample_with_known) overwrites the known frames after every update
+// with the forward diffusion of their latent, its epsilon from that generator too (stream 6).
 #include "common.cuh"
 #include "../../include/extdm_b200.h"
 
@@ -380,6 +382,63 @@ __global__ void __launch_bounds__(256) q_interpolate_kernel(const float* __restr
   }
 }
 
+// ------------------------------------------------------------------------------------------------ keyframes
+// Philox counter word 2 of the replacement noise of keyframe-conditioned sampling; word 1 is the replacement point k
+constexpr unsigned int kStreamKnown = 6u;
+// One row per replacement point of the ancestral loop: {a_k, b_k, final}
+constexpr int kKnownRow = 3;
+
+// Replacement point k of GaussianDiffusion.sample_with_known on (B, 3, tp, hw) tensors: every quad of frame f of video b
+// with known[b, f] becomes q_sample_of(x_known, eps_k, a, c), or x_known itself when final; a quad of an unknown frame is
+// neither read from x_known nor written.  eps_k is noise[k] of (K, B, n) when noise is given, else the Philox draw of
+// (seeds[b], k, stream 6).  hw4 = hw / 4 quads per (channel, frame) plane, so a quad never straddles two frames.
+__device__ __forceinline__ void impose_known_quads(float* x, const float* __restrict__ x_known,
+                                                   const unsigned char* __restrict__ known,
+                                                   const long long* __restrict__ seeds,
+                                                   const float* __restrict__ noise, float a, float c, unsigned int k,
+                                                   bool final, int tp, int hw4, int n4_per_sample, long long total4) {
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < total4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long b = i / n4_per_sample;
+    const unsigned int quad = static_cast<unsigned int>(i - b * n4_per_sample);
+    if (!__ldg(known + b * tp + (quad / hw4) % tp)) continue;
+    const float4 xk = reinterpret_cast<const float4*>(x_known)[i];
+    float4 o = xk;
+    if (!final) {
+      const float4 e = noise ? reinterpret_cast<const float4*>(noise)[static_cast<long long>(k) * total4 + i]
+                             : normal4(__ldg(seeds + b), quad, k, kStreamKnown);
+      o = make_float4(q_sample_of(xk.x, e.x, a, c), q_sample_of(xk.y, e.y, a, c), q_sample_of(xk.z, e.z, a, c),
+                      q_sample_of(xk.w, e.w, a, c));
+    }
+    reinterpret_cast<float4*>(x)[i] = o;
+  }
+}
+
+// DDIM: (a, c, k, final) are launch scalars, baked into the captured loop.
+__global__ void __launch_bounds__(256) impose_known_kernel(float* x, const float* __restrict__ x_known,
+                                                           const unsigned char* __restrict__ known,
+                                                           const long long* __restrict__ seeds,
+                                                           const float* __restrict__ noise, float a, float c,
+                                                           unsigned int k, int final, int tp, int hw4,
+                                                           int n4_per_sample, long long total4) {
+  impose_known_quads(x, x_known, known, seeds, noise, a, c, k, final != 0, tp, hw4, n4_per_sample, total4);
+}
+
+// Ancestral: k = *step, the counter ddpm_update reads, and (a, c, final) its row of the device table, so one captured
+// iteration serves every replacement point.
+__global__ void __launch_bounds__(256) impose_known_table_kernel(float* x, const float* __restrict__ x_known,
+                                                                 const unsigned char* __restrict__ known,
+                                                                 const long long* __restrict__ seeds,
+                                                                 const float* __restrict__ noise,
+                                                                 const float* __restrict__ rows,
+                                                                 const int* __restrict__ step, int tp, int hw4,
+                                                                 int n4_per_sample, long long total4) {
+  const int k = __ldg(step);
+  const float* row = rows + static_cast<long long>(k) * kKnownRow;
+  impose_known_quads(x, x_known, known, seeds, noise, __ldg(row + 0), __ldg(row + 1), static_cast<unsigned int>(k),
+                     __ldg(row + 2) != 0.f, tp, hw4, n4_per_sample, total4);
+}
+
 // One block per (video b, frame f) of (B, 3, tp, hw) tensors: out[b, f] = mean over (3, hw) of (eps - pred)^2 (or
 // |eps - pred|).  The difference of two floats is exact in double, so the terms are exact and the sum is in fp64; each
 // thread sums a fixed strided subset in order, then a fixed shared-memory tree: the result depends on the (b, f) slice
@@ -568,6 +627,29 @@ extern "C" int extdm_q_interpolate(const float* x1, const float* x2, int t, cons
   const long long total4 = static_cast<long long>(B) * n / 4;
   q_interpolate_kernel<<<ddpm_grid(total4), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       x1, x2, t, seeds, noise, sqrt_acp, sqrt_1m_acp, c1, c2, x_t_out, n / 4, total4);
+  EXTDM_CHECK_LAUNCH();
+  return EXTDM_OK;
+}
+
+extern "C" int extdm_impose_known(float* x, const float* x_known, const unsigned char* known, const long long* seeds,
+                                  const float* noise, float a, float b, int k, int final, const float* rows,
+                                  const int* step, int B, int tp, int hw, void* stream) {
+  if (B < 1 || tp < 1 || hw < 4 || hw % 4 || !x || !x_known || !known || (!noise == !seeds) || (!rows != !step) ||
+      (!rows && k < 0) || static_cast<long long>(3) * tp * hw > 0x7FFFFFFFLL) {
+    extdm_set_error("impose_known: need B, tp >= 1, h*w a positive multiple of 4, x, x_known, known, exactly one of "
+                    "seeds and noise, rows and step together (or k >= 0)", __FILE__, __LINE__);
+    return EXTDM_ERR_ARG;
+  }
+  const int n4 = 3 * tp * (hw / 4);
+  const long long total4 = static_cast<long long>(B) * n4;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (rows)
+    impose_known_table_kernel<<<ddpm_grid(total4), 256, 0, st>>>(x, x_known, known, seeds, noise, rows, step, tp,
+                                                                 hw / 4, n4, total4);
+  else
+    impose_known_kernel<<<ddpm_grid(total4), 256, 0, st>>>(x, x_known, known, seeds, noise, a, b,
+                                                           static_cast<unsigned int>(k), final != 0, tp, hw / 4, n4,
+                                                           total4);
   EXTDM_CHECK_LAUNCH();
   return EXTDM_OK;
 }

@@ -14,6 +14,9 @@ evaluations on DDIM's timestep grid, the whole loop captured as one CUDA graph a
 forward diffusion to one timestep per video, one UNet forward, the per-(video, frame) loss, as one CUDA graph.
 `interpolate()` (Diffusion.py:261-274) mixes the forward diffusions of two futures at one timestep and denoises the
 mix with the DDIM or the ancestral loop.
+`sample_with_known()` runs the DDIM or the ancestral loop with some future frames known: after every update each known
+frame is replaced by the forward diffusion of its latent to the level of the state (Song et al. 2021, Lugmayr et al.
+2022).
 Training itself (gradients, optimisers) is out of scope.
 """
 import math
@@ -96,7 +99,8 @@ def _require_cuda(x, who):
 
 
 def _load_seeds(dst, seeds):
-    """dst (device) <- seeds without a host synchronisation: host seeds go through pinned memory."""
+    """dst (device) <- seeds (or another call input) without a host synchronisation: host tensors go through pinned
+    memory."""
     dst.copy_(seeds.pin_memory() if seeds.device.type == "cpu" else seeds, non_blocking=True)
 
 
@@ -164,7 +168,8 @@ class GaussianDiffusion(nn.Module):
         for every later call with this key.  Otherwise run calls body on a fresh state.  Captured graphs hold raw
         pointers into the runner's weight and activation buffers, so they live ON the runner, in r.graphs:
         Unet3D.invalidate() (load_state_dict, device move) drops runner and graphs together.  The key starts with the
-        kind of loop ("ddim", "ddpm", "solver", "loss", "interp") and holds everything the capture bakes in."""
+        kind of loop ("ddim", "ddpm", "solver", "loss", "interp", "known_ddim", "known_ddpm") and holds everything the
+        capture bakes in."""
         if trace is not None or not self.use_cuda_graph:
             st = make_state()
             return st, lambda: body(st)
@@ -262,20 +267,24 @@ class GaussianDiffusion(nn.Module):
         return (kind, tuple(shape), float(self.ddim_sampling_eta), float(self.dynamic_thres_percentile),
                 int(self.sampling_timesteps), int(self.num_timesteps))
 
-    def _ddim_loop(self, r, sched, st, trace=None):
+    def _ddim_loop(self, r, sched, st, trace=None, after=None):
         """UNet prologue, x_T, then the DDIM iterations.  The noise is st["noise"][0] (x_T) and st["noise"][i + 1]
-        (iteration i), or, when st holds "seeds", the Philox draws of those seeds."""
+        (iteration i), or, when st holds "seeds", the Philox draws of those seeds.  after: optional hook, after(0) once
+        x_T is written, then as in _ddim_steps."""
         r.run_prologue()
         if st["seeds"] is not None:
             ops.ddpm_fill_normal(ops.IMMEDIATE, st["seeds"], r.x)
         else:
             r.x.copy_(st["noise"][0])
+        if after is not None:
+            after(0)
         return self._ddim_steps(r, sched, None if st["noise"] is None else st["noise"][1:], st["seeds"], st["s"],
-                                trace)
+                                trace, after)
 
-    def _ddim_steps(self, r, sched, noise, seeds, s, trace=None):
+    def _ddim_steps(self, r, sched, noise, seeds, s, trace=None, after=None):
         """The DDIM iterations of sched from r.x (after the UNet prologue): the noise of iteration i is noise[i], or,
-        with seeds, the Philox draw of (seeds[b], i, stream 0)."""
+        with seeds, the Philox draw of (seeds[b], i, stream 0).  after: optional hook, after(i + 1) once iteration i has
+        written r.x (keyframe replacement)."""
         rec = ops.IMMEDIATE
         q = float(self.dynamic_thres_percentile)
         ss = r.ss_for_times([s_[0] for s_ in sched])       # evaluated once per schedule, outside the captured loop
@@ -296,6 +305,8 @@ class GaussianDiffusion(nn.Module):
                 ops.ddim_update(rec, r.x, r.out, nz, s, c_recip, c_recipm1, san, c, sigma, r.x, xs)
             if trace is not None:
                 trace[-1].update(x_start=xs, s=s.clone(), img=r.x.clone())
+            if after is not None:
+                after(i + 1)
         return r.x
 
     # ------------------------------------------------------------------ DDPM (ancestral) sampler
@@ -728,3 +739,151 @@ class GaussianDiffusion(nn.Module):
                 run()
             outs.append(r.x.clone())
         return torch.stack(outs) if sweep else outs[0]
+
+    # ------------------------------------------------------------------ keyframes: known future frames imposed
+    def known_schedule(self):
+        """[(a_k, b_k, final)] for the replacement points k = 0 .. K of sample_with_known (DESIGN.md section 1): K = S =
+        sampling_timesteps for DDIM, K = num_timesteps for the ancestral loop.  Point k < K puts the known frames at the
+        level tau_k of the state the sampler has just produced:
+          * DDIM: tau_k = the k-th timestep of ddim_schedule's grid (t_0 for x_T, then iteration k-1's time_next);
+            a_k = alphas_cumprod_prev[tau].sqrt(), b_k = (1 - alphas_cumprod_prev[tau]).sqrt(), so a_k is the
+            sqrt_alpha_next of ddim_schedule's row k - 1, bit for bit.
+          * ancestral: tau_k = num_timesteps - 1 - k; a_k, b_k = sqrt_alphas_cumprod[tau],
+            sqrt_one_minus_alphas_cumprod[tau], as q_sample reads them.
+        Row K, after the update that reaches time 0, is final, (1.0, 0.0, True): x_known is copied verbatim.  fp32 torch
+        ops on the module's buffers (a checkpoint may overwrite them), on the host.  A selected solver is a ValueError."""
+        if self.solver is not None:
+            raise ValueError(f"sample_with_known: keyframes run the DDIM or the ancestral loop, not {self.solver!r}")
+        if self.is_ddim_sampling:
+            prev = self.alphas_cumprod_prev.detach().cpu()
+            rows = [(prev[t].sqrt().item(), (1 - prev[t]).sqrt().item(), False)
+                    for t in self._ddim_times(self.sampling_timesteps)[:-1]]
+        else:
+            T = self.num_timesteps
+            a, b = self.sqrt_alphas_cumprod.detach().cpu(), self.sqrt_one_minus_alphas_cumprod.detach().cpu()
+            rows = [(a[T - 1 - k].item(), b[T - 1 - k].item(), False) for k in range(T)]
+        return rows + [(1.0, 0.0, True)]
+
+    def known_args(self, shape, known, tc, seeds=None, noise=None, who="sample_with_known"):
+        """Check the arguments of sample_with_known for a latent of `shape` (B, 3, tp, h, w) and tc conditioning frames
+        on the host, before anything is launched: the solver, the shape, the (B, tp) bool mask, the seeds
+        (_seed_vector, not together with noise) and the noise ((2S, *shape) DDIM, (2T + 1, *shape) ancestral, fp32).
+        Returns the seeds, None when not given."""
+        if self.solver is not None:
+            raise ValueError(f"{who}: keyframes run the DDIM or the ancestral loop, not {self.solver!r}")
+        B, C, tp, h, w = shape
+        if B < 1 or C != 3 or tc + tp != self.num_frames:
+            raise ValueError(f"{who}: latent {tuple(shape)}: expected (B >= 1, 3, {self.num_frames - tc}, h, w)")
+        if (h * w) % 4:
+            raise ValueError(f"{who}: h * w = {h * w} must be a multiple of 4")
+        if not torch.is_tensor(known) or known.dtype != torch.bool or tuple(known.shape) != (B, tp):
+            got = f"{known.dtype} {tuple(known.shape)}" if torch.is_tensor(known) else type(known).__name__
+            raise ValueError(f"{who}: known must be a ({B}, {tp}) bool tensor, got {got}")
+        seeds = _seed_vector(seeds, noise, B, who)
+        S, T = int(self.sampling_timesteps), self.num_timesteps
+        _check_noise(noise, (2 * S if self.is_ddim_sampling else 2 * T + 1, *shape), who, "float32")
+        return seeds
+
+    @torch.no_grad()
+    def sample_with_known(self, x_cond, cond_fea, x_known, known, seeds=None, noise=None):
+        """sample() with some future frames known (DESIGN.md section 1): x_known (B, 3, tp, h, w) fp32, the latent of the
+        known frames (values at unknown frames are never read), known (B, tp) bool, one flag per (video, predicted
+        frame); x_cond, cond_fea as for sample().  Runs the loop sample() would pick (DDIM if sampling_timesteps <
+        timesteps, else ancestral; a selected solver is a ValueError) with its own noise unchanged, and after x_T and
+        after every update overwrites each known frame with
+
+            x = a_k * x_known + b_k * eps_k          (fp32, no FMA; known_schedule holds a_k, b_k)
+
+        at the level the update has just produced; the last replacement copies x_known, so the known frames of the
+        result equal x_known bit for bit.  Unknown frames are never written by the replacement.
+
+        seeds: optional (B,) int64 tensor or list; the loop noise is then that of ddim_sample / p_sample_loop with these
+        seeds, and eps_k of video b the Philox draw of (seeds[b], k, stream 6) (include/extdm_b200.h).  Default: seeds
+        drawn from torch's default generator, as p_sample_loop does.  noise: optional tensor instead of seeds, the plain
+        sampler's noise followed by the replacement draws: (2S, *shape) for DDIM (noise[:S] as in ddim_sample, noise[S +
+        k] = eps_k), (2T + 1, *shape) ancestral (noise[:T + 1] as in p_sample_loop, noise[T + 1 + k] = eps_k).
+
+        Each loop is one entry of the runner's graphs (_graph, keys "known_ddim": the whole loop, "known_ddpm": one
+        iteration read through the step counter); the mask, x_known and the seeds are staged into its state before
+        each replay without a host synchronisation, so one capture serves every mask, keyframe and seed vector.
+        Argument errors raise ValueError before anything runs; CPU tensors then RuntimeError."""
+        if not all(torch.is_tensor(v) and v.dim() == 5 for v in (x_cond, cond_fea)):
+            raise ValueError("sample_with_known: x_cond and cond_fea must be 5-D tensors")
+        if not torch.is_tensor(x_known) or x_known.dim() != 5 or x_known.dtype != torch.float32:
+            raise ValueError("sample_with_known: x_known must be a (B, 3, tp, h, w) float32 tensor")
+        tc = x_cond.shape[2]
+        seeds = self.known_args(tuple(x_known.shape), known, tc, seeds, noise)
+        shape = tuple(x_known.shape)
+        B, _, tp, h, w = shape
+        if tuple(x_cond.shape) != (B, 3, tc, h, w) or cond_fea.shape[0] != B:
+            raise ValueError(f"sample_with_known: x_cond {tuple(x_cond.shape)}, cond_fea {tuple(cond_fea.shape)}: "
+                             f"expected ({B}, 3, {tc}, {h}, {w}) and ({B}, ...)")
+        self._check_thresholding()
+        _require_cuda(x_known, "sample_with_known")
+        seeds = _default_seeds(seeds, noise, B)
+        r = self.denoise_fn.runner(B, h, w, cond_fea.shape[-1])
+        injected = noise is not None
+        krows = self.known_schedule()
+        K = len(krows) - 1
+        n_plain = K if self.is_ddim_sampling else K + 1          # the plain sampler's share of an injected noise tensor
+
+        def known_state(st):
+            st.update(x_known=torch.zeros(shape, device=r.dev), known=torch.zeros(B, tp, dtype=torch.bool, device=r.dev),
+                      eps=torch.zeros(K, *shape, device=r.dev) if injected else None)
+            return st
+
+        def stage_known(st):
+            _load_seeds(st["x_known"], x_known)                  # no host sync before the launches / replay
+            _load_seeds(st["known"], known)
+            if injected:
+                st["eps"].copy_(noise[n_plain:])
+
+        def impose(st, k=0, table=None):
+            """Replacement point k (scalars of krows), or, with the device table, the point the step counter holds."""
+            a, b, final = krows[k] if table is None else (0.0, 0.0, False)
+            ops.impose_known(ops.IMMEDIATE, r.x, st["x_known"], st["known"], None if injected else st["seeds"],
+                             st["eps"], a, b, k, final, table, None if table is None else st["step"])
+
+        if self.is_ddim_sampling:
+            sched = self.ddim_schedule()
+
+            def state():
+                return known_state(dict(s=torch.zeros(B, device=r.dev),
+                                        seeds=torch.zeros(B, dtype=torch.long, device=r.dev) if not injected else None,
+                                        noise=torch.zeros(K, *shape, device=r.dev) if injected else None))
+
+            def stage(st):
+                r.set_conditioning(x_cond.float(), cond_fea.float())
+                if injected:
+                    st["noise"].copy_(noise[:n_plain])
+                else:
+                    _load_seeds(st["seeds"], seeds)
+                stage_known(st)
+
+            # the schedule scalars and the replacement coefficients are baked into the capture, hence part of the key
+            st, run = self._graph(r, self._ddim_key("known_ddim", shape) + (injected,), state, stage,
+                                  lambda st: self._ddim_loop(r, sched, st, after=lambda k: impose(st, k)))
+            stage(st)
+            run()
+            return r.x.clone()
+
+        def state():
+            st = known_state(self._ddpm_state(r, injected))
+            st["krows"] = torch.tensor([[a, b, float(f)] for a, b, f in krows], dtype=torch.float32, device=r.dev)
+            return st
+
+        def start(st):
+            self._ddpm_round(r, st, x_cond, cond_fea, seeds, noise[:n_plain] if injected else None)
+            stage_known(st)
+            impose(st, table=st["krows"])                        # step = 0: x_T
+
+        def iteration(st):
+            self._ddpm_iteration(r, st)
+            impose(st, table=st["krows"])                        # after ddpm_advance: step = k = row + 1
+
+        st, run = self._graph(r, ("known_ddpm", shape, float(self.dynamic_thres_percentile), self.num_timesteps,
+                                  injected), state, start, iteration)
+        start(st)
+        for _ in range(self.num_timesteps):
+            run()
+        return r.x.clone()

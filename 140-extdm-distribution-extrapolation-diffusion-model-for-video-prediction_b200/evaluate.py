@@ -22,6 +22,11 @@ Interpolation between two futures of the same past (e.g. the encoded ground trut
 
     x1 = model.encode_future(real_vids);  x2 = model.diffusion.sample(...)    # (B, 3, tp, h, w) latents
     origin, result = evaluate.interpolate_videos(model, real_vids, x1, x2, lams=[0.0, 0.25, 0.5, 0.75, 1.0], seed=0)
+
+Goal-conditioned prediction: the last predicted frame (e.g. the goal of a BAIR push) is known, taken from the ground
+truth, and imposed in its rollout round:
+
+    origin, result = evaluate.sample_videos(model, real_vids, total_pred, keyframes=[total_pred - 1], seed=0)
 """
 import os
 
@@ -48,7 +53,8 @@ def load_dm_checkpoint(model, ckpt):
 
 
 @torch.no_grad()
-def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=True, seed=None, video_offset=0):
+def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=True, seed=None, video_offset=0,
+                  keyframes=None):
     """valid.py:156-197 for one batch: real_vids (B, C, T, H, W) in [0,1] with T >= cond frames (+ total_pred ground
     truth frames if available) -> (origin, result), both (B, n, T', C, H, W) on the CPU, result = cond frames followed
     by total_pred predicted frames.  on_device=False reproduces the reference's per-round .cpu()/.cuda() hops.
@@ -56,7 +62,11 @@ def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=Tr
     seed: optional int.  Then repeat k of video b is sampled with the per-video base seed
     sharding.video_seeds(seed, (video_offset + b) * num_sample_video + k), a function of its *global* index only:
     a sharded evaluation passes video_offset = lo of sharding.shard_range and samples every video with the same noise
-    as a single-GPU run.  Default: the sampler's own noise (torch's default generator)."""
+    as a single-GPU run.  Default: the sampler's own noise (torch's default generator).
+
+    keyframes: optional list of predicted-frame indices in [0, total_pred), known for every video, or a (B, total_pred)
+    bool mask.  Those frames are taken from the ground truth real_vids[:, :, tc + j] (so T >= tc + total_pred) and
+    imposed in their rollout round (configs.rollout); the decoded known frames are their LFAE reconstructions."""
     from .configs import rollout
     from .sharding import video_seeds
     tc = model.cond_frame_num
@@ -67,12 +77,28 @@ def sample_videos(model, real_vids, total_pred, num_sample_video=1, on_device=Tr
     seeds = None
     if seed is not None:                                                            # row b*n + k of rep = (b, k)
         seeds = video_seeds(seed, torch.arange(B * num_sample_video) + video_offset * num_sample_video)
+    kf = None
+    if keyframes is not None:
+        if real_vids.shape[2] < tc + total_pred:
+            raise ValueError(f"sample_videos: keyframes need {tc + total_pred} ground-truth frames, got "
+                             f"{real_vids.shape[2]}")
+        if torch.is_tensor(keyframes):
+            if keyframes.dtype != torch.bool or tuple(keyframes.shape) != (B, total_pred):
+                raise ValueError(f"sample_videos: a keyframe mask must be a ({B}, {total_pred}) bool tensor")
+            mask = keyframes.cpu()
+        else:
+            idx = list(keyframes)
+            if any(isinstance(j, bool) or not isinstance(j, int) or not 0 <= j < total_pred for j in idx):
+                raise ValueError(f"sample_videos: keyframes must be ints in [0, {total_pred}), got {keyframes!r}")
+            mask = torch.zeros(B, total_pred, dtype=torch.bool)
+            mask[:, idx] = True
+        kf = (rep[:, :, tc:tc + total_pred].to(dev).float(), mask.repeat_interleave(num_sample_video, dim=0))
     if on_device:
-        pred = rollout(model, cond, total_pred, seeds=seeds)
+        pred = rollout(model, cond, total_pred, seeds=seeds, keyframes=kf)
     else:
         pin_in = torch.empty(cond.shape).pin_memory()
         pin_out = torch.empty(cond.shape[0], cond.shape[1], tc + model.pred_frame_num, *cond.shape[3:]).pin_memory()
-        pred = rollout(model, cond.cpu(), total_pred, host_buffers=(pin_in, pin_out), seeds=seeds)
+        pred = rollout(model, cond.cpu(), total_pred, host_buffers=(pin_in, pin_out), seeds=seeds, keyframes=kf)
     res = torch.cat([rep[:, :, :tc].cpu().float(), pred.cpu()], dim=2)
 
     def shape(t):                                                                   # '(b n) c t h w -> b n t c h w'

@@ -5,6 +5,7 @@ VideoFlowDiffusion_multi1248.py, VideoFlowDiffusion_multi.py) with the same cons
   (A) conditioning  : torch (RegionPredictor / BGMotionPredictor / Generator.forward), batched over the tc frames
   (B) denoise       : GaussianDiffusion.sample  -> CUDA-graphed UNet3D + DDIM kernels
                       (interpolate_one_video: GaussianDiffusion.interpolate between two given futures)
+                      (sample_with_keyframes: GaussianDiffusion.sample_with_known, some future frames given)
   (C) decode        : Generator.decode_video    -> CUDA warp / blend / conv kernels
 """
 import torch
@@ -234,6 +235,30 @@ class FlowDiffusion(nn.Module):
         parts = [self._decode_sample(ret, ref, p) for p in pred]
         for k in parts[0]:
             ret[k] = parts[0][k] if k.startswith("real_") else torch.stack([d[k] for d in parts])
+        return ret
+
+    # ------------------------------------------------------------------ prediction with known future frames
+    @torch.no_grad()
+    def sample_with_keyframes(self, real_vid, known, seeds=None, noise=None):
+        """sample_one_video with some future frames known: real_vid (B, 3, tc + tp, H, W) in [0, 1], known (B, tp) bool,
+        one flag per (video, predicted frame); future frames at unknown positions may hold anything.  x_cond, cond_fea
+        and the conditioning entries are condition(real_vid[:, :, :tc]), as sample_one_video computes them; the known
+        frames enter as encode_future(real_vid), the LFAE flow of each future frame from source frame tc - 1, imposed
+        with GaussianDiffusion.sample_with_known (seeds, noise as there).  Returns sample_one_video's dict, decoded the
+        same way.  The latent of a known frame is its encoding bit for bit, so its decoded RGB is the LFAE
+        reconstruction of the keyframe, not the keyframe itself.  Argument errors raise ValueError before anything
+        runs."""
+        tc, tp = self.cond_frame_num, self.pred_frame_num
+        if not torch.is_tensor(real_vid) or real_vid.dim() != 5 or real_vid.shape[1] != 3 or \
+                real_vid.shape[2] != tc + tp:
+            raise ValueError(f"sample_with_keyframes: real_vid must be a (B, 3, {tc + tp} = tc + tp, H, W) tensor")
+        B, _, _, H, W = real_vid.shape
+        st = int(round(1 / self.region_predictor.scale_factor))
+        self.diffusion.known_args((B, 3, tp, H // st, W // st), known, tc, seeds, noise, who="sample_with_keyframes")
+        ret, x_cond, cond_fea, ref = self.condition(real_vid[:, :, :tc].contiguous())
+        x_known = self.encode_future(real_vid)
+        pred = self.diffusion.sample_with_known(x_cond, cond_fea, x_known, known, seeds=seeds, noise=noise)
+        ret.update(self._decode_sample(ret, ref, pred))
         return ret
 
     # ------------------------------------------------------------------ denoising loss (forward-only training objective)

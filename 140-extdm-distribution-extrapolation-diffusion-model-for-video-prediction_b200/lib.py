@@ -88,6 +88,7 @@ PROTOTYPES = {
     "extdm_q_sample": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P],
     "extdm_denoise_loss": [_P, _P, _P, _I, _I, _I, _I, _P],
     "extdm_q_interpolate": [_P, _P, _I, _P, _P, _P, _P, _F, _F, _P, _I, _I, _P],
+    "extdm_impose_known": [_P, _P, _P, _P, _P, _F, _F, _I, _I, _P, _P, _I, _I, _I, _P],
     "extdm_warp_blend_cl": [_P, _P, _P, _P, _P, _L, _L, _I, _I, _I, _I, _I, _I, _P],
     "extdm_warp_image": [_P, _P, _I, _P, _P, _P, _P, _L, _L, _I, _I, _I, _I, _P],
     "extdm_warp_taps": [_P, _P, _P, _P, _P, _L, _I, _I, _I, _I, _P],

@@ -702,6 +702,43 @@ def q_interpolate(rec, x1, x2, t, seeds, noise, sqrt_acp, sqrt_1m_acp, c1, c2, x
              keep=(x1, x2, seeds, noise, sqrt_acp, sqrt_1m_acp, x_t))
 
 
+def impose_known(rec, x, x_known, known, seeds, noise, a=0.0, b=0.0, k=0, final=False, rows=None, step=None):
+    """Replacement point k of keyframe-conditioned sampling, in place on x (B, 3, tp, h, w): the frames f of video b with
+    known[b, f] ((B, tp) bool) become a * x_known + b * eps_k, or x_known itself when final; other frames are untouched.
+    eps_k = noise[k] ((K, *x.shape)) when given, else the Philox draw of (seeds[b], k, stream 6).  With rows ((K + 1, 3)
+    {a, b, final}) and step (one int32), k = step and (a, b, final) = rows[k] on the device instead."""
+    for v, name in ((x, "x"), (x_known, "x_known")):
+        if v is None:
+            raise ValueError(f"impose_known: {name} is required")
+        _chk(v, torch.float32, name)
+    _chk(known, torch.bool, "known")
+    _chk(seeds, torch.int64, "seeds")
+    _chk(noise, torch.float32, "noise")
+    _chk(rows, torch.float32, "rows")
+    _chk(step, torch.int32, "step")
+    if x.dim() != 5 or x.shape[1] != 3 or x_known.shape != x.shape:
+        raise ValueError(f"impose_known: x and x_known must be one (B, 3, tp, h, w) shape, got {tuple(x.shape)} and "
+                         f"{tuple(x_known.shape)}")
+    B, _, tp, h, w = x.shape
+    if known is None or tuple(known.shape) != (B, tp) or known.device != x.device:
+        raise ValueError(f"impose_known: known must be a ({B}, {tp}) bool tensor on {x.device}")
+    if (seeds is None) == (noise is None):
+        raise ValueError("impose_known: pass exactly one of seeds and noise")
+    if seeds is not None and (seeds.numel() != B or seeds.device != x.device):
+        raise ValueError(f"impose_known: seeds must be {B} int64 on {x.device}")
+    if noise is not None and (noise.dim() != 6 or noise.shape[1:] != x.shape):
+        raise ValueError(f"impose_known: noise must be (K, *{tuple(x.shape)}), got {tuple(noise.shape)}")
+    if (rows is None) != (step is None) or (rows is not None and (rows.dim() != 2 or rows.shape[1] != 3)):
+        raise ValueError("impose_known: pass rows ((K + 1, 3)) and step together, or neither")
+    if rows is None and (int(k) < 0 or (noise is not None and not final and int(k) >= noise.shape[0])):
+        raise ValueError(f"impose_known: k = {k} outside the noise tensor")
+    if (h * w) % 4:
+        raise ValueError("impose_known: h * w must be a multiple of 4")
+    rec.emit("extdm_impose_known", (_p(x), _p(x_known), _p(known), _p(seeds), _p(noise), C.c_float(a), C.c_float(b),
+                                    int(k), int(bool(final)), _p(rows), _p(step), B, tp, h * w),
+             keep=(x, x_known, known, seeds, noise, rows, step))
+
+
 def denoise_loss(rec, eps, pred, out, l1=False):
     """out (B, tp) = mean over (3, h, w) of (eps - pred)^2, or |eps - pred| with l1, per (video, frame) of eps, pred
     (B, 3, tp, h, w)."""

@@ -305,6 +305,8 @@ int extdm_ddim_update_seeded(const float* img, const float* pred, const long lon
  * (extdm_dpmpp_update): iteration i draws counter (element index / 4 within the video, i, 3, 0); its x_T is stream 1.
  * Streams 4 and 5 are the epsilons of the two endpoints of an interpolation (extdm_q_interpolate): counter (element
  * index / 4 within the video, t, 4 or 5, 0), t the mix timestep; its loop noise is stream 0 as above.
+ * Stream 6 is the noise of the keyframe replacements (extdm_impose_known): replacement point k draws counter (element
+ * index / 4 within the video, k, 6, 0); the loop noise around it is that of the plain DDIM or ancestral sampler.
  */
 
 /* s[b] = max(1, quantile_q(|c_recip*img - c_recipm1*pred|)) with the coefficients of row *step (as
@@ -377,6 +379,23 @@ int extdm_denoise_loss(const float* eps, const float* pred, float* out, int B, i
 int extdm_q_interpolate(const float* x1, const float* x2, int t, const long long* seeds, const float* noise,
                         const float* sqrt_acp, const float* sqrt_1m_acp, float c1, float c2, float* x_t_out, int B,
                         int n, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Keyframe-conditioned sampling (GaussianDiffusion.sample_with_known: replacement of known frames, Song et al. 2021,
+ * Lugmayr et al. 2022), fp32.  Added under ABI version 5 (backward compatible).
+ */
+
+/* Replacement point k on x, x_known (B, 3, tp, hw) fp32 and known (B, tp) bool (one byte per flag): every element of
+ * frame f of video b with known[b, f] becomes
+ *   x = a * x_known + b * eps_k                                          (two roundings, one sum, no FMA)
+ * or x_known itself when final (nothing is drawn).  Elements of unknown frames are neither read from x_known nor
+ * written.  eps_k is noise[k] of noise ((K, B, 3*tp*hw)) when noise != NULL, else the Philox draw of (seeds[b], k,
+ * stream 6) documented above; exactly one of seeds ((B,) int64) and noise is given.  (a, b, k, final) are the launch
+ * scalars when rows == NULL (the DDIM loop); otherwise k = *step and (a, b, final != 0) = rows[k] of the (K + 1, 3)
+ * fp32 table (the ancestral loop, through the step counter of extdm_ddpm_update).  hw = h*w must be a multiple of 4. */
+int extdm_impose_known(float* x, const float* x_known, const unsigned char* known, const long long* seeds,
+                       const float* noise, float a, float b, int k, int final, const float* rows, const int* step,
+                       int B, int tp, int hw, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * LFAE decode (Generator.forward_with_flow / deform_input / apply_optical, model/LFAE/generator.py:63-93,
